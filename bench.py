@@ -2,6 +2,7 @@
 """bench.py -- spectrogram frames/sec on B200 (BASELINE.json metric).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload NAME]
+                    [--dump-outputs DIR]
 
 One process per GPU (under torchrun for N > 1: RANK / LOCAL_RANK / WORLD_SIZE from the
 environment).  A "step" is one pass of the fused spectrogram path over one rank's shard of
@@ -16,7 +17,7 @@ value  = frames/s with the samples already resident in HBM (device time, CUDA ev
 e2e    = the same metric through glfer_gram_run() with pinned HOST buffers: H2D of the samples
          and D2H of the rows inside the timed region, pipelined in chunks on two streams.
 roofline = algorithmic bytes (hop*4 + (N/2+1)*4 per frame) / the fused kernel's own duration,
-         against the measured HBM copy bandwidth in MEASURED_PEAKS.json.
+         against the measured HBM copy bandwidth HBM_PEAK_GBS.
 cpu_baseline / --impl reference = the reference's own C code (oracle/_ref, float radix-2
          build = what glfer ships) on the host cores, on a bounded sample of the workload.
 """
@@ -64,12 +65,10 @@ WORKLOADS = {
 CONFIG_BLOCK = ["c1", "c2", "c3", "c5", "lmp"]
 
 
-def measured_peak_gbs():
-    try:
-        with open(os.path.join(ROOT, "MEASURED_PEAKS.json")) as fh:
-            return float(json.load(fh)["hbm_gbs"]), "measured (MEASURED_PEAKS.json hbm_gbs)"
-    except Exception:
-        return 6650.0, "fallback (B200_PROFILING.md)"
+# the roofline's peak: read + write bytes of a 4 GiB device-to-device copy over its CUDA-event time, measured on
+# one NVIDIA B200 at a 1000 W power limit (three runs of 20 copies: 6659-6662 GB/s)
+HBM_PEAK_GBS = 6660.0
+HBM_PEAK_SOURCE = "measured: 4 GiB device-to-device copy on one B200 at a 1000 W power limit"
 
 
 # ----------------------------------------------------------------------------- clocks
@@ -194,9 +193,11 @@ def cpu_reference_rate(kw, target_s=6.0, cores=None, libkind="f32"):
     frames = sum(r[0] for r in res)
     tmax = max(r[1] for r in res)
     build = {"f32": "gcc -O2", "f32_o3": "gcc -O3 -march=x86-64-v3 (built off-box: -march=native of the build container would not be portable to this host)"}.get(libkind, libkind)
+    code = (f"reference float radix-2 build ({build}), fft_do+fft_psd loop" if kind == "reference"
+            else "numpy restatement (oracle/glfer_oracle.py): the reference's C build, oracle/_ref, is not present")
     return {"value": frames / tmax, "unit": "frames/s", "cores": cores, "kind": kind,
             "sample": f"{reps} x {frames_per_rep} frames ({nsamp / FS:.0f} s of signal) per core, {cores} core(s) concurrently; "
-                      f"reference float radix-2 build ({build}), fft_do+fft_psd loop; wall {wall:.1f} s",
+                      f"{code}; wall {wall:.1f} s",
             "frames": frames, "seconds": tmax}
 
 
@@ -225,6 +226,25 @@ def pin_to_gpu_numa_node(local_rank: int):
 def emit(line: dict) -> None:
     """The one JSON line of the contract, on the real stdout."""
     os.write(_STDOUT_FD, (json.dumps(line) + "\n").encode())
+
+
+DUMP_BYTES = 64 * 10**6 - 4096         # 64 MB in all, the .npy headers included
+
+
+def dump_outputs(res: dict, out_dir: str) -> None:
+    """Writes the arrays the timed path hands its caller (GramPlan.fetch) as out_dir/<name>.npy in float32 or
+    float64, so that two builds can be compared output for output.  When they exceed DUMP_BYTES, every array
+    keeps the same frames: a sample drawn with a fixed seed, in frame order."""
+    arrays = {k: v if v.dtype in (np.float32, np.float64) else v.astype(np.float64) for k, v in res.items() if v is not None}
+    nf = next(iter(arrays.values())).shape[0]
+    per_frame = sum(a.nbytes for a in arrays.values()) // max(nf, 1)
+    keep = DUMP_BYTES // max(per_frame, 1)
+    if nf > keep:
+        idx = np.sort(np.random.default_rng(0).choice(nf, keep, replace=False))
+        arrays = {k: a[idx] for k, a in arrays.items()}
+    os.makedirs(out_dir, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{k}.npy"), np.ascontiguousarray(a))
 
 
 def hop_of(kw):
@@ -261,7 +281,12 @@ def main():
     ap.add_argument("--seconds", type=int, default=0, help="override the seconds of signal per rank")
     ap.add_argument("--kernel-pref", type=int, default=0, help="experiment: 0 auto, 1 general, 2 ring, 3 warp-per-frame, 4 two frames per thread")
     ap.add_argument("--no-submean", action="store_true", help="experiment: opt.autoscale = 0 (no block-mean removal)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0's shard; "
+                         "a fixed, seeded sample of its frames when all of them would exceed 64 MB)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -337,7 +362,7 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.SUM)
         return float(t.item())
 
-    peak, peak_src = measured_peak_gbs()
+    peak, peak_src = HBM_PEAK_GBS, HBM_PEAK_SOURCE
 
     # this rank's shard of the (world x seconds) recording
     nframes_total = world * seconds * FS // hop
@@ -371,6 +396,8 @@ def main():
     t_wall = time.perf_counter() - t_wall0
     launches = api.kernel_launches() - launches0
     family = api.last_kernel_family()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(plan.fetch(nf), args.dump_outputs)
     dev_s = max_over_ranks(sum(step_ms) * 1e-3)
     gram_s = sum(gram_ms) * 1e-3 / len(gram_ms)
     value = world * nf * args.steps / dev_s          # all ranks do nf (+-1) frames per step
