@@ -60,6 +60,11 @@ class DisplayConfig(C.Structure):      # include/glfer_b200.h glfer_display_conf
                 ("min_level_db", C.c_float), ("thr_level", C.c_float), ("colortab", C.c_void_p)]
 
 
+class ZoomConfig(C.Structure):       # include/glfer_b200.h glfer_zoom_config
+    _fields_ = [("n", C.c_int), ("decim", C.c_int), ("window_type", C.c_int), ("overlap", C.c_float),
+                ("center_hz", C.c_double), ("sample_rate", C.c_double), ("device", C.c_int)]
+
+
 class Wav(C.Structure):
     _fields_ = [("sample_rate", C.c_int), ("bits", C.c_int), ("channels", C.c_int), ("nsamples", C.c_longlong),
                 ("data", C.c_void_p)]
@@ -118,6 +123,22 @@ def lib() -> C.CDLL:
         l.glfer_wav_num_frames.argtypes = [C.c_void_p, C.POINTER(Wav)]
         l.glfer_wav_num_frames.restype = C.c_longlong
         l.glfer_gram_run_wav.argtypes = [C.c_void_p, C.POINTER(Wav)] + [C.c_void_p] * 5
+        # zoom spectrogram
+        l.glfer_zoom_plan_create.argtypes = [C.POINTER(ZoomConfig), C.POINTER(C.c_void_p)]
+        l.glfer_zoom_plan_destroy.argtypes = [C.c_void_p]
+        l.glfer_zoom_hop.argtypes = [C.c_void_p]
+        l.glfer_zoom_bins.argtypes = [C.c_void_p]
+        l.glfer_zoom_center_hz.argtypes = [C.c_void_p]
+        l.glfer_zoom_center_hz.restype = C.c_double
+        l.glfer_zoom_num_frames.argtypes = [C.c_void_p, C.c_longlong]
+        l.glfer_zoom_num_frames.restype = C.c_longlong
+        l.glfer_zoom_required_span.argtypes = [C.c_void_p, C.c_longlong, C.c_longlong, C.POINTER(C.c_longlong),
+                                               C.POINTER(C.c_longlong)]
+        l.glfer_zoom_required_span.restype = None
+        zoom_args = [C.c_void_p, C.c_void_p, C.c_longlong, C.c_longlong, C.c_longlong, C.c_longlong, C.c_void_p]
+        l.glfer_zoom_run.argtypes = zoom_args
+        l.glfer_zoom_run_pcm16.argtypes = zoom_args
+        l.glfer_zoom_taps.argtypes = [C.c_int, C.c_void_p]
         # per-call interface
         l.fft_init.argtypes = [C.POINTER(FftParams)]
         l.fft_do.argtypes = [C.c_void_p, C.POINTER(FftParams)]
@@ -381,6 +402,68 @@ class GramPlan:
                         bits=wav.bits)
         finally:
             lib().glfer_wav_free(C.byref(wav))
+
+
+class ZoomPlan:
+    """glfer_zoom_plan: mix center_hz to DC, low-pass and decimate by `decim`, complex FFT frames of n points.
+    Rows hold n bins in frequency order, bin j at center_hz() + (j - n/2) * sample_rate / (decim * n)."""
+
+    def __init__(self, n=4096, decim=256, window_type=HANNING, overlap=0.0, center_hz=800.0, sample_rate=48000.0,
+                 device=0):
+        self.cfg = ZoomConfig(n, decim, window_type, overlap, center_hz, sample_rate, device)
+        self._h = C.c_void_p()
+        _check(lib().glfer_zoom_plan_create(C.byref(self.cfg), C.byref(self._h)))
+        self.n = n
+        self.decim = decim
+        self.hop = lib().glfer_zoom_hop(self._h)
+        self.bins = lib().glfer_zoom_bins(self._h)
+
+    def close(self):
+        if self._h:
+            lib().glfer_zoom_plan_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def center_hz(self) -> float:
+        """the actual centre, step * sample_rate / 2**32"""
+        return float(lib().glfer_zoom_center_hz(self._h))
+
+    def num_frames(self, nsamples: int) -> int:
+        return int(lib().glfer_zoom_num_frames(self._h, nsamples))
+
+    def required_span(self, first_frame: int, nframes: int):
+        lo, hi = C.c_longlong(), C.c_longlong()
+        lib().glfer_zoom_required_span(self._h, first_frame, nframes, C.byref(lo), C.byref(hi))
+        return lo.value, hi.value
+
+    def taps(self) -> np.ndarray:
+        return zoom_taps(self.decim)
+
+    def run(self, samples: np.ndarray, origin: int = 0, first_frame: int = 0, nframes: int | None = None,
+            out: np.ndarray | None = None) -> np.ndarray:
+        """glfer_zoom_run / glfer_zoom_run_pcm16 (int16 samples): rows [nframes][n].  out: optional
+        pre-allocated (e.g. pinned) rows."""
+        pcm = samples.dtype == np.int16
+        assert samples.flags["C_CONTIGUOUS"] and (pcm or samples.dtype == np.float32)
+        if nframes is None:
+            nframes = self.num_frames(origin + len(samples)) - first_frame
+        rows = out if out is not None else np.empty((nframes, self.bins), np.float32)
+        assert rows.dtype == np.float32 and rows.size >= nframes * self.bins
+        fn = lib().glfer_zoom_run_pcm16 if pcm else lib().glfer_zoom_run
+        _check(fn(self._h, samples.ctypes.data, origin, len(samples), first_frame, nframes, rows.ctypes.data))
+        return rows
+
+
+def zoom_taps(decim: int) -> np.ndarray:
+    """glfer_zoom_taps: the zoom low-pass h[l], l = -K..K (K = 16 decim), as float32; needs no device"""
+    h = np.empty(32 * decim + 1 if 2 <= decim <= 1024 else 1, dtype=np.float32)   # the library rejects other values
+    _check(lib().glfer_zoom_taps(decim, h.ctypes.data))
+    return h
 
 
 def run_sharded(samples: np.ndarray, ndev: int, devices=None, want_psd: bool = True, **kw):

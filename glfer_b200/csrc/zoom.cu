@@ -1,0 +1,188 @@
+// zoom.cu -- kernels of the zoom spectrogram (host/zoom.c): mix a centre frequency to DC, low-pass and
+// decimate by D, then turn the general spectrogram kernel's real-FFT output of the decimated stream into
+// complex-FFT rows.
+//
+//   zoom_decim_kernel<T>  the hot path.  y[m] = e^{-2 pi i phi(mD)} sum_j g[j] x[mD - K + j], j = 0..2K,
+//                         with the complex taps g[j] = h[K - j] e^{+2 pi i phi(K - j)} built on the host.
+//                         Polyphase form: phase p = j mod D owns the 33 taps g[p + tD] (zero-padded past
+//                         2K), and its contribution to output m is a 33-tap FIR over the stream
+//                         u_p[q] = x[qD - K + p].  A lane holds the taps of one phase in registers and
+//                         streams u_p once for kZR consecutive outputs: each loaded sample feeds up to
+//                         2 kZR FMAs, so the loop runs on the FP32 pipe, not on loads.  Lanes take
+//                         consecutive phases (coalesced loads of x and of the taps, no shared-memory
+//                         stride-D access); a lane walks the phases p = sl, sl + 32, ... of its group in
+//                         order, and the lane partials are summed in a fixed order through shared memory.
+//                         The sum order of an output therefore depends on D only, never on where the
+//                         output falls in a launch or chunk.  int16 input is converted in registers.
+//   zoom_split_kernel     X[k], k = 0..Nz, of the interleaved (re, im) stream seen as 2 Nz real points ->
+//                         Z[k] = E + iO of the complex frame -> |Z|^2 / Nz in fft-shifted bin order.
+#include <cuda_runtime.h>
+#include <atomic>
+#include <cstdio>
+#include "../../include/glb_shim.h"
+
+extern std::atomic<unsigned long long> g_launches;   // gram_kernels.cu
+
+#define ZCU(call)                                                                             \
+  do {                                                                                        \
+    cudaError_t e_ = (call);                                                                  \
+    if (e_ != cudaSuccess) {                                                                  \
+      char m_[512];                                                                           \
+      snprintf(m_, sizeof m_, "%s failed: %s (%s:%d)", #call, cudaGetErrorString(e_),         \
+               __FILE__, __LINE__);                                                           \
+      glb_set_error(m_);                                                                      \
+      return GLB_ECUDA;                                                                       \
+    }                                                                                         \
+  } while (0)
+
+constexpr int kZR = 16;        // outputs per lane group
+constexpr int kZT = 33;        // taps per phase: 32 D + 1 taps, zero-padded to 33 D
+constexpr int kZWarps = 8;
+
+static __device__ __forceinline__ float zload(const float *x, long long i, long long count) {
+  return (i >= 0 && i < count) ? __ldg(x + i) : 0.f;
+}
+// wav_fmt.c:113: (float) s / 32768 (a power-of-two scale: exact, so equal to the float path's input)
+static __device__ __forceinline__ float zload(const short *x, long long i, long long count) {
+  return (i >= 0 && i < count) ? (float) __ldg(x + i) * (1.f / 32768.f) : 0.f;
+}
+
+template <typename T>
+__global__ void __launch_bounds__(kZWarps * 32)
+zoom_decim_kernel(const T *__restrict__ x, long long origin, long long count, int D, int LG, int G,
+                  const float2 *__restrict__ taps, unsigned dstep, long long m_first, long long m_count,
+                  float2 *__restrict__ y) {
+  __shared__ float part[kZWarps][32][2 * kZR + 1];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int per_blk = G * kZR;
+  const long long nblk = (m_count + per_blk - 1) / per_blk;
+  const int gi = lane / LG, sl = lane - gi * LG;
+  const bool active = gi < G;
+  const long long K = 16LL * D;
+  for (long long b = (long long) blockIdx.x * kZWarps + w; b < nblk; b += (long long) gridDim.x * kZWarps) {
+    const long long mb = m_first + b * per_blk;
+    float ar[kZR], ai[kZR];
+#pragma unroll
+    for (int r = 0; r < kZR; r++) ar[r] = ai[r] = 0.f;
+    if (active) {
+      const long long i0 = (mb + (long long) gi * kZR) * D - K - origin;
+      for (int p = sl; p < D; p += LG) {
+        float tr[kZT], ti[kZT];
+#pragma unroll
+        for (int t = 0; t < kZT; t++) {
+          const float2 c = __ldg(taps + t * D + p);
+          tr[t] = c.x;
+          ti[t] = c.y;
+        }
+        const long long ip = i0 + p;
+#pragma unroll
+        for (int q = 0; q < kZR + kZT - 1; q++) {
+          const float u = zload(x, ip + (long long) q * D, count);
+#pragma unroll
+          for (int r = 0; r < kZR; r++) {
+            const int t = q - r;
+            if (t >= 0 && t < kZT) {
+              ar[r] = fmaf(tr[t], u, ar[r]);
+              ai[r] = fmaf(ti[t], u, ai[r]);
+            }
+          }
+        }
+      }
+    }
+#pragma unroll
+    for (int r = 0; r < kZR; r++) {
+      part[w][lane][2 * r] = ar[r];
+      part[w][lane][2 * r + 1] = ai[r];
+    }
+    __syncwarp();
+    for (int o = lane; o < per_blk; o += 32) {
+      const int g = o / kZR, r = o - g * kZR;
+      const long long m = mb + o;
+      float sr = 0.f, si = 0.f;
+      for (int s = 0; s < LG; s++) {
+        sr += part[w][g * LG + s][2 * r];
+        si += part[w][g * LG + s][2 * r + 1];
+      }
+      if (m < m_first + m_count) {
+        // phi(mD) 2^32 exactly in 32-bit arithmetic; as a signed value / 2^31 it is the angle in half-turns
+        const unsigned ph = (unsigned) (unsigned long long) m * dstep;
+        float sn, cs;
+        sincospif((float) (int) ph * 4.656612873077393e-10f, &sn, &cs);
+        y[m - m_first] = make_float2(fmaf(sr, cs, si * sn), fmaf(si, cs, -(sr * sn)));
+      }
+    }
+    __syncwarp();
+  }
+}
+
+__global__ void zoom_split_kernel(const float2 *__restrict__ spec, int nz, long long nframes, float inv_nz,
+                                  float *__restrict__ rows) {
+  const long long total = nframes * nz;
+  const long long stride = (long long) gridDim.x * blockDim.x;
+  for (long long idx = (long long) blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += stride) {
+    const long long f = idx / nz;
+    const int j = (int) (idx - f * nz);
+    const int k = (j + nz / 2) & (nz - 1);
+    const float2 *X = spec + f * (nz + 1);
+    const float2 a = X[k], c = X[nz - k];
+    // E = (X[k] + conj X[Nz-k]) / 2,  O = (X[k] - conj X[Nz-k]) / (2 W^k),  W = e^{-i pi / Nz}
+    const float er = 0.5f * (a.x + c.x), ei = 0.5f * (a.y - c.y);
+    const float dr = 0.5f * (a.x - c.x), di = 0.5f * (a.y + c.y);
+    float sn, cs;
+    sincospif((float) k / (float) nz, &sn, &cs);
+    const float orr = dr * cs - di * sn, oi = dr * sn + di * cs;
+    const float zr = er - oi, zi = ei + orr;          // Z = E + i O
+    rows[idx] = (zr * zr + zi * zi) * inv_nz;
+  }
+}
+
+static int sm_count() {
+  int dev = 0, sms = 148;
+  if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  return sms;
+}
+
+template <typename T>
+static int launch_decim(const T *x, long long origin, long long count, int decim, const void *taps, unsigned dstep,
+                        long long m_first, long long m_count, void *y, void *stream) {
+  const int lg = decim < 32 ? decim : 32;
+  const int g = 32 / lg;
+  const long long nblk = (m_count + (long long) g * kZR - 1) / ((long long) g * kZR);
+  long long ctas = (nblk + kZWarps - 1) / kZWarps;
+  const long long cap = (long long) sm_count() * 8;
+  if (ctas > cap) ctas = cap;
+  zoom_decim_kernel<T><<<(int) ctas, kZWarps * 32, 0, (cudaStream_t) stream>>>(
+      x, origin, count, decim, lg, g, (const float2 *) taps, dstep, m_first, m_count, (float2 *) y);
+  ZCU(cudaGetLastError());
+  g_launches++;
+  return GLB_OK;
+}
+
+extern "C" int glb_launch_zoom_decim(const void *x, int pcm16, long long origin, long long count, int decim,
+                                     const void *taps, unsigned dstep, long long m_first, long long m_count,
+                                     void *y, void *stream) {
+  if (decim < 2 || decim > 1024 || !taps || !y || origin < 0 || count < 0 || m_first < 0) {
+    glb_set_error("glb_launch_zoom_decim: invalid arguments");
+    return GLB_EINVAL;
+  }
+  if (m_count <= 0) return GLB_OK;
+  if (pcm16) return launch_decim((const short *) x, origin, count, decim, taps, dstep, m_first, m_count, y, stream);
+  return launch_decim((const float *) x, origin, count, decim, taps, dstep, m_first, m_count, y, stream);
+}
+
+extern "C" int glb_launch_zoom_split(const void *spec, int nz, long long nframes, float *rows, void *stream) {
+  if (nz < 2 || (nz & (nz - 1)) != 0 || !spec || !rows) {
+    glb_set_error("glb_launch_zoom_split: invalid arguments");
+    return GLB_EINVAL;
+  }
+  if (nframes <= 0) return GLB_OK;
+  const long long total = nframes * nz;
+  long long ctas = (total + 255) / 256;
+  const long long cap = (long long) sm_count() * 16;
+  if (ctas > cap) ctas = cap;
+  zoom_split_kernel<<<(int) ctas, 256, 0, (cudaStream_t) stream>>>((const float2 *) spec, nz, nframes,
+                                                                  (float) (1.0 / nz), rows);
+  ZCU(cudaGetLastError());
+  g_launches++;
+  return GLB_OK;
+}

@@ -13,6 +13,10 @@ double glb_bessel_i0(double x);
 void glb_window_table(int n, int window_type, float *w);
 int glb_dpss(int n, double nw, int kmax, double *tapers, double *lambda);
 int glb_hop(int n, float overlap);
+/* the message slot of glfer_b200_last_error() (gram.c), for the other host units */
+int glb_host_fail(int code, const char *msg);
+int glb_host_shim(int rc);
+void glb_host_clear_error(void);
 
 /* display mapping tables (host/levels.c) */
 #define GLB_DB_JMIN (-450)

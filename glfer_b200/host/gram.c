@@ -119,6 +119,10 @@ static int shim(int rc)
 
 #define TRY(x) do { int rc_ = shim(x); if (rc_ != 0) return rc_; } while (0)
 
+int glb_host_fail(int code, const char *msg) { return fail(code, msg); }
+int glb_host_shim(int rc) { return shim(rc); }
+void glb_host_clear_error(void) { g_msg[0] = 0; }
+
 int glfer_b200_device_count(void)
 {
   int c = 0;

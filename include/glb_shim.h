@@ -195,6 +195,17 @@ int glb_launch_levels(const float *rows, long long stride, int nbins, long long 
 int glb_launch_ftest(const float *spec, long long nframes, int nbins, int n, int ntapers, const double *u0,
                      double sum_u0_sqr, float *ftest, long long stride, void *stream);
 
+/* Zoom spectrogram (glfer_b200/csrc/zoom.cu).
+ * Decimator: y[m - m_first] = e^{-2 pi i (m dstep mod 2^32) / 2^32} sum_{j=0..32 decim} taps[j] x[m decim - 16 decim + j]
+ * for m in [m_first, m_first + m_count); taps: device, [33 decim] (re, im) pairs, zero past index 32 decim;
+ * dstep = decim * phase step mod 2^32.  x (float, or int16 PCM when pcm16 = 1, converted as wav_fmt.c:113) holds
+ * stream samples [origin, origin + count); indices outside read as 0.  y: device, (re, im) pairs. */
+int glb_launch_zoom_decim(const void *x, int pcm16, long long origin, long long count, int decim, const void *taps,
+                          unsigned dstep, long long m_first, long long m_count, void *y, void *stream);
+/* rows[f][j] = |Z_f[(j + nz/2) mod nz]|^2 / nz, with Z_f the complex FFT recovered from spec = [nframes][nz + 1]
+ * (re, im) pairs, the real FFT of frame f's interleaved (re, im) samples as 2 nz real points */
+int glb_launch_zoom_split(const void *spec, int nz, long long nframes, float *rows, void *stream);
+
 /* counters */
 unsigned long long glb_kernel_launches(void);
 /* family of the last spectrogram kernel launched: 1 general, 2 TMA ring, 3 warp-per-frame, 4 two frames per thread,

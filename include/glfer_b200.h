@@ -209,6 +209,48 @@ long long glfer_wav_num_frames(const glfer_gram_plan *plan, const glfer_wav *wav
 int glfer_gram_run_wav(glfer_gram_plan *plan, const glfer_wav *wav, float *psd_rows, float *avg_rows,
                        double *avg_ret, int *avg_peakbin, double *avg_variance);
 
+/* ---- zoom spectrogram: sub-hertz bins around a chosen frequency ----
+ * The stream is mixed by the centre frequency to DC (phase phi(n) = (n step mod 2^32) / 2^32, exact from the
+ * absolute sample index, step = llround(center_hz / sample_rate 2^32)), low-passed by a 32 D + 1 tap Kaiser
+ * windowed sinc (glfer_zoom_taps) and decimated by D:
+ *     y[m] = sum_{l=-K..K} h[l] x[mD - l] e^{-2 pi i phi(mD - l)},  K = 16 D,  x[n < 0] = 0,  y[m < 0] = 0.
+ * Frames of n complex samples at hop glb_hop(n, overlap) cover y[f hop - (n - hop), f hop + hop); a row is
+ *     P[f][j] = |sum_i w[i] y_f[i] e^{-2 pi i (j - n/2) i / n}|^2 / n,   j = 0..n-1,
+ * with w the spectrogram window of that size (rectangular: all ones).  Bin j is at
+ * center + (j - n/2) sample_rate / (D n); the clean span is |f - center| <= 0.4 sample_rate / D. */
+typedef struct {
+  int n;               /* complex FFT size: power of two, 32..16384 */
+  int decim;           /* decimation D: 2..1024 */
+  int window_type;     /* fft.h window enum */
+  float overlap;       /* hop = (int)(n * (1.0 - overlap)), as the spectrogram */
+  double center_hz;    /* 0 <= center_hz <= sample_rate / 2 */
+  double sample_rate;
+  int device;          /* CUDA device ordinal */
+} glfer_zoom_config;
+
+typedef struct glfer_zoom_plan glfer_zoom_plan;
+
+void glfer_zoom_config_default(glfer_zoom_config *cfg);
+int glfer_zoom_plan_create(const glfer_zoom_config *cfg, glfer_zoom_plan **plan);
+void glfer_zoom_plan_destroy(glfer_zoom_plan *plan);
+int glfer_zoom_hop(const glfer_zoom_plan *plan);
+int glfer_zoom_bins(const glfer_zoom_plan *plan);                       /* n */
+double glfer_zoom_center_hz(const glfer_zoom_plan *plan);               /* step sample_rate / 2^32 */
+/* frames of a stream of nsamples samples: floor(Md / hop), Md = number of m >= 0 with mD + K <= nsamples - 1 */
+long long glfer_zoom_num_frames(const glfer_zoom_plan *plan, long long nsamples);
+/* stream span [lo, hi) the frames [first_frame, first_frame + nframes) read (lo may be negative: indices < 0 are
+ * the zero history) */
+void glfer_zoom_required_span(const glfer_zoom_plan *plan, long long first_frame, long long nframes,
+                              long long *lo, long long *hi);
+/* samples point at stream index `origin`, `count` samples long, and must cover glfer_zoom_required_span()
+ * clipped to [0, inf).  rows: [nframes][n] */
+int glfer_zoom_run(glfer_zoom_plan *plan, const float *samples, long long origin, long long count,
+                   long long first_frame, long long nframes, float *rows);
+int glfer_zoom_run_pcm16(glfer_zoom_plan *plan, const short *pcm, long long origin, long long count,
+                         long long first_frame, long long nframes, float *rows);
+/* the low-pass filter h[l], l = -K..K, as taps[l + K] (32 decim + 1 floats); host only, needs no device */
+int glfer_zoom_taps(int decim, float *taps);
+
 /* ---- hidden inputs of the per-call interface (fft.c:99,186: globals `glfer`, `opt`) ----
  * When the host program defines `opt` and `glfer` (as glfer.c:56-62 does) the per-call
  * functions read them.  Otherwise these setters provide the two values. */
