@@ -1488,6 +1488,18 @@ inline int launch_gram_m(const KParams &kp, bool multi, int groups_hint, cudaStr
         const bool worth = occ >= 2 || (occ >= 1 && occ_generic_bound <= 1) || GeoM::THREADS >= 512 || g_kernel_pref == 2;
         if (occ >= 1 && worth) {
           long long groups = groups_hint > 0 ? groups_hint : (long long) sms * occ * GeoM::G;
+          // Several waves of shorter frame runs instead of one run per resident group: groups that share an SM
+          // do not progress at the same rate, and with a single wave the early finishers leave their slots
+          // idle for the rest of the launch; with more CTAs than slots the block scheduler refills them.  A run
+          // pays one prologue (the nb - 1 history blocks and their means, other CTAs of the SM hide it), so
+          // runs stay >= kRingMinRun frames.  Metric workload (N = 4096, 84 375 frames, B200): 1 / 2 / 3 / 4 / 6
+          // waves 0.423 / 0.405 / 0.398 / 0.395 / 0.396-0.401 ms.  Rows do not depend on the split.
+          constexpr int kRingWaves = 4, kRingMinRun = 16;
+          if (groups_hint <= 0 && occ >= 2) {
+            int waves = kRingWaves;
+            while (waves > 1 && kp.nframes < groups * waves * kRingMinRun) waves--;
+            groups *= waves;
+          }
           if (groups > kp.nframes) groups = kp.nframes;
           if (groups < 1) groups = 1;
           KParams k = kp;
