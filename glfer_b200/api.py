@@ -65,6 +65,10 @@ class ZoomConfig(C.Structure):       # include/glfer_b200.h glfer_zoom_config
                 ("center_hz", C.c_double), ("sample_rate", C.c_double), ("device", C.c_int)]
 
 
+class IqConfig(C.Structure):         # include/glfer_b200.h glfer_iq_config
+    _fields_ = [("n", C.c_int), ("window_type", C.c_int), ("overlap", C.c_float), ("device", C.c_int)]
+
+
 class Wav(C.Structure):
     _fields_ = [("sample_rate", C.c_int), ("bits", C.c_int), ("channels", C.c_int), ("nsamples", C.c_longlong),
                 ("data", C.c_void_p)]
@@ -139,6 +143,21 @@ def lib() -> C.CDLL:
         l.glfer_zoom_run.argtypes = zoom_args
         l.glfer_zoom_run_pcm16.argtypes = zoom_args
         l.glfer_zoom_taps.argtypes = [C.c_int, C.c_void_p]
+        l.glfer_zoom_plan_create_iq.argtypes = [C.POINTER(ZoomConfig), C.POINTER(C.c_void_p)]
+        l.glfer_zoom_run_iq.argtypes = zoom_args
+        l.glfer_zoom_run_iq_pcm16.argtypes = zoom_args
+        # I/Q spectrogram
+        l.glfer_iq_plan_create.argtypes = [C.POINTER(IqConfig), C.POINTER(C.c_void_p)]
+        l.glfer_iq_plan_destroy.argtypes = [C.c_void_p]
+        l.glfer_iq_hop.argtypes = [C.c_void_p]
+        l.glfer_iq_bins.argtypes = [C.c_void_p]
+        l.glfer_iq_num_frames.argtypes = [C.c_void_p, C.c_longlong]
+        l.glfer_iq_num_frames.restype = C.c_longlong
+        l.glfer_iq_required_span.argtypes = [C.c_void_p, C.c_longlong, C.c_longlong, C.POINTER(C.c_longlong),
+                                             C.POINTER(C.c_longlong)]
+        l.glfer_iq_required_span.restype = None
+        l.glfer_iq_run.argtypes = zoom_args
+        l.glfer_iq_run_pcm16.argtypes = zoom_args
         # per-call interface
         l.fft_init.argtypes = [C.POINTER(FftParams)]
         l.fft_do.argtypes = [C.c_void_p, C.POINTER(FftParams)]
@@ -404,15 +423,29 @@ class GramPlan:
             lib().glfer_wav_free(C.byref(wav))
 
 
+def _iq_samples(iq: np.ndarray):
+    """(pointer, complex sample count, pcm16) of an I/Q array: 1-D complex64 (its memory is already interleaved,
+    no copy), float32 [count, 2] or int16 [count, 2] (I, Q)"""
+    assert iq.flags["C_CONTIGUOUS"], "I/Q samples must be C-contiguous"
+    if iq.dtype == np.complex64 and iq.ndim == 1:
+        return iq.ctypes.data, len(iq), False
+    assert iq.ndim == 2 and iq.shape[1] == 2 and iq.dtype in (np.float32, np.int16), \
+        "I/Q samples: complex64 [count], float32 [count, 2] or int16 [count, 2]"
+    return iq.ctypes.data, iq.shape[0], iq.dtype == np.int16
+
+
 class ZoomPlan:
     """glfer_zoom_plan: mix center_hz to DC, low-pass and decimate by `decim`, complex FFT frames of n points.
-    Rows hold n bins in frequency order, bin j at center_hz() + (j - n/2) * sample_rate / (decim * n)."""
+    Rows hold n bins in frequency order, bin j at center_hz() + (j - n/2) * sample_rate / (decim * n).
+    iq=True: complex (I/Q) input (glfer_zoom_plan_create_iq), centre in [-sample_rate/2, sample_rate/2]."""
 
     def __init__(self, n=4096, decim=256, window_type=HANNING, overlap=0.0, center_hz=800.0, sample_rate=48000.0,
-                 device=0):
+                 device=0, iq=False):
         self.cfg = ZoomConfig(n, decim, window_type, overlap, center_hz, sample_rate, device)
         self._h = C.c_void_p()
-        _check(lib().glfer_zoom_plan_create(C.byref(self.cfg), C.byref(self._h)))
+        self.iq = iq
+        create = lib().glfer_zoom_plan_create_iq if iq else lib().glfer_zoom_plan_create
+        _check(create(C.byref(self.cfg), C.byref(self._h)))
         self.n = n
         self.decim = decim
         self.hop = lib().glfer_zoom_hop(self._h)
@@ -447,7 +480,16 @@ class ZoomPlan:
     def run(self, samples: np.ndarray, origin: int = 0, first_frame: int = 0, nframes: int | None = None,
             out: np.ndarray | None = None) -> np.ndarray:
         """glfer_zoom_run / glfer_zoom_run_pcm16 (int16 samples): rows [nframes][n].  out: optional
-        pre-allocated (e.g. pinned) rows."""
+        pre-allocated (e.g. pinned) rows.  An I/Q plan takes the formats of IqPlan.run."""
+        if self.iq:
+            ptr, count, pcm = _iq_samples(samples)
+            if nframes is None:
+                nframes = self.num_frames(origin + count) - first_frame
+            rows = out if out is not None else np.empty((nframes, self.bins), np.float32)
+            assert rows.dtype == np.float32 and rows.size >= nframes * self.bins
+            fn = lib().glfer_zoom_run_iq_pcm16 if pcm else lib().glfer_zoom_run_iq
+            _check(fn(self._h, ptr, origin, count, first_frame, nframes, rows.ctypes.data))
+            return rows
         pcm = samples.dtype == np.int16
         assert samples.flags["C_CONTIGUOUS"] and (pcm or samples.dtype == np.float32)
         if nframes is None:
@@ -456,6 +498,52 @@ class ZoomPlan:
         assert rows.dtype == np.float32 and rows.size >= nframes * self.bins
         fn = lib().glfer_zoom_run_pcm16 if pcm else lib().glfer_zoom_run
         _check(fn(self._h, samples.ctypes.data, origin, len(samples), first_frame, nframes, rows.ctypes.data))
+        return rows
+
+
+class IqPlan:
+    """glfer_iq_plan: two-sided spectrogram of complex (I/Q) input.  Rows hold n bins, bin j at
+    (j - n/2) * sample_rate / n (DC at n/2): |FFT(w z_f)|^2 / n, fft-shifted."""
+
+    def __init__(self, n=4096, window_type=HANNING, overlap=0.5, device=0):
+        self.cfg = IqConfig(n, window_type, overlap, device)
+        self._h = C.c_void_p()
+        _check(lib().glfer_iq_plan_create(C.byref(self.cfg), C.byref(self._h)))
+        self.n = n
+        self.hop = lib().glfer_iq_hop(self._h)
+        self.bins = lib().glfer_iq_bins(self._h)
+
+    def close(self):
+        if self._h:
+            lib().glfer_iq_plan_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):
+        try:
+            self.close()
+        except Exception:
+            pass
+
+    def num_frames(self, nsamples: int) -> int:
+        return int(lib().glfer_iq_num_frames(self._h, nsamples))
+
+    def required_span(self, first_frame: int, nframes: int):
+        lo, hi = C.c_longlong(), C.c_longlong()
+        lib().glfer_iq_required_span(self._h, first_frame, nframes, C.byref(lo), C.byref(hi))
+        return lo.value, hi.value
+
+    def run(self, iq: np.ndarray, origin: int = 0, first_frame: int = 0, nframes: int | None = None,
+            out: np.ndarray | None = None) -> np.ndarray:
+        """glfer_iq_run / glfer_iq_run_pcm16: rows [nframes][n] of complex64 [count], float32 [count, 2] or int16
+        [count, 2] I/Q samples (origin and count in complex samples).  out: optional pre-allocated (e.g. pinned)
+        rows."""
+        ptr, count, pcm = _iq_samples(iq)
+        if nframes is None:
+            nframes = self.num_frames(origin + count) - first_frame
+        rows = out if out is not None else np.empty((nframes, self.bins), np.float32)
+        assert rows.dtype == np.float32 and rows.size >= nframes * self.bins
+        fn = lib().glfer_iq_run_pcm16 if pcm else lib().glfer_iq_run
+        _check(fn(self._h, ptr, origin, count, first_frame, nframes, rows.ctypes.data))
         return rows
 
 

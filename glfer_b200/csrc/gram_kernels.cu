@@ -25,7 +25,7 @@ static thread_local char g_err[512] = "";
 std::atomic<unsigned long long> g_launches{0};
 int g_kernel_pref = 0;               // 0 auto, 1 general, 2 ring, 3 warp-per-frame, 4 two frames per thread
 int g_last_family = 0;
-static int g_force_generic = 0;     // tests: run the general kernel where the ring kernel would be chosen
+int g_force_generic = 0;            // tests: run the general kernel where the ring kernel would be chosen (also iq.cu)
 
 extern "C" const char *glb_last_error(void) { return g_err; }
 extern "C" void glb_set_error(const char *msg) { snprintf(g_err, sizeof g_err, "%s", msg ? msg : ""); }
@@ -143,6 +143,16 @@ extern "C" int glb_tables_create(int n, void **out) {
   CU(cudaMemcpy(t->tw, tw.data(), tw.size() * sizeof(float2), cudaMemcpyHostToDevice));
   CU(cudaMemcpy(t->vtab, vt.data(), vt.size() * sizeof(float2), cudaMemcpyHostToDevice));
   *out = t;
+  return GLB_OK;
+}
+
+// the tables of a launch made outside this unit (iq.cu)
+int glb_tables_get(const void *tp, int *n, const float2 **tw, const float2 **vtab) {
+  const GramTables *t = (const GramTables *) tp;
+  if (!t) return GLB_EINVAL;
+  *n = t->n;
+  *tw = t->tw;
+  *vtab = t->vtab;
   return GLB_OK;
 }
 

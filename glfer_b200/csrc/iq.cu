@@ -1,0 +1,286 @@
+// iq.cu -- two-sided spectrogram of complex (I/Q) input: rows[f][j] = |Z_f[(j + n/2) mod n]|^2 / n, Z_f the
+// complex FFT of frame f's n tapered complex samples (include/glfer_b200.h, glfer_iq_*).
+//
+//   gram_iq_kernel<M, QSC>  the fused path for the regular geometry (complex hop h = (n/16) << s, n - h a
+//                           multiple of h).  An interleaved (I, Q) frame of n complex samples is a frame of
+//                           N = 2n floats of the TMA ring kernel (gram_ring_kernel, gram_common.cuh), and the
+//                           ring kernel already transforms it as the M = n complex points (I, Q).  So this is
+//                           the ring kernel at M = n -- same ring of hop blocks, same bulk copies, same taper
+//                           multiply, same passes -- without block means and with another epilogue: instead of
+//                           the real-FFT split (emit_bins_rt), |Z[k]|^2 goes straight to row position
+//                           (k + n/2) mod n (iq_core.cuh).
+//   everything else         the general spectrogram kernel's spectrum output on the 2n-float frames, then
+//                           zoom_split_kernel (glb_launch_iq_gram_general, zoom.cu): the zoom's frame stage.
+//
+// glb_launch_iq_gram picks the path from the geometry; glb_force_generic_kernel(1) forces the general one.
+#include "gram_common.cuh"
+#include "iq_core.cuh"
+
+extern int g_force_generic;           // gram_kernels.cu
+int glb_tables_get(const void *tables, int *n, const float2 **tw, const float2 **vtab);
+
+// The taper carries taper_scale = 1 / (2 sqrt(2n)) as the zoom's (host/zoom.c), so |Z|^2 of the tapered frame is
+// the contract's |Z|^2 / n divided by 8: the epilogue multiplies by 8, exactly.
+constexpr float kIqPowerScale = 8.f;
+
+template <int M, int QSC>
+__global__ void __launch_bounds__(Geo<M>::THREADS, (RingGeo<M, false>::MINB)) gram_iq_kernel(const KParams p) {
+  using GeoM = Geo<M>;
+  constexpr int T = GeoM::T, G = GeoM::G;
+  constexpr bool RT = RingGeo<M, false>::RT;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int g = threadIdx.x / T;
+  const int t = threadIdx.x % T;
+  const int qs = QSC >= 0 ? QSC : p.qs;
+  const int hop = QSC >= 0 ? ((2 * T) << (QSC >= 0 ? QSC : 0)) : p.hop;   // floats: 2 complex hops
+  const int nb = kPoints >> qs;
+  const RingLayout L = ring_layout<M>(hop, nb);                  // the real kernel's layout (the mean slots stay unused)
+  const int slots = L.slots;
+  unsigned char *gbase = smem_raw + (size_t) g * L.group_bytes;
+  float2 *buf = reinterpret_cast<float2 *>(gbase);
+  float *ring = reinterpret_cast<float *>(gbase + L.ring_off);
+  float *red = reinterpret_cast<float *>(gbase + L.red_off);
+  float *mu = reinterpret_cast<float *>(gbase + L.mu_off);
+  unsigned long long *mbar = reinterpret_cast<unsigned long long *>(gbase + L.mbar_off);
+  const long long gid = (long long) blockIdx.x * G + g;
+  const long long fb = gid * p.frames_per_group;
+  const bool group_active = fb < p.nframes;
+  const long long f_first = p.first_frame + fb;
+  const long long b0 = f_first - (nb - 1);                       // oldest block of the first frame
+  const unsigned blk_bytes = (unsigned) hop * 4u;
+  unsigned phase_bits = 0;
+
+  TwRegs tr;
+  if constexpr (RT) load_tw_regs<M>(tr, t, p.tw, p.vtab);
+  if (t == 0) {
+    for (int sl = 0; sl < slots; sl++) mbar_init(&mbar[sl], 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  const float2 *tw_mid = p.tw;
+  if constexpr (!RT) {
+    float2 *tws = reinterpret_cast<float2 *>(smem_raw + (size_t) G * L.group_bytes);
+    constexpr int kMid = TwOffset<M, Plan<M>::NP - 1>::value;
+    for (int i = threadIdx.x; i < kMid; i += GeoM::THREADS) tws[i] = p.tw[i];
+    tw_mid = tws;
+  }
+  group_sync<M>(g);
+
+  // prologue: the nb blocks of the first frame, zeros before the stream start
+  for (int lb = 0; lb < nb; lb++) {
+    const long long blk = b0 + lb;
+    if (group_active) {
+      if (blk < 0) {
+        float2 *z = reinterpret_cast<float2 *>(ring + (size_t) lb * hop);
+        for (int i = 0; i < (1 << qs); i++) z[t + T * i] = make_float2(0.f, 0.f);
+      } else if (t == 0) {
+        GLB_CHECK_SRC(p, p.samples + (blk * hop - p.origin), hop);
+        mbar_expect_tx(&mbar[lb], blk_bytes);
+        tma_load_1d(ring + (size_t) lb * hop, p.samples + (blk * hop - p.origin), blk_bytes, &mbar[lb]);
+      }
+    }
+  }
+  for (int lb = 0; lb < nb; lb++) {
+    if (group_active && b0 + lb >= 0) {
+      mbar_wait(&mbar[lb], 0);
+      phase_bits ^= 1u << lb;
+    }
+  }
+  group_sync<M>(g);                                               // zero fill visible
+
+  int slot_new = nb - 1;
+  const int nact = group_active ? (int) ((p.nframes - fb < p.frames_per_group) ? p.nframes - fb : p.frames_per_group) : 0;
+  float *row_ptr = p.rows + fb * p.row_stride;                   // (never dereferenced past nact)
+  const float *next_src = p.samples + ((f_first + 1) * (long long) hop - p.origin);
+  int ob[4];
+  iq_row_bases<M>(t, ob);
+  float mu_new = 0.f;
+  for (int it = 0; it < p.frames_per_group; ++it, row_ptr += p.row_stride, next_src += hop) {
+    const bool active = it < nact;
+    const bool next_there = it + 1 < nact;
+    const int slot_next = (slot_new + 1 == slots) ? 0 : slot_new + 1;
+    if (it > 0 && active) {
+      mbar_wait(&mbar[slot_new], (phase_bits >> slot_new) & 1u);
+      phase_bits ^= 1u << slot_new;
+    }
+    auto request_next = [&]() {
+      GLB_CHECK_SRC(p, next_src, hop);
+      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+      mbar_expect_tx(&mbar[slot_next], blk_bytes);
+      tma_load_1d(ring + (size_t) slot_next * hop, next_src, blk_bytes, &mbar[slot_next]);
+    };
+    if (GLB_RING_EXTRA && next_there && t == 0) request_next();
+    const int slot_oldest = GLB_RING_EXTRA ? ((slot_next + 1 == slots) ? 0 : slot_next + 1) : slot_next;
+    float2 v[kPoints];
+    {
+      float2 x[kPoints];
+      if constexpr (QSC >= 0) {
+        ring_fetch<M, (QSC >= 0 ? QSC : 0)>(x, t, ring, hop, slot_oldest, slots, mu, mu_new, false, false, red, 0.f, g);
+      } else {
+        switch (qs) {
+          case 4: ring_fetch<M, 4>(x, t, ring, hop, slot_oldest, slots, mu, mu_new, false, false, red, 0.f, g); break;
+          case 3: ring_fetch<M, 3>(x, t, ring, hop, slot_oldest, slots, mu, mu_new, false, false, red, 0.f, g); break;
+          case 2: ring_fetch<M, 2>(x, t, ring, hop, slot_oldest, slots, mu, mu_new, false, false, red, 0.f, g); break;
+          case 1: ring_fetch<M, 1>(x, t, ring, hop, slot_oldest, slots, mu, mu_new, false, false, red, 0.f, g); break;
+          default: ring_fetch<M, 0>(x, t, ring, hop, slot_oldest, slots, mu, mu_new, false, false, red, 0.f, g); break;
+        }
+      }
+      apply_taper<M, true>(v, x, t, p, p.tapers);
+    }
+    if constexpr (RT) {
+      pass_compute_rt<M, 0>(v, tr);
+      group_sync<M>(g);                // (A) the previous transform's last pass has been read by all
+      pass_scatter<M, 0>(v, t, buf);
+    } else {
+      group_sync<M>(g);
+      pass_store<M, 0>(v, t, buf, p.tw);
+    }
+    // the frame is in registers: past (A) nobody reads the oldest ring slot any more
+    if (!GLB_RING_EXTRA && next_there && t == 0) request_next();
+    group_sync<M>(g);
+    RingMidPasses<M, 1, RT>::run(v, t, buf, tw_mid, tr, g);
+    float yv[17];
+    yv[16] = 0.f;
+    const bool w0 = t < 32;           // warp-uniform: only the warp that holds thread 0 pays for its re-ordering
+    if constexpr (RT) {
+      last_pass_rt<M>(v, t, buf, p.tw, tr);
+    } else {
+      TwRegs tl;
+      load_last_regs<M>(tl, t, p.tw, p.vtab);
+      last_pass_load<M>(v, t, buf);
+      last_pass_compute_rt<M>(v, t, tl);
+    }
+    if (w0) iq_emit_power<M, true>(v, t, kIqPowerScale, yv);
+    else iq_emit_power<M, false>(v, t, kIqPowerScale, yv);
+    if (active) {
+      GLB_CHECK_ROW(p, row_ptr);
+      GLB_CHECK_ROW(p, row_ptr + M - 1);
+#pragma unroll
+      for (int slot = 0; slot < 17; slot++) {
+        if (slot == 16) {
+          if (t == 0) st_row(row_ptr, yv[16]);
+        } else if (slot != 1 || t != 0) {
+          st_row(row_ptr + iq_slot_offset<M>(ob, slot), yv[slot]);
+        }
+      }
+    }
+    slot_new = slot_next;
+    // no barrier here: (A) of the next transform orders these reads of `buf` before its stores
+  }
+}
+
+// regular geometry, staged span covers every block of the launch, 16-byte aligned blocks: fused kernel.
+// Returns 1 when launched, 0 when the launch is not served, < 0 on error.
+template <int M>
+static int launch_iq_fused(const KParams &kp, cudaStream_t st) {
+  using GeoM = Geo<M>;
+  constexpr bool RT = RingGeo<M, false>::RT;
+  const int unit = 2 * GeoM::T;
+  int qs = -1;
+  for (int s2 = 0; s2 <= 4; s2++)
+    if (kp.hop == (unit << s2)) qs = s2;
+  if (qs < 0 || (kp.n_ov % kp.hop) != 0 || (kp.hop % 4) != 0 || (kp.origin % 4) != 0 ||
+      (reinterpret_cast<uintptr_t>(kp.samples) & 15) != 0)
+    return 0;
+  const long long blk_lo = (kp.first_frame - kp.n_ov / kp.hop) * (long long) kp.hop;
+  const long long blk_hi = (kp.first_frame + kp.nframes) * (long long) kp.hop;
+  if (!(kp.origin <= (blk_lo > 0 ? blk_lo : 0) && blk_hi <= kp.origin + kp.count)) return 0;
+  const RingLayout L = ring_layout<M>(kp.hop, kPoints >> qs);
+  const size_t smem = (size_t) GeoM::G * L.group_bytes + (RT ? 0 : Geo<M>::TWS_BYTES);
+  if (smem > 227 * 1024) return 0;
+  void (*rk)(const KParams) = qs == 3 ? gram_iq_kernel<M, 3> : (qs == 2 ? gram_iq_kernel<M, 2> : gram_iq_kernel<M, -1>);
+  int dev = 0, sms = 0;
+  CU(cudaGetDevice(&dev));
+  CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  static thread_local int occ_iq[5][64];
+  int &occ = occ_iq[qs][dev & 63];
+  if (occ == 0) {
+    CU(cudaFuncSetAttribute(rk, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, rk, GeoM::THREADS, smem));
+    if (occ < 1) occ = -1;
+  }
+  if (occ < 1) return 0;
+  // the launch policy of the real ring kernel (launch_gram_m): up to four waves of runs of >= 16 frames
+  long long groups = (long long) sms * occ * GeoM::G;
+  constexpr int kRingWaves = 4, kRingMinRun = 16;
+  if (occ >= 2) {
+    int waves = kRingWaves;
+    while (waves > 1 && kp.nframes < groups * waves * kRingMinRun) waves--;
+    groups *= waves;
+  }
+  if (groups > kp.nframes) groups = kp.nframes;
+  if (groups < 1) groups = 1;
+  KParams k = kp;
+  k.qs = qs;
+  k.frames_per_group = (int) ((kp.nframes + groups - 1) / groups);
+  const long long used = (kp.nframes + k.frames_per_group - 1) / k.frames_per_group;
+  const int ctas = (int) ((used + GeoM::G - 1) / GeoM::G);
+  rk<<<ctas, GeoM::THREADS, smem, st>>>(k);
+  CU(cudaGetLastError());
+  g_launches++;
+  g_last_family = 2;
+  return 1;
+}
+
+static int iq_fused_n(int n) { return n >= 32 && n <= 8192 && (n & (n - 1)) == 0; }
+
+static bool iq_fused_geometry(int n, int hop) {
+  if (!iq_fused_n(n) || hop < 1 || hop > n || (n - hop) % hop != 0) return false;
+  for (int s = 0; s <= 4; s++)
+    if (hop == ((n / 16) << s)) return true;
+  return false;
+}
+
+static bool iq_fused_allowed() { return g_force_generic == 0 && g_kernel_pref != 1; }
+
+extern "C" long long glb_iq_gram_scratch_bytes(int n, int hop, long long nframes) {
+  if (nframes <= 0 || (iq_fused_allowed() && iq_fused_geometry(n, hop))) return 0;
+  return nframes * (long long) (n + 1) * 2 * (long long) sizeof(float);
+}
+
+extern "C" int glb_launch_iq_gram(const glb_iq_gram_args *a, void *stream) {
+  if (!a || !a->tables || !a->samples || !a->taper || !a->rows || a->n < 32 || a->n > 16384 || (a->n & (a->n - 1)) != 0 ||
+      a->hop < 1 || a->hop > a->n || a->origin < 0 || a->count < 0 || a->first_frame < 0) {
+    glb_set_error("glb_launch_iq_gram: invalid arguments");
+    return GLB_EINVAL;
+  }
+  if (a->nframes <= 0) return GLB_OK;
+  int tn = 0;
+  const float2 *tw = nullptr, *vtab = nullptr;
+  if (glb_tables_get(a->tables, &tn, &tw, &vtab) != GLB_OK || tn != 2 * a->n) {
+    glb_set_error("glb_launch_iq_gram: tables must be built for 2 n");
+    return GLB_EINVAL;
+  }
+  if (iq_fused_allowed() && iq_fused_geometry(a->n, a->hop)) {
+    KParams k;
+    memset(&k, 0, sizeof k);
+    k.samples = a->samples;
+    k.origin = 2 * a->origin;
+    k.count = 2 * a->count;
+    k.tapers = a->taper;
+    k.ntapers = 1;
+    k.hop = 2 * a->hop;
+    k.n_ov = 2 * (a->n - a->hop);
+    k.first_frame = a->first_frame;
+    k.nframes = a->nframes;
+    k.rows = a->rows;
+    k.row_stride = a->n;
+    k.tw = tw;
+    k.vtab = vtab;
+    cudaStream_t st = (cudaStream_t) stream;
+    int rc = 0;
+    switch (a->n) {
+      case 32: rc = launch_iq_fused<32>(k, st); break;
+      case 64: rc = launch_iq_fused<64>(k, st); break;
+      case 128: rc = launch_iq_fused<128>(k, st); break;
+      case 256: rc = launch_iq_fused<256>(k, st); break;
+      case 512: rc = launch_iq_fused<512>(k, st); break;
+      case 1024: rc = launch_iq_fused<1024>(k, st); break;
+      case 2048: rc = launch_iq_fused<2048>(k, st); break;
+      case 4096: rc = launch_iq_fused<4096>(k, st); break;
+      case 8192: rc = launch_iq_fused<8192>(k, st); break;
+      default: break;
+    }
+    if (rc != 0) return rc < 0 ? rc : GLB_OK;
+  }
+  return glb_launch_iq_gram_general(a, stream);
+}

@@ -14,11 +14,14 @@
 //                         order, and the lane partials are summed in a fixed order through shared memory.
 //                         The sum order of an output therefore depends on D only, never on where the
 //                         output falls in a launch or chunk.  int16 input is converted in registers.
+//                         T = float2 / short2: complex (I, Q) input, four FMAs per tap in an order that
+//                         rounds exactly as the real kernel's when Q = 0.
 //   zoom_split_kernel     X[k], k = 0..Nz, of the interleaved (re, im) stream seen as 2 Nz real points ->
 //                         Z[k] = E + iO of the complex frame -> |Z|^2 / Nz in fft-shifted bin order.
 #include <cuda_runtime.h>
 #include <atomic>
 #include <cstdio>
+#include <cstring>
 #include "../../include/glb_shim.h"
 
 extern std::atomic<unsigned long long> g_launches;   // gram_kernels.cu
@@ -46,9 +49,21 @@ static __device__ __forceinline__ float zload(const float *x, long long i, long 
 static __device__ __forceinline__ float zload(const short *x, long long i, long long count) {
   return (i >= 0 && i < count) ? (float) __ldg(x + i) * (1.f / 32768.f) : 0.f;
 }
+// complex input: interleaved (I, Q) floats or int16 pairs, converted as above
+static __device__ __forceinline__ float2 zload(const float2 *x, long long i, long long count) {
+  return (i >= 0 && i < count) ? __ldg(x + i) : make_float2(0.f, 0.f);
+}
+static __device__ __forceinline__ float2 zload(const short2 *x, long long i, long long count) {
+  if (i < 0 || i >= count) return make_float2(0.f, 0.f);
+  const short2 s = __ldg(x + i);
+  return make_float2((float) s.x * (1.f / 32768.f), (float) s.y * (1.f / 32768.f));
+}
+template <typename T> struct ZComplex { static constexpr bool value = false; };
+template <> struct ZComplex<float2> { static constexpr bool value = true; };
+template <> struct ZComplex<short2> { static constexpr bool value = true; };
 
 template <typename T>
-__global__ void __launch_bounds__(kZWarps * 32)
+__global__ void __launch_bounds__(kZWarps * 32, ZComplex<T>::value ? 1 : 0)
 zoom_decim_kernel(const T *__restrict__ x, long long origin, long long count, int D, int LG, int G,
                   const float2 *__restrict__ taps, unsigned dstep, long long m_first, long long m_count,
                   float2 *__restrict__ y) {
@@ -77,13 +92,20 @@ zoom_decim_kernel(const T *__restrict__ x, long long origin, long long count, in
         const long long ip = i0 + p;
 #pragma unroll
         for (int q = 0; q < kZR + kZT - 1; q++) {
-          const float u = zload(x, ip + (long long) q * D, count);
+          const auto u = zload(x, ip + (long long) q * D, count);
 #pragma unroll
           for (int r = 0; r < kZR; r++) {
             const int t = q - r;
             if (t >= 0 && t < kZT) {
-              ar[r] = fmaf(tr[t], u, ar[r]);
-              ai[r] = fmaf(ti[t], u, ai[r]);
+              if constexpr (ZComplex<T>::value) {
+                ar[r] = fmaf(tr[t], u.x, ar[r]);
+                ar[r] = fmaf(-ti[t], u.y, ar[r]);
+                ai[r] = fmaf(ti[t], u.x, ai[r]);
+                ai[r] = fmaf(tr[t], u.y, ai[r]);
+              } else {
+                ar[r] = fmaf(tr[t], u, ar[r]);
+                ai[r] = fmaf(ti[t], u, ai[r]);
+              }
             }
           }
         }
@@ -170,6 +192,18 @@ extern "C" int glb_launch_zoom_decim(const void *x, int pcm16, long long origin,
   return launch_decim((const float *) x, origin, count, decim, taps, dstep, m_first, m_count, y, stream);
 }
 
+extern "C" int glb_launch_zoom_decim_iq(const void *x, int pcm16, long long origin, long long count, int decim,
+                                        const void *taps, unsigned dstep, long long m_first, long long m_count,
+                                        void *y, void *stream) {
+  if (decim < 2 || decim > 1024 || !taps || !y || origin < 0 || count < 0 || m_first < 0) {
+    glb_set_error("glb_launch_zoom_decim_iq: invalid arguments");
+    return GLB_EINVAL;
+  }
+  if (m_count <= 0) return GLB_OK;
+  if (pcm16) return launch_decim((const short2 *) x, origin, count, decim, taps, dstep, m_first, m_count, y, stream);
+  return launch_decim((const float2 *) x, origin, count, decim, taps, dstep, m_first, m_count, y, stream);
+}
+
 extern "C" int glb_launch_zoom_split(const void *spec, int nz, long long nframes, float *rows, void *stream) {
   if (nz < 2 || (nz & (nz - 1)) != 0 || !spec || !rows) {
     glb_set_error("glb_launch_zoom_split: invalid arguments");
@@ -185,4 +219,38 @@ extern "C" int glb_launch_zoom_split(const void *spec, int nz, long long nframes
   ZCU(cudaGetLastError());
   g_launches++;
   return GLB_OK;
+}
+
+// The general path of complex frames: the interleaved stream seen as a real stream of 2n floats per frame at hop
+// 2 hop, the general spectrogram kernel's spectrum output X[k], k = 0..n, then zoom_split_kernel.  The zoom's frame
+// stage (host/zoom.c) and the I/Q spectrogram's non-fused launches (iq.cu).
+extern "C" int glb_launch_iq_gram_general(const glb_iq_gram_args *a, void *stream) {
+  if (!a || !a->rows || a->nframes < 0) {
+    glb_set_error("glb_launch_iq_gram_general: invalid arguments");
+    return GLB_EINVAL;
+  }
+  if (a->nframes == 0) return GLB_OK;
+  if (!a->scratch) {
+    glb_set_error("glb_launch_iq_gram_general: needs scratch for the spectrum (glb_iq_gram_scratch_bytes)");
+    return GLB_EINVAL;
+  }
+  glb_gram_args g;
+  memset(&g, 0, sizeof g);
+  g.n = 2 * a->n;
+  g.hop = 2 * a->hop;
+  g.samples = a->samples;
+  g.origin = 2 * a->origin;
+  g.count = 2 * a->count;
+  g.tapers = a->taper;
+  g.ntapers = 1;
+  g.taper_symmetric = a->taper_symmetric;
+  g.taper_scale = a->taper_scale;
+  g.first_frame = a->first_frame;
+  g.nframes = a->nframes;
+  g.spectrum = (float *) a->scratch;
+  g.tables = a->tables;
+  g.general_only = 1;
+  int rc = glb_launch_gram(&g, stream);
+  if (rc != GLB_OK) return rc;
+  return glb_launch_zoom_split(a->scratch, a->n, a->nframes, a->rows, stream);
 }

@@ -1,0 +1,245 @@
+/* iq.c -- I/Q spectrogram plans: two-sided rows of complex (SDR baseband) recordings (include/glfer_b200.h).
+ *
+ * The frames of an interleaved (I, Q) stream are complex FFT frames of n samples; one shim entry,
+ * glb_launch_iq_gram (csrc/iq.cu), computes their rows on whichever path serves the geometry (the fused ring
+ * kernel, or the general kernel followed by the zoom's split).  This file only moves data: a run walks the frames
+ * in chunks of ~32 MiB of input on ISLOT streams, each chunk uploads its complex samples (the n - hop samples it
+ * shares with the previous chunk again), converts int16 input to float on the device, computes its rows and copies
+ * them back while the next chunk uploads.  Device memory is bounded by the chunk, not by the recording.
+ */
+#include <math.h>
+#include <stdlib.h>
+#include <string.h>
+#include "glb_host.h"
+
+#define ISLOT 3
+
+#define ITRY(x) do { int rc_ = glb_host_shim(x); if (rc_ != 0) return rc_; } while (0)
+
+typedef struct {
+  void *stream;
+  short *d_pcm;               /* int16 input of the chunk */
+  size_t pcm_cap;             /* shorts */
+  float *d_in;                /* interleaved (I, Q) floats of the chunk */
+  size_t in_cap;              /* floats */
+  float *d_rows;
+  size_t rows_cap;            /* floats */
+  void *d_scratch;
+  size_t scratch_cap;         /* bytes */
+} islot;
+
+struct glfer_iq_plan {
+  glfer_iq_config cfg;
+  int hop;
+  float *d_taper;             /* [2n]: w[i] on both halves of complex sample i, times taper_scale */
+  int taper_sym;
+  float taper_scale;
+  void *tables;               /* FFT tables of the 2n-float frames */
+  islot slot[ISLOT];
+};
+
+void glfer_iq_config_default(glfer_iq_config *c)
+{
+  memset(c, 0, sizeof *c);
+  c->n = 4096;
+  c->window_type = HANNING_WINDOW;
+  c->overlap = 0.5f;
+  c->device = 0;
+}
+
+int glfer_iq_hop(const glfer_iq_plan *p) { return p->hop; }
+int glfer_iq_bins(const glfer_iq_plan *p) { return p->cfg.n; }
+
+long long glfer_iq_num_frames(const glfer_iq_plan *p, long long nsamples)
+{
+  return nsamples <= 0 ? 0 : nsamples / p->hop;
+}
+
+void glfer_iq_required_span(const glfer_iq_plan *p, long long first_frame, long long nframes, long long *lo,
+                            long long *hi)
+{
+  *lo = first_frame * p->hop - (p->cfg.n - p->hop);
+  *hi = (first_frame + nframes) * p->hop;
+}
+
+void glfer_iq_plan_destroy(glfer_iq_plan *p)
+{
+  if (!p) return;
+  glb_set_device(p->cfg.device);
+  for (int i = 0; i < ISLOT; i++) {
+    islot *s = &p->slot[i];
+    if (s->stream) glb_stream_sync(s->stream);
+    glb_free(s->d_pcm); glb_free(s->d_in); glb_free(s->d_rows); glb_free(s->d_scratch);
+    glb_stream_destroy(s->stream);
+  }
+  glb_free(p->d_taper);
+  glb_tables_destroy(p->tables);
+  free(p);
+}
+
+static int build_taper(glfer_iq_plan *p)
+{
+  const int n = p->cfg.n;
+  float *w = malloc(sizeof(float) * n);
+  float *taper = malloc(sizeof(float) * 2 * n);
+  int rc = 0;
+  if (!w || !taper) rc = glb_host_fail(GLFER_ENOMEM, "out of memory");
+  if (rc == 0) {
+    /* as the zoom (host/zoom.c): the window on both floats of a complex sample, times 1 / (2 sqrt(2n)) */
+    glb_window_table(n, p->cfg.window_type, w);
+    p->taper_scale = (float) (1.0 / (2.0 * sqrt(2.0 * n)));
+    for (int i = 0; i < n; i++) {
+      const double wi = p->cfg.window_type == RECTANGULAR_WINDOW ? 1.0 : (double) w[i];
+      taper[2 * i] = taper[2 * i + 1] = (float) (wi * (double) p->taper_scale);
+    }
+    p->taper_sym = 1;
+    for (int i = 0; i < n; i++)
+      if (memcmp(&taper[i], &taper[2 * n - 1 - i], sizeof(float)) != 0) { p->taper_sym = 0; break; }
+    rc = glb_host_shim(glb_malloc((void **) &p->d_taper, sizeof(float) * 2 * (size_t) n));
+    if (rc == 0) rc = glb_host_shim(glb_memcpy_h2d(p->d_taper, taper, sizeof(float) * 2 * (size_t) n, NULL));
+    if (rc == 0) rc = glb_host_shim(glb_tables_create(2 * n, &p->tables));
+  }
+  free(w); free(taper);
+  return rc;
+}
+
+int glfer_iq_plan_create(const glfer_iq_config *cfg, glfer_iq_plan **out)
+{
+  glb_host_clear_error();
+  if (!cfg || !out) return glb_host_fail(GLFER_EINVAL, "null argument");
+  *out = NULL;
+  if (cfg->n < 32 || cfg->n > 16384 || (cfg->n & (cfg->n - 1)) != 0)
+    return glb_host_fail(GLFER_EINVAL, "I/Q FFT size must be a power of two in 32..16384");
+  if (cfg->window_type < 0 || cfg->window_type > 7) return glb_host_fail(GLFER_EINVAL, "unknown window type");
+  const int hop = glb_hop(cfg->n, cfg->overlap);
+  if (hop < 1 || hop > cfg->n) return glb_host_fail(GLFER_EINVAL, "overlap leaves no new samples per block");
+  int ndev = 0;
+  if (glb_device_count(&ndev) != GLB_OK || ndev < 1)
+    return glb_host_fail(GLFER_ENODEV, "no CUDA device (libglfer_b200 has no CPU fallback)");
+  if (cfg->device < 0 || cfg->device >= ndev) return glb_host_fail(GLFER_EINVAL, "device ordinal out of range");
+  ITRY(glb_set_device(cfg->device));
+
+  glfer_iq_plan *p = calloc(1, sizeof *p);
+  if (!p) return glb_host_fail(GLFER_ENOMEM, "out of memory");
+  p->cfg = *cfg;
+  p->hop = hop;
+  int rc = build_taper(p);
+  for (int i = 0; i < ISLOT && rc == 0; i++) rc = glb_host_shim(glb_stream_create(&p->slot[i].stream));
+  if (rc != 0) {
+    char keep[512];
+    strncpy(keep, glfer_b200_last_error(), sizeof keep - 1);
+    keep[sizeof keep - 1] = 0;
+    glfer_iq_plan_destroy(p);
+    glb_host_fail(rc, keep);
+    return rc;
+  }
+  *out = p;
+  return GLFER_OK;
+}
+
+/* grow-only device buffers */
+static int iensure(void **ptr, size_t *cap, size_t want, size_t elem)
+{
+  if (want <= *cap) return 0;
+  if (*ptr) ITRY(glb_free(*ptr));
+  *ptr = NULL;
+  *cap = 0;
+  ITRY(glb_malloc(ptr, want * elem));
+  *cap = want;
+  return 0;
+}
+
+static long long iq_chunk_frames(const glfer_iq_plan *p)
+{
+  /* ~32 MiB of new float input per chunk, as the spectrogram's and the zoom's pipelines; at least one frame */
+  const long long f = (32LL << 20) / ((long long) p->hop * 8);
+  return f < 1 ? 1 : f;
+}
+
+/* frames [c0, c0 + cn) on slot s */
+static int iq_chunk(glfer_iq_plan *p, islot *s, const void *src, int pcm16, long long origin, long long c0,
+                    long long cn, float *rows)
+{
+  const long long n = p->cfg.n, hop = p->hop;
+  long long lo = c0 * hop - (n - hop);
+  const long long hi = (c0 + cn) * hop;
+  if (lo < 0) lo = 0;
+  /* the fused kernel reads whole hop blocks with 16-byte bulk copies: stage from an even complex index when the
+     caller's samples reach that far back (the regular hops are even, so lo already is) */
+  if ((lo & 1) && lo - 1 >= origin) lo--;
+  const long long cnt = hi - lo;
+  ITRY(iensure((void **) &s->d_in, &s->in_cap, (size_t) (2 * cnt), sizeof(float)));
+  if (pcm16) {
+    ITRY(iensure((void **) &s->d_pcm, &s->pcm_cap, (size_t) (2 * cnt), sizeof(short)));
+    ITRY(glb_memcpy_h2d(s->d_pcm, (const short *) src + 2 * (lo - origin), sizeof(short) * 2 * (size_t) cnt, s->stream));
+    ITRY(glb_launch_pcm16_to_float(s->d_pcm, s->d_in, 2 * cnt, s->stream));
+  } else {
+    ITRY(glb_memcpy_h2d(s->d_in, (const float *) src + 2 * (lo - origin), sizeof(float) * 2 * (size_t) cnt, s->stream));
+  }
+  ITRY(iensure((void **) &s->d_rows, &s->rows_cap, (size_t) (cn * n), sizeof(float)));
+  const long long sb = glb_iq_gram_scratch_bytes((int) n, (int) hop, cn);
+  if (sb > 0) ITRY(iensure(&s->d_scratch, &s->scratch_cap, (size_t) sb, 1));
+  glb_iq_gram_args g;
+  memset(&g, 0, sizeof g);
+  g.n = (int) n;
+  g.hop = (int) hop;
+  g.samples = s->d_in;
+  g.origin = lo;
+  g.count = cnt;
+  g.taper = p->d_taper;
+  g.taper_symmetric = p->taper_sym;
+  g.taper_scale = p->taper_scale;
+  g.first_frame = c0;
+  g.nframes = cn;
+  g.rows = s->d_rows;
+  g.tables = p->tables;
+  g.scratch = sb > 0 ? s->d_scratch : NULL;
+  ITRY(glb_launch_iq_gram(&g, s->stream));
+  ITRY(glb_memcpy_d2h(rows, s->d_rows, sizeof(float) * (size_t) (cn * n), s->stream));
+  return 0;
+}
+
+static int iq_run_impl(glfer_iq_plan *p, const void *src, int pcm16, long long origin, long long count,
+                       long long first_frame, long long nframes, float *rows)
+{
+  glb_host_clear_error();
+  if (!p || !src || !rows) return glb_host_fail(GLFER_EINVAL, "null argument");
+  if (nframes < 0 || first_frame < 0) return glb_host_fail(GLFER_EINVAL, "negative frame range");
+  if (origin < 0 || count < 0) return glb_host_fail(GLFER_EINVAL, "negative origin or sample count");
+  if (nframes == 0) return 0;
+  ITRY(glb_set_device(p->cfg.device));
+  long long lo, hi;
+  glfer_iq_required_span(p, first_frame, nframes, &lo, &hi);
+  if (lo < 0) lo = 0;
+  if (lo < origin || hi > origin + count)
+    return glb_host_fail(GLFER_EINVAL, "samples do not cover the requested frames (see glfer_iq_required_span)");
+  const long long cf = iq_chunk_frames(p);
+  int rc = 0, ci = 0;
+  long long done = 0;
+  while (done < nframes && rc == 0) {
+    islot *s = &p->slot[ci % ISLOT];
+    const long long cn = (nframes - done < cf) ? nframes - done : cf;
+    rc = glb_host_shim(glb_stream_sync(s->stream));
+    if (rc) break;
+    rc = iq_chunk(p, s, src, pcm16, origin, first_frame + done, cn, rows + (size_t) done * p->cfg.n);
+    done += cn;
+    ci++;
+  }
+  for (int i = 0; i < ISLOT; i++) {
+    const int r2 = glb_host_shim(glb_stream_sync(p->slot[i].stream));
+    if (rc == 0) rc = r2;
+  }
+  return rc;
+}
+
+int glfer_iq_run(glfer_iq_plan *p, const float *iq, long long origin, long long count, long long first_frame,
+                 long long nframes, float *rows)
+{
+  return iq_run_impl(p, iq, 0, origin, count, first_frame, nframes, rows);
+}
+
+int glfer_iq_run_pcm16(glfer_iq_plan *p, const short *iq, long long origin, long long count, long long first_frame,
+                       long long nframes, float *rows)
+{
+  return iq_run_impl(p, iq, 1, origin, count, first_frame, nframes, rows);
+}

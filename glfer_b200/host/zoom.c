@@ -10,6 +10,9 @@
  * of its new decimated samples (plus the 2K-sample filter halo) and takes the n - hop decimated samples its
  * first frame shares with the previous chunk from that chunk's buffer, device to device: every input sample
  * crosses PCIe once, and device memory is bounded by the chunk, not by the recording.
+ *
+ * I/Q plans (glfer_zoom_plan_create_iq) take complex input, interleaved (I, Q), through the complex decimator
+ * (glb_launch_zoom_decim_iq) and accept a signed centre; everything after the decimator is the same.
  */
 #include <math.h>
 #include <stdlib.h>
@@ -41,6 +44,7 @@ struct glfer_zoom_plan {
   float *d_taper;             /* [2n]: w[i] on both halves of complex sample i, times taper_scale */
   int taper_sym;
   float taper_scale;
+  int iq;                     /* 1: complex (I, Q) input (glfer_zoom_plan_create_iq), signed centre */
   void *tables;               /* FFT tables of the 2n-point real transform */
   zslot slot[ZSLOT];
 };
@@ -96,7 +100,12 @@ void glfer_zoom_config_default(glfer_zoom_config *c)
 
 int glfer_zoom_hop(const glfer_zoom_plan *p) { return p->hop; }
 int glfer_zoom_bins(const glfer_zoom_plan *p) { return p->cfg.n; }
-double glfer_zoom_center_hz(const glfer_zoom_plan *p) { return (double) p->step * p->cfg.sample_rate / 4294967296.0; }
+double glfer_zoom_center_hz(const glfer_zoom_plan *p)
+{
+  /* an I/Q plan's step is a signed 32-bit fraction of a turn: centres below the dial are negative */
+  const double s = p->iq ? (double) (int) p->step : (double) p->step;
+  return s * p->cfg.sample_rate / 4294967296.0;
+}
 
 long long glfer_zoom_num_frames(const glfer_zoom_plan *p, long long nsamples)
 {
@@ -171,7 +180,7 @@ static int build_tables(glfer_zoom_plan *p)
   return rc;
 }
 
-int glfer_zoom_plan_create(const glfer_zoom_config *cfg, glfer_zoom_plan **out)
+static int zoom_plan_create(const glfer_zoom_config *cfg, int iq, glfer_zoom_plan **out)
 {
   glb_host_clear_error();
   if (!cfg || !out) return glb_host_fail(GLFER_EINVAL, "null argument");
@@ -183,8 +192,10 @@ int glfer_zoom_plan_create(const glfer_zoom_config *cfg, glfer_zoom_plan **out)
   const int hop = glb_hop(cfg->n, cfg->overlap);
   if (hop < 1 || hop > cfg->n) return glb_host_fail(GLFER_EINVAL, "overlap leaves no new samples per block");
   if (!(cfg->sample_rate > 0.0) || !isfinite(cfg->sample_rate)) return glb_host_fail(GLFER_EINVAL, "sample rate must be positive");
-  if (!(cfg->center_hz >= 0.0 && cfg->center_hz <= 0.5 * cfg->sample_rate))
+  if (!iq && !(cfg->center_hz >= 0.0 && cfg->center_hz <= 0.5 * cfg->sample_rate))
     return glb_host_fail(GLFER_EINVAL, "centre frequency must be in [0, sample_rate / 2]");
+  if (iq && !(cfg->center_hz >= -0.5 * cfg->sample_rate && cfg->center_hz <= 0.5 * cfg->sample_rate))
+    return glb_host_fail(GLFER_EINVAL, "I/Q centre frequency must be in [-sample_rate / 2, sample_rate / 2]");
   int ndev = 0;
   if (glb_device_count(&ndev) != GLB_OK || ndev < 1)
     return glb_host_fail(GLFER_ENODEV, "no CUDA device (libglfer_b200 has no CPU fallback)");
@@ -196,7 +207,9 @@ int glfer_zoom_plan_create(const glfer_zoom_config *cfg, glfer_zoom_plan **out)
   p->cfg = *cfg;
   p->hop = hop;
   p->K = 16 * cfg->decim;
-  p->step = (unsigned) llround(cfg->center_hz / cfg->sample_rate * 4294967296.0);
+  p->iq = iq;
+  /* modulo 2^32: a negative I/Q centre is a step above 2^31 */
+  p->step = (unsigned) (unsigned long long) llround(cfg->center_hz / cfg->sample_rate * 4294967296.0);
   int rc = build_tables(p);
   for (int i = 0; i < ZSLOT && rc == 0; i++) {
     rc = glb_host_shim(glb_stream_create(&p->slot[i].stream));
@@ -214,6 +227,16 @@ int glfer_zoom_plan_create(const glfer_zoom_config *cfg, glfer_zoom_plan **out)
   return GLFER_OK;
 }
 
+int glfer_zoom_plan_create(const glfer_zoom_config *cfg, glfer_zoom_plan **out)
+{
+  return zoom_plan_create(cfg, 0, out);
+}
+
+int glfer_zoom_plan_create_iq(const glfer_zoom_config *cfg, glfer_zoom_plan **out)
+{
+  return zoom_plan_create(cfg, 1, out);
+}
+
 /* grow-only device buffers */
 static int zensure(void **ptr, size_t *cap, size_t want, size_t elem)
 {
@@ -229,7 +252,7 @@ static int zensure(void **ptr, size_t *cap, size_t want, size_t elem)
 static long long zoom_chunk_frames(const glfer_zoom_plan *p)
 {
   /* ~32 MiB of new float input per chunk, as the spectrogram's pipeline; at least one frame */
-  const long long per_frame = (long long) p->hop * p->cfg.decim * 4;
+  const long long per_frame = (long long) p->hop * p->cfg.decim * (p->iq ? 8 : 4);
   const long long f = (32LL << 20) / per_frame;
   return f < 1 ? 1 : f;
 }
@@ -253,7 +276,7 @@ static int zoom_chunk(glfer_zoom_plan *p, zslot *s, const zslot *prev, const voi
   long long x_lo = from * D - p->K;
   const long long x_hi = (m_hi - 1) * D + p->K + 1;
   if (x_lo < 0) x_lo = 0;
-  const size_t esz = pcm16 ? sizeof(short) : sizeof(float);
+  const size_t esz = (pcm16 ? sizeof(short) : sizeof(float)) * (p->iq ? 2 : 1);
   ZTRY(zensure(&s->d_in, &s->in_cap, (size_t) (x_hi - x_lo) * esz, 1));
   ZTRY(glb_memcpy_h2d(s->d_in, (const char *) src + (size_t) (x_lo - origin) * esz, (size_t) (x_hi - x_lo) * esz,
                       s->stream));
@@ -263,42 +286,48 @@ static int zoom_chunk(glfer_zoom_plan *p, zslot *s, const zslot *prev, const voi
     ZTRY(glb_memcpy_d2d(s->d_y, prev->d_y + 2 * (base - prev->y_base), (size_t) (from - base) * 2 * sizeof(float),
                         s->stream));
   }
-  ZTRY(glb_launch_zoom_decim(s->d_in, pcm16, x_lo, x_hi - x_lo, (int) D, p->d_taps,
-                             (unsigned) ((unsigned long long) D * p->step), from, m_hi - from,
-                             s->d_y + 2 * (from - base), s->stream));
+  if (p->iq)
+    ZTRY(glb_launch_zoom_decim_iq(s->d_in, pcm16, x_lo, x_hi - x_lo, (int) D, p->d_taps,
+                                  (unsigned) ((unsigned long long) D * p->step), from, m_hi - from,
+                                  s->d_y + 2 * (from - base), s->stream));
+  else
+    ZTRY(glb_launch_zoom_decim(s->d_in, pcm16, x_lo, x_hi - x_lo, (int) D, p->d_taps,
+                               (unsigned) ((unsigned long long) D * p->step), from, m_hi - from,
+                               s->d_y + 2 * (from - base), s->stream));
   ZTRY(glb_event_record(s->ev_dec, s->stream));
   s->y_base = base;
   s->y_end = m_hi;
 
   ZTRY(zensure((void **) &s->d_spec, &s->spec_cap, (size_t) cn * (n + 1) * 2, sizeof(float)));
   ZTRY(zensure((void **) &s->d_rows, &s->rows_cap, (size_t) cn * n, sizeof(float)));
-  glb_gram_args g;
+  glb_iq_gram_args g;
   memset(&g, 0, sizeof g);
-  g.n = (int) (2 * n);
-  g.hop = (int) (2 * hop);
+  g.n = (int) n;
+  g.hop = (int) hop;
   g.samples = s->d_y;
-  g.origin = 2 * base;
-  g.count = 2 * (m_hi - base);
-  g.tapers = p->d_taper;
-  g.ntapers = 1;
+  g.origin = base;
+  g.count = m_hi - base;
+  g.taper = p->d_taper;
   g.taper_symmetric = p->taper_sym;
   g.taper_scale = p->taper_scale;
   g.first_frame = c0;
   g.nframes = cn;
-  g.spectrum = s->d_spec;
+  g.rows = s->d_rows;
   g.tables = p->tables;
-  g.general_only = 1;
-  ZTRY(glb_launch_gram(&g, s->stream));
-  ZTRY(glb_launch_zoom_split(s->d_spec, (int) n, cn, s->d_rows, s->stream));
+  g.scratch = s->d_spec;
+  ZTRY(glb_launch_iq_gram_general(&g, s->stream));
   ZTRY(glb_memcpy_d2h(rows, s->d_rows, sizeof(float) * (size_t) cn * n, s->stream));
   return 0;
 }
 
-static int zoom_run_impl(glfer_zoom_plan *p, const void *src, int pcm16, long long origin, long long count,
+static int zoom_run_impl(glfer_zoom_plan *p, int iq, const void *src, int pcm16, long long origin, long long count,
                          long long first_frame, long long nframes, float *rows)
 {
   glb_host_clear_error();
   if (!p || !src || !rows) return glb_host_fail(GLFER_EINVAL, "null argument");
+  if (iq != p->iq)
+    return glb_host_fail(GLFER_EINVAL, iq ? "glfer_zoom_run_iq needs a plan from glfer_zoom_plan_create_iq"
+                                          : "an I/Q zoom plan runs through glfer_zoom_run_iq / glfer_zoom_run_iq_pcm16");
   if (nframes < 0 || first_frame < 0) return glb_host_fail(GLFER_EINVAL, "negative frame range");
   if (origin < 0 || count < 0) return glb_host_fail(GLFER_EINVAL, "negative origin or sample count");
   if (nframes == 0) return 0;
@@ -332,11 +361,23 @@ static int zoom_run_impl(glfer_zoom_plan *p, const void *src, int pcm16, long lo
 int glfer_zoom_run(glfer_zoom_plan *p, const float *samples, long long origin, long long count,
                    long long first_frame, long long nframes, float *rows)
 {
-  return zoom_run_impl(p, samples, 0, origin, count, first_frame, nframes, rows);
+  return zoom_run_impl(p, 0, samples, 0, origin, count, first_frame, nframes, rows);
 }
 
 int glfer_zoom_run_pcm16(glfer_zoom_plan *p, const short *pcm, long long origin, long long count,
                          long long first_frame, long long nframes, float *rows)
 {
-  return zoom_run_impl(p, pcm, 1, origin, count, first_frame, nframes, rows);
+  return zoom_run_impl(p, 0, pcm, 1, origin, count, first_frame, nframes, rows);
+}
+
+int glfer_zoom_run_iq(glfer_zoom_plan *p, const float *iq, long long origin, long long count,
+                      long long first_frame, long long nframes, float *rows)
+{
+  return zoom_run_impl(p, 1, iq, 0, origin, count, first_frame, nframes, rows);
+}
+
+int glfer_zoom_run_iq_pcm16(glfer_zoom_plan *p, const short *iq, long long origin, long long count,
+                            long long first_frame, long long nframes, float *rows)
+{
+  return zoom_run_impl(p, 1, iq, 1, origin, count, first_frame, nframes, rows);
 }

@@ -75,6 +75,34 @@ def tiled_stream(nsamples: int, fs: int = 48000, block_s: float = 60.0, seed: in
     return np.tile(blk, reps)[:nsamples]
 
 
+def iq_stream_int16(nsamples: int, fs: int = 48000, seed: int = 0x5EED, dot_s: float = 3.0,
+                    noise_sigma: float = 0.03) -> np.ndarray:
+    """A complex (I/Q) QRSS-like recording centred on the dial frequency, [nsamples, 2] int16 (I, Q): a keyed QRSS
+    carrier at -300 Hz below the dial, a DFCW pair at +400 / +410 Hz above it, steady weak carriers on both sides
+    (-1000, +150, +1200 Hz), a small LO-leakage offset at DC and complex Gaussian noise.  Offsets scale with fs
+    below 4 kHz so the tones stay in band."""
+    rng = np.random.Generator(np.random.Philox(seed))
+    t = np.arange(nsamples, dtype=np.float64) / fs
+    sc = 1.0 if fs >= 4000 else fs / 4000.0
+    z = noise_sigma / np.sqrt(2.0) * (rng.standard_normal(nsamples) + 1j * rng.standard_normal(nsamples))
+    gate, sel = _keying("GLFER ", nsamples, fs, dot_s)
+    z += 0.02 * gate * np.exp(1j * (2 * np.pi * (-300.0 * sc) * t + 0.3))
+    fd = (400.0 + 10.0 * sel) * sc
+    z += 0.01 * np.exp(1j * (2 * np.pi * np.cumsum(fd) / fs + 1.1))
+    for fc, amp, ph in ((-1000.0, 0.003, 0.0), (150.0, 0.01, 0.7), (1200.0, 0.03, 2.1)):
+        z += amp * np.exp(1j * (2 * np.pi * fc * sc * t + ph))
+    z += 0.002 - 0.001j
+    pcm = np.stack([z.real, z.imag], axis=1)
+    return np.clip(np.rint(pcm * 32768.0), -32768, 32767).astype(np.int16)
+
+
+def iq_stream(nsamples: int, fs: int = 48000, seed: int = 0x5EED, dot_s: float = 3.0,
+              noise_sigma: float = 0.03) -> np.ndarray:
+    """iq_stream_int16 as complex64 [nsamples] (I + iQ, each (float) s / 32768)"""
+    pcm = pcm16_to_float(iq_stream_int16(nsamples, fs, seed, dot_s, noise_sigma))
+    return np.ascontiguousarray(pcm).view(np.complex64)[:, 0]
+
+
 def write_wav16(path: str, pcm: np.ndarray, fs: int, channels: int = 1) -> None:
     """Canonical 44-byte-header 16-bit PCM WAV (the layout wav_fmt.h:34-52 describes); pcm is the interleaved
     sample stream ([frames][channels] flattened)."""

@@ -195,7 +195,7 @@ int glb_launch_levels(const float *rows, long long stride, int nbins, long long 
 int glb_launch_ftest(const float *spec, long long nframes, int nbins, int n, int ntapers, const double *u0,
                      double sum_u0_sqr, float *ftest, long long stride, void *stream);
 
-/* Zoom spectrogram (glfer_b200/csrc/zoom.cu).
+/* Zoom spectrogram (glfer_b200/csrc/zoom.cu) and I/Q spectrogram (glfer_b200/csrc/iq.cu).
  * Decimator: y[m - m_first] = e^{-2 pi i (m dstep mod 2^32) / 2^32} sum_{j=0..32 decim} taps[j] x[m decim - 16 decim + j]
  * for m in [m_first, m_first + m_count); taps: device, [33 decim] (re, im) pairs, zero past index 32 decim;
  * dstep = decim * phase step mod 2^32.  x (float, or int16 PCM when pcm16 = 1, converted as wav_fmt.c:113) holds
@@ -205,11 +205,44 @@ int glb_launch_zoom_decim(const void *x, int pcm16, long long origin, long long 
 /* rows[f][j] = |Z_f[(j + nz/2) mod nz]|^2 / nz, with Z_f the complex FFT recovered from spec = [nframes][nz + 1]
  * (re, im) pairs, the real FFT of frame f's interleaved (re, im) samples as 2 nz real points */
 int glb_launch_zoom_split(const void *spec, int nz, long long nframes, float *rows, void *stream);
+/* Decimator of complex input: as glb_launch_zoom_decim with x the complex stream, interleaved (I, Q) floats, or
+ * (I, Q) int16 PCM when pcm16 = 1; origin and count in complex samples.  Per tap the sum runs
+ *     ar = fma(tr, ur, ar); ar = fma(-ti, ui, ar); ai = fma(ti, ur, ai); ai = fma(tr, ui, ai),
+ * so with Q = 0 every output is bit-identical to glb_launch_zoom_decim's of I. */
+int glb_launch_zoom_decim_iq(const void *x, int pcm16, long long origin, long long count, int decim, const void *taps,
+                             unsigned dstep, long long m_first, long long m_count, void *y, void *stream);
+
+/* Rows of complex frames (I/Q spectrogram, zoom frame stage) of an interleaved (I, Q) stream z:
+ *     rows[f - first_frame][j] = |sum_i w[i] z[f hop - (n - hop) + i] e^{-2 pi i (j - n/2) i / n}|^2 / n
+ * The taper holds w[i] taper_scale on both floats of complex sample i, with taper_scale = (float) (1 / (2 sqrt(2 n)))
+ * (the fused kernel folds 1 / (n taper_scale^2) = 8 into its epilogue). */
+typedef struct {
+  int n;                       /* complex frame length: power of two, 32..16384 */
+  int hop;                     /* complex samples per frame */
+  const float *samples;        /* device: interleaved (I, Q) of complex samples [origin, origin + count) */
+  long long origin, count;     /* complex samples; indices < 0 read as 0 */
+  const float *taper;          /* device: [2n] floats */
+  int taper_symmetric;         /* taper[i] == taper[2n - 1 - i] bit for bit */
+  float taper_scale;
+  long long first_frame, nframes;
+  float *rows;                 /* device out: [nframes][n] */
+  const void *tables;          /* glb_tables_create(2 n) */
+  void *scratch;               /* device: glb_iq_gram_scratch_bytes() bytes, or NULL when that is 0 */
+} glb_iq_gram_args;
+/* The one entry of the I/Q spectrogram: the fused kernel (iq.cu, regular geometry n = 32..8192, hop = (n/16) << s
+ * with n - hop a multiple of hop; needs an even origin, a 16-byte aligned samples pointer and samples that cover
+ * every frame's blocks) or, for any other launch or under glb_force_generic_kernel(1), the general path below. */
+int glb_launch_iq_gram(const glb_iq_gram_args *a, void *stream);
+/* device scratch glb_launch_iq_gram needs for nframes frames (0 when the fused kernel serves the geometry) */
+long long glb_iq_gram_scratch_bytes(int n, int hop, long long nframes);
+/* the general path: the general spectrogram kernel's spectrum output on the 2n-float frames (into scratch, at
+ * least nframes (n + 1) (re, im) pairs), then glb_launch_zoom_split */
+int glb_launch_iq_gram_general(const glb_iq_gram_args *a, void *stream);
 
 /* counters */
 unsigned long long glb_kernel_launches(void);
-/* family of the last spectrogram kernel launched: 1 general, 2 TMA ring, 3 warp-per-frame, 4 two frames per thread,
- * 5 32 points per thread */
+/* family of the last spectrogram kernel launched: 1 general, 2 TMA ring (or its I/Q form, gram_iq_kernel), 3 warp-per-frame,
+ * 4 two frames per thread, 5 32 points per thread */
 int glb_last_kernel_family(void);
 
 #ifdef __cplusplus

@@ -251,6 +251,53 @@ int glfer_zoom_run_pcm16(glfer_zoom_plan *plan, const short *pcm, long long orig
 /* the low-pass filter h[l], l = -K..K, as taps[l + K] (32 decim + 1 floats); host only, needs no device */
 int glfer_zoom_taps(int decim, float *taps);
 
+/* ---- complex (I/Q) input: SDR baseband recordings ----
+ * An I/Q stream is interleaved: iq[2s] is I and iq[2s + 1] is Q of complex sample s, z[s] = I + iQ; origin and
+ * count are in complex samples.  The pcm16 forms take the data chunk of a 16-bit stereo WAV exactly as
+ * glfer_wav_load returns it (I on the left channel, Q on the right), with count = wav.nsamples / 2; samples are
+ * converted as the mono reader does ((float) s / 32768).  Frequencies are relative to the recording's centre (the
+ * receiver's dial frequency): negative below it, positive above. */
+
+/* I/Q zoom: the zoom above with complex x, no mirror image.  The centre may be anywhere in
+ * [-sample_rate / 2, sample_rate / 2]; step = (uint32) llround(center_hz / sample_rate 2^32), modulo 2^32, and
+ * glfer_zoom_center_hz of an I/Q plan reads the step as a signed 32-bit value.  The clean span is again
+ * |f - center| <= 0.4 sample_rate / D.  Real entry points reject I/Q plans and the reverse (GLFER_EINVAL). */
+int glfer_zoom_plan_create_iq(const glfer_zoom_config *cfg, glfer_zoom_plan **plan);
+int glfer_zoom_run_iq(glfer_zoom_plan *plan, const float *iq, long long origin, long long count,
+                      long long first_frame, long long nframes, float *rows);
+int glfer_zoom_run_iq_pcm16(glfer_zoom_plan *plan, const short *iq, long long origin, long long count,
+                            long long first_frame, long long nframes, float *rows);
+
+/* I/Q spectrogram: two-sided rows of complex FFT frames at the full sample rate.  Frame f covers complex samples
+ * [f hop - (n - hop), f hop + hop) (samples before index 0 are zero) and its row is
+ *     P[f][j] = |sum_i w[i] z[f hop - (n - hop) + i] e^{-2 pi i (j - n/2) i / n}|^2 / n,   j = 0..n-1,
+ * so bin j lies at (j - n/2) sample_rate / n and DC is at j = n/2.  No block-mean removal, RA9MB or limiter;
+ * glfer_b200_map_levels turns the rows into pixels. */
+typedef struct {
+  int n;               /* complex FFT size: power of two, 32..16384 */
+  int window_type;     /* fft.h window enum (rectangular: all ones, as the zoom) */
+  float overlap;       /* hop = (int)(n * (1.0 - overlap)), as the spectrogram */
+  int device;          /* CUDA device ordinal */
+} glfer_iq_config;
+
+typedef struct glfer_iq_plan glfer_iq_plan;
+
+void glfer_iq_config_default(glfer_iq_config *cfg);
+int glfer_iq_plan_create(const glfer_iq_config *cfg, glfer_iq_plan **plan);
+void glfer_iq_plan_destroy(glfer_iq_plan *plan);
+int glfer_iq_hop(const glfer_iq_plan *plan);
+int glfer_iq_bins(const glfer_iq_plan *plan);                           /* n */
+long long glfer_iq_num_frames(const glfer_iq_plan *plan, long long nsamples);   /* nsamples / hop */
+/* complex-sample span [lo, hi) the frames [first_frame, first_frame + nframes) read (lo may be negative) */
+void glfer_iq_required_span(const glfer_iq_plan *plan, long long first_frame, long long nframes,
+                            long long *lo, long long *hi);
+/* iq points at complex sample `origin`, `count` complex samples long, and must cover glfer_iq_required_span()
+ * clipped to [0, inf).  rows: [nframes][n] */
+int glfer_iq_run(glfer_iq_plan *plan, const float *iq, long long origin, long long count,
+                 long long first_frame, long long nframes, float *rows);
+int glfer_iq_run_pcm16(glfer_iq_plan *plan, const short *iq, long long origin, long long count,
+                       long long first_frame, long long nframes, float *rows);
+
 /* ---- hidden inputs of the per-call interface (fft.c:99,186: globals `glfer`, `opt`) ----
  * When the host program defines `opt` and `glfer` (as glfer.c:56-62 does) the per-call
  * functions read them.  Otherwise these setters provide the two values. */
