@@ -158,6 +158,9 @@ def lib() -> C.CDLL:
         l.glfer_iq_required_span.restype = None
         l.glfer_iq_run.argtypes = zoom_args
         l.glfer_iq_run_pcm16.argtypes = zoom_args
+        for name in ("glfer_iq_run_display", "glfer_iq_run_display_pcm16", "glfer_zoom_run_display",
+                     "glfer_zoom_run_display_pcm16", "glfer_zoom_run_display_iq", "glfer_zoom_run_display_iq_pcm16"):
+            getattr(l, name).argtypes = disp_args
         # per-call interface
         l.fft_init.argtypes = [C.POINTER(FftParams)]
         l.fft_do.argtypes = [C.c_void_p, C.POINTER(FftParams)]
@@ -423,6 +426,27 @@ class GramPlan:
             lib().glfer_wav_free(C.byref(wav))
 
 
+def _run_display(fn, handle, ptr, count, bins, nframes, log_scale, autoscale, max_level_db, min_level_db, thr_level,
+                 colortab, origin, first_frame, agc_state, want_rgb, out, want_range):
+    """one *_run_display call of an I/Q or zoom plan, with the keywords and outputs of GramPlan.run_display"""
+    out = out or {}
+    levels = out.get("levels") if "levels" in out else np.empty((nframes, bins), np.uint8)
+    assert levels.dtype == np.uint8 and levels.size >= nframes * bins
+    rgb = np.empty((nframes, bins, 3), np.uint8) if want_rgb else None
+    rng = None
+    if autoscale and want_range:
+        rng = out.get("range") if "range" in out else np.empty((nframes, 2), np.float32)
+    if colortab is not None:
+        colortab = np.ascontiguousarray(colortab, dtype=np.uint8)
+        assert colortab.size == 768
+    dc = DisplayConfig(int(log_scale), int(autoscale), max_level_db, min_level_db, thr_level,
+                       colortab.ctypes.data if colortab is not None else None)
+    state = agc_state if agc_state is not None else np.zeros(2, np.float32)
+    _check(fn(handle, ptr, origin, count, first_frame, nframes, C.byref(dc), state.ctypes.data, _ptr(levels), _ptr(rgb),
+              _ptr(rng)))
+    return dict(levels=levels, rgb=rgb, range=rng, agc_state=state)
+
+
 def _iq_samples(iq: np.ndarray):
     """(pointer, complex sample count, pcm16) of an I/Q array: 1-D complex64 (its memory is already interleaved,
     no copy), float32 [count, 2] or int16 [count, 2] (I, Q)"""
@@ -500,6 +524,25 @@ class ZoomPlan:
         _check(fn(self._h, samples.ctypes.data, origin, len(samples), first_frame, nframes, rows.ctypes.data))
         return rows
 
+    def run_display(self, samples: np.ndarray, log_scale=True, autoscale=True, max_level_db=-20.0, min_level_db=-80.0,
+                    thr_level=0.0, colortab: np.ndarray | None = None, origin: int = 0, first_frame: int = 0,
+                    nframes: int | None = None, agc_state: np.ndarray | None = None, want_rgb: bool = False,
+                    out: dict | None = None, want_range: bool = True):
+        """glfer_zoom_run_display*: the plan's rows -> 8-bit levels (and RGB) as main_window_draw maps them, pixel i =
+        bin n - 1 - i.  Keywords and outputs of GramPlan.run_display; an I/Q plan takes the formats of IqPlan.run."""
+        if self.iq:
+            ptr, count, pcm = _iq_samples(samples)
+            fn = lib().glfer_zoom_run_display_iq_pcm16 if pcm else lib().glfer_zoom_run_display_iq
+        else:
+            pcm = samples.dtype == np.int16
+            assert samples.flags["C_CONTIGUOUS"] and (pcm or samples.dtype == np.float32)
+            ptr, count = samples.ctypes.data, len(samples)
+            fn = lib().glfer_zoom_run_display_pcm16 if pcm else lib().glfer_zoom_run_display
+        if nframes is None:
+            nframes = self.num_frames(origin + count) - first_frame
+        return _run_display(fn, self._h, ptr, count, self.bins, nframes, log_scale, autoscale, max_level_db, min_level_db,
+                            thr_level, colortab, origin, first_frame, agc_state, want_rgb, out, want_range)
+
 
 class IqPlan:
     """glfer_iq_plan: two-sided spectrogram of complex (I/Q) input.  Rows hold n bins, bin j at
@@ -545,6 +588,19 @@ class IqPlan:
         fn = lib().glfer_iq_run_pcm16 if pcm else lib().glfer_iq_run
         _check(fn(self._h, ptr, origin, count, first_frame, nframes, rows.ctypes.data))
         return rows
+
+    def run_display(self, iq: np.ndarray, log_scale=True, autoscale=True, max_level_db=-20.0, min_level_db=-80.0,
+                    thr_level=0.0, colortab: np.ndarray | None = None, origin: int = 0, first_frame: int = 0,
+                    nframes: int | None = None, agc_state: np.ndarray | None = None, want_rgb: bool = False,
+                    out: dict | None = None, want_range: bool = True):
+        """glfer_iq_run_display / _pcm16: the plan's rows -> 8-bit levels (and RGB) as main_window_draw maps them,
+        pixel i = row position n - 1 - i.  Input formats of IqPlan.run; keywords and outputs of GramPlan.run_display."""
+        ptr, count, pcm = _iq_samples(iq)
+        if nframes is None:
+            nframes = self.num_frames(origin + count) - first_frame
+        fn = lib().glfer_iq_run_display_pcm16 if pcm else lib().glfer_iq_run_display
+        return _run_display(fn, self._h, ptr, count, self.bins, nframes, log_scale, autoscale, max_level_db, min_level_db,
+                            thr_level, colortab, origin, first_frame, agc_state, want_rgb, out, want_range)
 
 
 def zoom_taps(decim: int) -> np.ndarray:

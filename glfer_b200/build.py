@@ -19,7 +19,7 @@ OBJ = os.path.join(HERE, "_build")
 CU_UNITS = ([("csrc/gram_kernels.cu", "", []), ("csrc/gram_big.cu", "", []), ("csrc/zoom.cu", "", []), ("csrc/iq.cu", "", [])]
             + [("csrc/gram_part.cu", f".p{k}", [f"-DGLB_PART={k}"]) for k in range(4)])
 C_SOURCES = ["host/window.c", "host/dpss.c", "host/gram.c", "host/dropin.c", "host/wav.c", "host/levels.c",
-             "host/zoom.c", "host/iq.c"]
+             "host/zoom.c", "host/iq.c", "host/display.c"]
 HEADERS = ["csrc/fft_core.cuh", "csrc/fft_wpf.cuh", "csrc/fft_big.cuh", "csrc/levels.cuh", "csrc/avg_frame.cuh", "csrc/twiddle_consts.cuh", "csrc/gram_common.cuh", "csrc/iq_core.cuh", "csrc/tables.hpp", "host/glb_host.h", "../include/glb_shim.h", "../include/fft.h",
            "../include/mtm.h", "../include/avg.h", "../include/lmp.h", "../include/glfer_b200.h"]
 

@@ -167,11 +167,6 @@ extern "C" int glb_tables_destroy(void *tp) {
 }
 
 // ------------------------------------------------------------------------- display tables
-struct LevelTables {
-  float *thr_f;
-  double *thr_d;
-};
-
 extern "C" int glb_level_tables_create(const float *thr_f, const double *thr_d, int count, void **out) {
   if (!thr_f || !thr_d || count != kDbN) {
     glb_set_error("glb_level_tables_create: expected GLB_DB_NTHR thresholds");

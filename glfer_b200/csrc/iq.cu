@@ -12,6 +12,11 @@
 //   everything else         the general spectrogram kernel's spectrum output on the 2n-float frames, then
 //                           zoom_split_kernel (glb_launch_iq_gram_general, zoom.cu): the zoom's frame stage.
 //
+// LEV instantiations write 8-bit display levels (levels.cuh) instead of the float row: pixel n - 1 - j shows row
+// position j (iq_core.cuh).  Separate instantiations, for the reason the real ring kernel has them (store_levels,
+// gram_common.cuh): as a run-time branch the level mapping would cost the float-row path registers.  Launches with
+// levels that the fused kernel does not serve write float rows into scratch and map them with levels_kernel.
+//
 // glb_launch_iq_gram picks the path from the geometry; glb_force_generic_kernel(1) forces the general one.
 #include "gram_common.cuh"
 #include "iq_core.cuh"
@@ -23,7 +28,7 @@ int glb_tables_get(const void *tables, int *n, const float2 **tw, const float2 *
 // the contract's |Z|^2 / n divided by 8: the epilogue multiplies by 8, exactly.
 constexpr float kIqPowerScale = 8.f;
 
-template <int M, int QSC>
+template <int M, int QSC, bool LEV = false>
 __global__ void __launch_bounds__(Geo<M>::THREADS, (RingGeo<M, false>::MINB)) gram_iq_kernel(const KParams p) {
   using GeoM = Geo<M>;
   constexpr int T = GeoM::T, G = GeoM::G;
@@ -92,7 +97,9 @@ __global__ void __launch_bounds__(Geo<M>::THREADS, (RingGeo<M, false>::MINB)) gr
   float *row_ptr = p.rows + fb * p.row_stride;                   // (never dereferenced past nact)
   const float *next_src = p.samples + ((f_first + 1) * (long long) hop - p.origin);
   int ob[4];
-  iq_row_bases<M>(t, ob);
+  if constexpr (LEV) iq_pixel_bases<M>(t, ob);
+  else iq_row_bases<M>(t, ob);
+  unsigned char *lev_ptr = LEV ? p.levels + fb * p.lev_stride : nullptr;
   float mu_new = 0.f;
   for (int it = 0; it < p.frames_per_group; ++it, row_ptr += p.row_stride, next_src += hop) {
     const bool active = it < nact;
@@ -151,7 +158,19 @@ __global__ void __launch_bounds__(Geo<M>::THREADS, (RingGeo<M, false>::MINB)) gr
     }
     if (w0) iq_emit_power<M, true>(v, t, kIqPowerScale, yv);
     else iq_emit_power<M, false>(v, t, kIqPowerScale, yv);
-    if (active) {
+    if constexpr (LEV) {
+      if (active) {
+#pragma unroll
+        for (int slot = 0; slot < 17; slot++) {
+          if (slot == 16) {
+            if (t == 0) lev_ptr[M - 1] = map_level(yv[16], p.lm);
+          } else if (slot != 1 || t != 0) {
+            lev_ptr[iq_pixel_offset<M>(ob, slot)] = map_level(yv[slot], p.lm);
+          }
+        }
+      }
+      lev_ptr += p.lev_stride;
+    } else if (active) {
       GLB_CHECK_ROW(p, row_ptr);
       GLB_CHECK_ROW(p, row_ptr + M - 1);
 #pragma unroll
@@ -187,12 +206,14 @@ static int launch_iq_fused(const KParams &kp, cudaStream_t st) {
   const RingLayout L = ring_layout<M>(kp.hop, kPoints >> qs);
   const size_t smem = (size_t) GeoM::G * L.group_bytes + (RT ? 0 : Geo<M>::TWS_BYTES);
   if (smem > 227 * 1024) return 0;
-  void (*rk)(const KParams) = qs == 3 ? gram_iq_kernel<M, 3> : (qs == 2 ? gram_iq_kernel<M, 2> : gram_iq_kernel<M, -1>);
+  const bool lev = kp.levels != nullptr;
+  void (*rk)(const KParams) = lev ? (qs == 3 ? gram_iq_kernel<M, 3, true> : (qs == 2 ? gram_iq_kernel<M, 2, true> : gram_iq_kernel<M, -1, true>))
+                                  : (qs == 3 ? gram_iq_kernel<M, 3> : (qs == 2 ? gram_iq_kernel<M, 2> : gram_iq_kernel<M, -1>));
   int dev = 0, sms = 0;
   CU(cudaGetDevice(&dev));
   CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  static thread_local int occ_iq[5][64];
-  int &occ = occ_iq[qs][dev & 63];
+  static thread_local int occ_iq[2][5][64];
+  int &occ = occ_iq[lev][qs][dev & 63];
   if (occ == 0) {
     CU(cudaFuncSetAttribute(rk, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, rk, GeoM::THREADS, smem));
@@ -232,15 +253,21 @@ static bool iq_fused_geometry(int n, int hop) {
 
 static bool iq_fused_allowed() { return g_force_generic == 0 && g_kernel_pref != 1; }
 
-extern "C" long long glb_iq_gram_scratch_bytes(int n, int hop, long long nframes) {
+// general path: the spectrum [nframes][n + 1] (re, im) pairs, then, for a launch with levels, the float rows
+// [nframes][n] that levels_kernel maps
+extern "C" long long glb_iq_gram_scratch_bytes(int n, int hop, long long nframes, int levels) {
   if (nframes <= 0 || (iq_fused_allowed() && iq_fused_geometry(n, hop))) return 0;
-  return nframes * (long long) (n + 1) * 2 * (long long) sizeof(float);
+  return nframes * ((long long) (n + 1) * 2 + (levels ? n : 0)) * (long long) sizeof(float);
 }
 
 extern "C" int glb_launch_iq_gram(const glb_iq_gram_args *a, void *stream) {
-  if (!a || !a->tables || !a->samples || !a->taper || !a->rows || a->n < 32 || a->n > 16384 || (a->n & (a->n - 1)) != 0 ||
-      a->hop < 1 || a->hop > a->n || a->origin < 0 || a->count < 0 || a->first_frame < 0) {
-    glb_set_error("glb_launch_iq_gram: invalid arguments");
+  if (!a || !a->tables || !a->samples || !a->taper || !a->rows == !a->levels || a->n < 32 || a->n > 16384 ||
+      (a->n & (a->n - 1)) != 0 || a->hop < 1 || a->hop > a->n || a->origin < 0 || a->count < 0 || a->first_frame < 0) {
+    glb_set_error("glb_launch_iq_gram: invalid arguments (exactly one of rows and levels)");
+    return GLB_EINVAL;
+  }
+  if (a->levels && (!a->level_tables || a->levels_stride != a->n)) {
+    glb_set_error("glb_launch_iq_gram: levels need level_tables and levels_stride = n");
     return GLB_EINVAL;
   }
   if (a->nframes <= 0) return GLB_OK;
@@ -264,6 +291,16 @@ extern "C" int glb_launch_iq_gram(const glb_iq_gram_args *a, void *stream) {
     k.nframes = a->nframes;
     k.rows = a->rows;
     k.row_stride = a->n;
+    if (a->levels) {
+      k.levels = a->levels;
+      k.lev_stride = a->levels_stride;
+      k.lm.thr = ((const LevelTables *) a->level_tables)->thr_f;
+      k.lm.lut = a->levels_log ? a->level_lut : nullptr;
+      k.lm.log_scale = a->levels_log;
+      k.lm.dmin = a->level_min;
+      k.lm.dmax = a->level_max;
+      k.lm.thr_level = a->level_thr;
+    }
     k.tw = tw;
     k.vtab = vtab;
     cudaStream_t st = (cudaStream_t) stream;
@@ -282,5 +319,18 @@ extern "C" int glb_launch_iq_gram(const glb_iq_gram_args *a, void *stream) {
     }
     if (rc != 0) return rc < 0 ? rc : GLB_OK;
   }
-  return glb_launch_iq_gram_general(a, stream);
+  if (!a->levels) return glb_launch_iq_gram_general(a, stream);
+  // two passes: float rows into the scratch behind the spectrum, then the fixed-range mapping of the fused epilogue
+  if (!a->scratch) {
+    glb_set_error("glb_launch_iq_gram: needs scratch for the spectrum and rows (glb_iq_gram_scratch_bytes)");
+    return GLB_EINVAL;
+  }
+  glb_iq_gram_args g = *a;
+  g.rows = (float *) a->scratch + a->nframes * (long long) (a->n + 1) * 2;
+  g.levels = nullptr;
+  int rc = glb_launch_iq_gram_general(&g, stream);
+  if (rc != GLB_OK) return rc;
+  const float fixed[2] = {a->level_max, a->level_min};
+  return glb_launch_levels(g.rows, a->n, a->n, a->nframes, nullptr, fixed, a->levels_log, a->level_thr, a->level_tables,
+                           a->level_lut, nullptr, a->levels, nullptr, stream);
 }

@@ -50,4 +50,20 @@ template <int M> GLB_HD int iq_slot_offset(const int (&b)[4], int slot) {
   return (slot & 1) ? b[1 + hi] - 2 * rp * T : b[hi] + 2 * rp * T;
 }
 
+// Display pixels of the LEV epilogue: pixel i shows row position M - 1 - i (highest frequency first, as
+// main_window_draw draws a row), so the bases are the row bases mirrored and the offsets change sign.  A run of
+// 32 consecutive row positions stays 32 consecutive bytes, now descending for slots 2 rp and ascending for
+// slots 2 rp + 1; slot 16 (row position 0) lands on pixel M - 1.
+template <int M> GLB_HD void iq_pixel_bases(int t, int (&b)[4]) {
+  iq_row_bases<M>(t, b);
+#pragma unroll
+  for (int i = 0; i < 4; i++) b[i] = M - 1 - b[i];
+}
+template <int M> GLB_HD int iq_pixel_offset(const int (&b)[4], int slot) {
+  constexpr int T = M / kPoints;
+  if (slot == 16) return M - 1;
+  const int rp = slot >> 1, hi = rp >= 4 ? 2 : 0;
+  return (slot & 1) ? b[1 + hi] + 2 * rp * T : b[hi] - 2 * rp * T;
+}
+
 }  // namespace glb

@@ -59,6 +59,12 @@ __device__ __forceinline__ unsigned char level_u8(float sig_level, float dmin, f
   return (unsigned char) (((double) f - 255.0 * (double) thr) / (1.0 - (double) thr));
 }
 
+// the device tables behind glb_level_tables_create's handle
+struct LevelTables {
+  float *thr_f;
+  double *thr_d;
+};
+
 // what the fused epilogue and levels_kernel need to map a value
 struct LevelMap {
   const float *thr;            // [kDbN] float thresholds (log scales)

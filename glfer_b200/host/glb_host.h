@@ -30,6 +30,48 @@ unsigned char glb_level_u8(float sig_level, float dmin, float dmax, float thr);
 void glb_level_lut(float dmin, float dmax, float thr, unsigned char *lut);
 void glb_fixed_display_range(float max_level_db, float min_level_db, int log_scale, float *dmax, float *dmin);
 
+/* the display chain over device rows (host/display.c), shared by the plans' *_run_display entries */
+typedef struct {                /* per plan */
+  float *d_agc_state;           /* carried AGC levels (display_max_lvl, display_min_lvl) */
+  unsigned char *d_colortab, *d_level_lut;
+  void *level_tables;           /* dB thresholds on the device (host/levels.c) */
+  float *h_range;               /* pinned staging of the per-frame display range */
+  size_t h_range_cap;           /* bytes */
+} glb_display;
+typedef struct {                /* per slot (stream) of a plan */
+  void *ev_agc;                 /* this slot's AGC step is queued: the next chunk's recurrence waits for it */
+  float *d_stats, *d_range;
+  unsigned char *d_levels, *d_rgb;
+  size_t stats_cap, levels_cap, rgb_cap;
+} glb_display_slot;
+typedef struct {                /* one run */
+  const glfer_display_config *dc;
+  float thr;                    /* thr_level / 100 */
+  float fixed[2];               /* fixed display range (display_max, display_min), dB in the log scales */
+  float *st_range;              /* staging of the caller's display_range, or NULL */
+} glb_display_run;
+int glb_make_level_tables(void **tables);
+void glb_display_free(glb_display *d);
+void glb_display_slot_free(glb_display_slot *s);
+/* device state for a run (synchronises `stream`); want_range: the caller asked for display_range */
+int glb_display_begin(glb_display *d, glb_display_run *r, const glfer_display_config *dc, const float *agc_state,
+                      long long nframes, int want_range, void *stream);
+/* the slot's level (and RGB) buffers for nframes rows of nbins */
+int glb_display_reserve(glb_display_slot *s, long long nframes, int nbins, int rgb);
+/* levels (and RGB) of the cn device rows d_shown (floor statistics of d_psd when autoscaling) of frames [c0, c0 + cn),
+ * frames [done, done + cn) of the run; prev: the slot of the run's previous chunk, or NULL for the first */
+int glb_display_map(const glb_display *d, const glb_display_run *r, glb_display_slot *s, const glb_display_slot *prev,
+                    const float *d_psd, const float *d_shown, int nbins, long long c0, long long cn, long long done,
+                    float overlap, int rgb, void *stream);
+/* download the slot's levels / RGB (either may be NULL) to rows [done, done + cn) */
+int glb_display_fetch(const glb_display_slot *s, long long cn, int nbins, long long done, unsigned char *levels,
+                      unsigned char *rgb, void *stream);
+/* after the run's streams are synchronised: the carried AGC state and the staged display range */
+int glb_display_end(const glb_display *d, const glb_display_run *r, long long nframes, float *agc_state,
+                    float *range_out);
+/* testing aid glfer_b200_set_fused_levels (gram.c): 0 = levels always in a second pass over float rows */
+int glb_host_fused_levels(void);
+
 /* values of the hidden globals (weak `opt` / `glfer` when the host program has them) */
 int glb_autoscale(void);
 int glb_first_buffer(void);

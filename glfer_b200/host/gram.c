@@ -45,11 +45,7 @@ typedef struct {
   int *d_cand, *d_peak, *d_unres;
   size_t scal_cap;      /* frames */
   long long out_first, out_nframes, out_halo;
-  /* display mapping */
-  void *ev_agc;
-  float *d_stats, *d_range;
-  unsigned char *d_levels, *d_rgb;
-  size_t stats_cap, levels_cap, rgb_cap;
+  glb_display_slot disp;  /* display mapping */
 } slot_t;
 
 struct glfer_gram_plan {
@@ -66,18 +62,15 @@ struct glfer_gram_plan {
   slot_t slot[NSLOT];
   int *d_cand_all, *d_peak_all;   /* whole-run *peakbin candidates / carried values */
   size_t cand_all_cap;
-  float *d_agc_state;   /* display mapping: carried AGC levels */
-  unsigned char *d_colortab;
+  glb_display disp;     /* display mapping */
   /* harmonic F-test (mtm_ftest): hn and the unit-energy tapers scaled for the spectrum output, U0 */
   float *d_ftapers;     /* [ntapers + 1][n] */
   double *d_u0;
   double sum_u0_sqr;
   float *d_fspec, *d_ftest;
   size_t fspec_cap, ftest_cap;
-  void *level_tables;   /* dB thresholds on the device (host/levels.c) */
-  void *h_scal;         /* pinned staging of the small per-frame outputs (ret / variance / peakbin / display range) */
+  void *h_scal;         /* pinned staging of the small per-frame outputs (ret / variance / peakbin) */
   size_t h_scal_cap;
-  unsigned char *d_level_lut;
 };
 
 /* what a display run asks of exec_slot: levels written by the spectrogram kernel itself */
@@ -86,7 +79,6 @@ typedef struct {
   float dmin, dmax, thr;
 } fused_levels;
 
-static int make_level_tables(void **tables);
 /* Frame averaging inside the spectrogram kernel exists and is bit-identical to the two-pass form, but it is
    OFF by default: measured on B200 (C2: N=4096 Kaiser 75 %, depth 4, band of 68 bins, 168 750 frames) the
    fused kernel takes 1.31 ms against 0.82 ms + 0.20 ms in two passes -- the averaging of a frame is a
@@ -97,6 +89,7 @@ void glfer_b200_set_fused_avg(int on) { g_fused_avg = on; }
 static int g_fused_levels = 1;
 /* testing aid: 0 = always map levels in a second pass over float rows */
 void glfer_b200_set_fused_levels(int on) { g_fused_levels = on; }
+int glb_host_fused_levels(void) { return g_fused_levels; }
 
 static __thread char g_msg[512];
 
@@ -216,16 +209,14 @@ void glfer_gram_plan_destroy(glfer_gram_plan *p)
     glb_free(s->d_samples); glb_free(s->d_pcm); glb_free(s->d_means); glb_free(s->d_psd); glb_free(s->d_avg);
     glb_free(s->d_ret); glb_free(s->d_var); glb_free(s->d_cand); glb_free(s->d_peak); glb_free(s->d_unres);
     glb_event_destroy(s->ev0); glb_event_destroy(s->ev1); glb_event_destroy(s->ev2); glb_event_destroy(s->ev3);
-    glb_event_destroy(s->ev_agc);
-    glb_free(s->d_stats); glb_free(s->d_range); glb_free(s->d_levels); glb_free(s->d_rgb);
+    glb_display_slot_free(&s->disp);
     glb_stream_destroy(s->stream);
   }
   glb_free(p->d_tapers);
   glb_free(p->d_ftapers); glb_free(p->d_u0); glb_free(p->d_fspec); glb_free(p->d_ftest);
   glb_free(p->d_cand_all);
   glb_free(p->d_peak_all);
-  glb_free(p->d_agc_state); glb_free(p->d_colortab); glb_free(p->d_level_lut);
-  glb_level_tables_destroy(p->level_tables);
+  glb_display_free(&p->disp);
   glb_tables_destroy(p->tables);
   if (p->h_scal) glb_host_free(p->h_scal);
   free(p->h_window); free(p->h_tapers); free(p->h_lambda);
@@ -347,7 +338,7 @@ int glfer_gram_plan_create(const glfer_gram_config *cfg, glfer_gram_plan **out)
     if (rc == 0) rc = shim(glb_event_create(&p->slot[i].ev1));
     if (rc == 0) rc = shim(glb_event_create(&p->slot[i].ev2));
     if (rc == 0) rc = shim(glb_event_create(&p->slot[i].ev3));
-    if (rc == 0) rc = shim(glb_event_create(&p->slot[i].ev_agc));
+    if (rc == 0) rc = shim(glb_event_create(&p->slot[i].disp.ev_agc));
     if (rc == 0) rc = shim(glb_malloc((void **) &p->slot[i].d_unres, sizeof(int)));
   }
   if (rc != 0) {
@@ -446,11 +437,11 @@ static int exec_slot(glfer_gram_plan *p, slot_t *s, long long first, long long n
   g.rows = fl ? NULL : s->d_psd;
   g.row_stride = p->bins;
   if (fl) {                           /* levels straight from the kernel's registers: no float rows at all */
-    g.levels = s->d_levels;
+    g.levels = s->disp.d_levels;
     g.levels_stride = p->bins;
-    g.level_tables = p->level_tables;
+    g.level_tables = p->disp.level_tables;
     g.levels_log = fl->log_scale;
-    g.level_lut = p->d_level_lut;
+    g.level_lut = p->disp.d_level_lut;
     g.level_min = fl->dmin;
     g.level_max = fl->dmax;
     g.level_thr = fl->thr;
@@ -704,7 +695,7 @@ int glfer_gram_run_mtm_ftest(glfer_gram_plan *p, const float *samples, long long
 }
 
 /* ---------------------------------------------------------------- host-buffer API */
-/* The small per-frame outputs (ret, variance, peakbin, display range) are downloaded chunk by chunk.  Into the
+/* The small per-frame outputs (ret, variance, peakbin) are downloaded chunk by chunk.  Into the
    caller's arrays directly, each of those copies would block the host thread whenever the array is pageable
    -- and with it the chunk pipeline (measured: C2 end to end 48 ms instead of 28 ms per hour of signal) -- so
    they land in pinned staging owned by the plan and are handed over once at the end of the run. */
@@ -850,10 +841,10 @@ int glfer_gram_run_pcm16(glfer_gram_plan *p, const short *pcm, long long origin,
 }
 
 /* ---------------------------------------------------------------- display mapping
- * The tail of main_window_draw (g_main.c:1109-1229) for a whole run: per-row floor statistics
- * (compute_floor), the AGC of the display range (a recurrence over frames, walked in order on
- * the device and carried from chunk to chunk through an event chain between the slots),
- * then 8-bit levels / RGB.  Only 1 (levels) or 3 (RGB) bytes per bin go back to the host. */
+ * The tail of main_window_draw (g_main.c:1109-1229) for a whole run: the estimator's rows of each chunk go
+ * through the display chain of host/display.c (floor statistics, AGC, levels / RGB), or, with a fixed range
+ * and the estimator's own rows shown, the spectrogram kernel writes the levels itself.  Only 1 (levels) or
+ * 3 (RGB) bytes per bin go back to the host. */
 static int run_display_impl(glfer_gram_plan *p, const float *samples, const short *pcm, long long origin,
                             long long count, long long first_frame, long long nframes,
                             const glfer_display_config *dc, float *agc_state, unsigned char *levels,
@@ -875,38 +866,15 @@ static int run_display_impl(glfer_gram_plan *p, const float *samples, const shor
   if (lo < 0) lo = 0;
   if (lo < origin || hi > origin + count)
     return fail(GLFER_EINVAL, "samples do not cover the requested frames (see glfer_gram_required_span)");
-  if (!p->d_agc_state) {
-    TRY(glb_malloc((void **) &p->d_agc_state, 2 * sizeof(float)));
-    TRY(glb_malloc((void **) &p->d_colortab, 768));
-    TRY(glb_malloc((void **) &p->d_level_lut, GLB_DB_NTHR));
-    /* the device never evaluates 10 log10 itself */
-    int rt = make_level_tables(&p->level_tables);
-    if (rt != 0) return rt;
-  }
-  float *st_range = NULL;
-  if (range_out && dc->autoscale) TRY(scal_staging(p, sizeof(float) * 2 * (size_t) nframes, (void **) &st_range));
-  void *st0 = p->slot[0].stream;
-  float state[2] = { agc_state ? agc_state[0] : 0.0f, agc_state ? agc_state[1] : 0.0f };
-  TRY(glb_memcpy_h2d(p->d_agc_state, state, sizeof state, st0));
-  const float thr = dc->thr_level / 100.0;                  /* g_main.c:1098 */
-  float fixed[2] = { 0.0f, 0.0f };                          /* (display_max, display_min) */
-  if (!dc->autoscale) {
-    /* fixed levels, g_main.c:1126-1138; in the log scales the level of every integer dB value is
-       tabulated once on the host with the reference's own arithmetic */
-    unsigned char lut[GLB_DB_NTHR];
-    glb_fixed_display_range(dc->max_level_db, dc->min_level_db, dc->log_scale, &fixed[0], &fixed[1]);
-    glb_level_lut(fixed[1], fixed[0], thr, lut);
-    TRY(glb_memcpy_h2d(p->d_level_lut, lut, sizeof lut, st0));
-  }
-  if (dc->colortab) TRY(glb_memcpy_h2d(p->d_colortab, dc->colortab, 768, st0));
-  TRY(glb_stream_sync(st0));
+  glb_display_run dr;
+  TRY(glb_display_begin(&p->disp, &dr, dc, agc_state, nframes, range_out != NULL, p->slot[0].stream));
   const long long cf = chunk_frames(p);
   const int avg_on = p->cfg.avg_mode != GLFER_NO_AVG;
   /* fixed display range, rows shown = the estimator's own rows: the spectrogram kernel writes the 8-bit
      levels itself and no float row ever reaches HBM (1 byte per bin instead of 4 + 4 + 1) */
   const int plain = p->cfg.mode != GLFER_MODE_FFT || (p->cfg.a <= 0.0f && !p->cfg.limiter);   /* RA9MB / limiter: two passes */
   const int fuse = g_fused_levels && !dc->autoscale && !avg_on && p->cfg.mode != GLFER_MODE_LMP && !rgb && plain;
-  const fused_levels fl = { dc->log_scale, fixed[1], fixed[0], thr };
+  const fused_levels fl = { dc->log_scale, dr.fixed[1], dr.fixed[0], dr.thr };
   int rc = 0, ci = 0;
   long long done = 0;
   while (done < nframes && rc == 0) {
@@ -920,47 +888,19 @@ static int run_display_impl(glfer_gram_plan *p, const float *samples, const shor
     if (clo < 0) clo = 0;
     rc = stage_slot(p, s, samples ? samples + (clo - origin) : NULL, pcm ? pcm + (clo - origin) : NULL, clo, chi - clo);
     if (rc) break;
-    rc = ensure((void **) &s->d_levels, &s->levels_cap, (size_t) cn * p->bins, 1);
-    if (rc == 0 && rgb) rc = ensure((void **) &s->d_rgb, &s->rgb_cap, (size_t) cn * p->bins * 3, 1);
+    rc = glb_display_reserve(&s->disp, cn, p->bins, rgb != NULL);
     if (rc) break;
     rc = exec_slot(p, s, c0, cn, NULL, fuse ? &fl : NULL);
     if (rc) break;
-    if (fuse) {
-      if (levels) rc = shim(glb_memcpy_d2h(levels + (size_t) done * p->bins, s->d_levels, (size_t) cn * p->bins, s->stream));
-      done += cn;
-      ci++;
-      continue;
-    }
-    /* psdbuf of the GUI: the estimator's output row, which in LMP mode is the statistic */
-    const float *d_psd = (p->cfg.mode == GLFER_MODE_LMP) ? s->d_avg : s->d_psd + (size_t) s->out_halo * p->bins;
-    const float *d_shown = avg_on ? s->d_avg : d_psd;               /* g_main.c:1192-1201 */
-    const float *d_range = NULL;
-    if (dc->autoscale) {
-      if ((size_t) cn > s->stats_cap) {
-        glb_free(s->d_stats); glb_free(s->d_range);
-        s->d_stats = s->d_range = NULL; s->stats_cap = 0;
-        rc = shim(glb_malloc((void **) &s->d_stats, sizeof(float) * 4 * (size_t) cn));
-        if (rc == 0) rc = shim(glb_malloc((void **) &s->d_range, sizeof(float) * 2 * (size_t) cn));
-        if (rc) break;
-        s->stats_cap = (size_t) cn;
-      }
-      /* compute_floor always looks at the raw PSD row (g_main.c:1109) */
-      rc = shim(glb_launch_floor_stats(d_psd, p->bins, p->bins, cn, s->d_stats, s->stream));
-      /* the recurrence continues where the previous chunk (other slot) stopped */
-      if (rc == 0 && ci > 0) rc = shim(glb_stream_wait_event(s->stream, p->slot[(ci - 1) % NSLOT].ev_agc));
-      if (rc == 0) rc = shim(glb_launch_agc(s->d_stats, cn, c0, p->cfg.overlap, dc->log_scale, p->d_agc_state, s->d_range, s->stream));
-      if (rc == 0) rc = shim(glb_event_record(s->ev_agc, s->stream));
-      if (rc) break;
-      d_range = s->d_range;
-      if (range_out) rc = shim(glb_memcpy_d2h(st_range + 2 * done, s->d_range, sizeof(float) * 2 * (size_t) cn, s->stream));
+    if (!fuse) {
+      /* psdbuf of the GUI: the estimator's output row, which in LMP mode is the statistic */
+      const float *d_psd = (p->cfg.mode == GLFER_MODE_LMP) ? s->d_avg : s->d_psd + (size_t) s->out_halo * p->bins;
+      const float *d_shown = avg_on ? s->d_avg : d_psd;               /* g_main.c:1192-1201 */
+      rc = glb_display_map(&p->disp, &dr, &s->disp, ci > 0 ? &p->slot[(ci - 1) % NSLOT].disp : NULL, d_psd, d_shown,
+                           p->bins, c0, cn, done, p->cfg.overlap, rgb != NULL, s->stream);
       if (rc) break;
     }
-    rc = shim(glb_launch_levels(d_shown, p->bins, p->bins, cn, d_range, dc->autoscale ? NULL : fixed, dc->log_scale, thr,
-                                p->level_tables, p->d_level_lut, dc->colortab ? p->d_colortab : NULL, s->d_levels,
-                                rgb ? s->d_rgb : NULL, s->stream));
-    if (rc) break;
-    if (levels) rc = shim(glb_memcpy_d2h(levels + (size_t) done * p->bins, s->d_levels, (size_t) cn * p->bins, s->stream));
-    if (rc == 0 && rgb) rc = shim(glb_memcpy_d2h(rgb + (size_t) done * p->bins * 3, s->d_rgb, (size_t) cn * p->bins * 3, s->stream));
+    rc = glb_display_fetch(&s->disp, cn, p->bins, done, levels, rgb, s->stream);
     done += cn;
     ci++;
   }
@@ -968,8 +908,7 @@ static int run_display_impl(glfer_gram_plan *p, const float *samples, const shor
     int r2 = shim(glb_stream_sync(p->slot[i].stream));
     if (rc == 0) rc = r2;
   }
-  if (rc == 0 && agc_state && dc->autoscale) rc = shim(glb_memcpy_d2h(agc_state, p->d_agc_state, 2 * sizeof(float), NULL));
-  if (rc == 0 && st_range) memcpy(range_out, st_range, sizeof(float) * 2 * (size_t) nframes);
+  if (rc == 0) rc = glb_display_end(&p->disp, &dr, nframes, agc_state, range_out);
   return rc;
 }
 
@@ -989,19 +928,6 @@ int glfer_gram_run_display_pcm16(glfer_gram_plan *p, const short *pcm, long long
   return run_display_impl(p, NULL, pcm, origin, count, first_frame, nframes, dc, agc_state, levels, rgb, display_range);
 }
 
-/* dB thresholds from the host's libm (host/levels.c) on the current device */
-static int make_level_tables(void **tables)
-{
-  float *tf = malloc(sizeof(float) * GLB_DB_NTHR);
-  double *td = malloc(sizeof(double) * GLB_DB_NTHR);
-  if (!tf || !td) { free(tf); free(td); return fail(GLFER_ENOMEM, "out of memory"); }
-  glb_db_thresholds_f(tf);
-  glb_db_thresholds_d(td);
-  const int rc = shim(glb_level_tables_create(tf, td, GLB_DB_NTHR, tables));
-  free(tf); free(td);
-  return rc;
-}
-
 int glfer_b200_map_levels(const float *rows, long long nrows, int nbins, const glfer_display_config *dc,
                           const float *range, unsigned char *levels, int device)
 {
@@ -1015,7 +941,7 @@ int glfer_b200_map_levels(const float *rows, long long nrows, int nbins, const g
   const size_t cells = (size_t) nrows * nbins;
   const float thr = dc->thr_level / 100.0;
   float fixed[2] = { 0.0f, 0.0f };
-  int rc = make_level_tables(&tables);
+  int rc = glb_make_level_tables(&tables);
   if (rc == 0) rc = shim(glb_malloc(&d_rows, sizeof(float) * cells));
   if (rc == 0) rc = shim(glb_malloc(&d_lev, cells));
   if (rc == 0) rc = shim(glb_memcpy_h2d(d_rows, rows, sizeof(float) * cells, NULL));

@@ -6,6 +6,10 @@
  * in chunks of ~32 MiB of input on ISLOT streams, each chunk uploads its complex samples (the n - hop samples it
  * shares with the previous chunk again), converts int16 input to float on the device, computes its rows and copies
  * them back while the next chunk uploads.  Device memory is bounded by the chunk, not by the recording.
+ *
+ * The display entries (glfer_iq_run_display*) bring back 8-bit levels instead of rows.  With a fixed range and no
+ * RGB the spectrogram kernel maps its own powers (glb_iq_gram_args.levels) and no float row is ever stored;
+ * otherwise each chunk's rows stay on the device and go through the display chain of host/display.c.
  */
 #include <math.h>
 #include <stdlib.h>
@@ -26,6 +30,7 @@ typedef struct {
   size_t rows_cap;            /* floats */
   void *d_scratch;
   size_t scratch_cap;         /* bytes */
+  glb_display_slot disp;      /* display mapping */
 } islot;
 
 struct glfer_iq_plan {
@@ -36,6 +41,7 @@ struct glfer_iq_plan {
   float taper_scale;
   void *tables;               /* FFT tables of the 2n-float frames */
   islot slot[ISLOT];
+  glb_display disp;
 };
 
 void glfer_iq_config_default(glfer_iq_config *c)
@@ -70,8 +76,10 @@ void glfer_iq_plan_destroy(glfer_iq_plan *p)
     islot *s = &p->slot[i];
     if (s->stream) glb_stream_sync(s->stream);
     glb_free(s->d_pcm); glb_free(s->d_in); glb_free(s->d_rows); glb_free(s->d_scratch);
+    glb_display_slot_free(&s->disp);
     glb_stream_destroy(s->stream);
   }
+  glb_display_free(&p->disp);
   glb_free(p->d_taper);
   glb_tables_destroy(p->tables);
   free(p);
@@ -124,7 +132,10 @@ int glfer_iq_plan_create(const glfer_iq_config *cfg, glfer_iq_plan **out)
   p->cfg = *cfg;
   p->hop = hop;
   int rc = build_taper(p);
-  for (int i = 0; i < ISLOT && rc == 0; i++) rc = glb_host_shim(glb_stream_create(&p->slot[i].stream));
+  for (int i = 0; i < ISLOT && rc == 0; i++) {
+    rc = glb_host_shim(glb_stream_create(&p->slot[i].stream));
+    if (rc == 0) rc = glb_host_shim(glb_event_create(&p->slot[i].disp.ev_agc));
+  }
   if (rc != 0) {
     char keep[512];
     strncpy(keep, glfer_b200_last_error(), sizeof keep - 1);
@@ -156,9 +167,9 @@ static long long iq_chunk_frames(const glfer_iq_plan *p)
   return f < 1 ? 1 : f;
 }
 
-/* frames [c0, c0 + cn) on slot s */
+/* frames [c0, c0 + cn) on slot s: rows into s->d_rows, or with fl the fixed-range levels into s->disp.d_levels */
 static int iq_chunk(glfer_iq_plan *p, islot *s, const void *src, int pcm16, long long origin, long long c0,
-                    long long cn, float *rows)
+                    long long cn, const glb_display_run *fl)
 {
   const long long n = p->cfg.n, hop = p->hop;
   long long lo = c0 * hop - (n - hop);
@@ -176,8 +187,8 @@ static int iq_chunk(glfer_iq_plan *p, islot *s, const void *src, int pcm16, long
   } else {
     ITRY(glb_memcpy_h2d(s->d_in, (const float *) src + 2 * (lo - origin), sizeof(float) * 2 * (size_t) cnt, s->stream));
   }
-  ITRY(iensure((void **) &s->d_rows, &s->rows_cap, (size_t) (cn * n), sizeof(float)));
-  const long long sb = glb_iq_gram_scratch_bytes((int) n, (int) hop, cn);
+  if (!fl) ITRY(iensure((void **) &s->d_rows, &s->rows_cap, (size_t) (cn * n), sizeof(float)));
+  const long long sb = glb_iq_gram_scratch_bytes((int) n, (int) hop, cn, fl != NULL);
   if (sb > 0) ITRY(iensure(&s->d_scratch, &s->scratch_cap, (size_t) sb, 1));
   glb_iq_gram_args g;
   memset(&g, 0, sizeof g);
@@ -191,11 +202,20 @@ static int iq_chunk(glfer_iq_plan *p, islot *s, const void *src, int pcm16, long
   g.taper_scale = p->taper_scale;
   g.first_frame = c0;
   g.nframes = cn;
-  g.rows = s->d_rows;
+  g.rows = fl ? NULL : s->d_rows;
   g.tables = p->tables;
   g.scratch = sb > 0 ? s->d_scratch : NULL;
+  if (fl) {
+    g.levels = s->disp.d_levels;
+    g.levels_stride = n;
+    g.level_tables = p->disp.level_tables;
+    g.levels_log = fl->dc->log_scale;
+    g.level_lut = p->disp.d_level_lut;
+    g.level_min = fl->fixed[1];
+    g.level_max = fl->fixed[0];
+    g.level_thr = fl->thr;
+  }
   ITRY(glb_launch_iq_gram(&g, s->stream));
-  ITRY(glb_memcpy_d2h(rows, s->d_rows, sizeof(float) * (size_t) (cn * n), s->stream));
   return 0;
 }
 
@@ -221,7 +241,10 @@ static int iq_run_impl(glfer_iq_plan *p, const void *src, int pcm16, long long o
     const long long cn = (nframes - done < cf) ? nframes - done : cf;
     rc = glb_host_shim(glb_stream_sync(s->stream));
     if (rc) break;
-    rc = iq_chunk(p, s, src, pcm16, origin, first_frame + done, cn, rows + (size_t) done * p->cfg.n);
+    rc = iq_chunk(p, s, src, pcm16, origin, first_frame + done, cn, NULL);
+    if (rc == 0)
+      rc = glb_host_shim(glb_memcpy_d2h(rows + (size_t) done * p->cfg.n, s->d_rows, sizeof(float) * (size_t) (cn * p->cfg.n),
+                                        s->stream));
     done += cn;
     ci++;
   }
@@ -242,4 +265,67 @@ int glfer_iq_run_pcm16(glfer_iq_plan *p, const short *iq, long long origin, long
                        long long nframes, float *rows)
 {
   return iq_run_impl(p, iq, 1, origin, count, first_frame, nframes, rows);
+}
+
+/* main_window_draw's mapping of the plan's own rows (include/glfer_b200.h, glfer_iq_run_display) */
+static int iq_run_display_impl(glfer_iq_plan *p, const void *src, int pcm16, long long origin, long long count,
+                               long long first_frame, long long nframes, const glfer_display_config *dc,
+                               float *agc_state, unsigned char *levels, unsigned char *rgb, float *range_out)
+{
+  glb_host_clear_error();
+  if (!p || !src || !dc) return glb_host_fail(GLFER_EINVAL, "null argument");
+  if (nframes < 0 || first_frame < 0) return glb_host_fail(GLFER_EINVAL, "negative frame range");
+  if (origin < 0 || count < 0) return glb_host_fail(GLFER_EINVAL, "negative origin or sample count");
+  if (rgb && !dc->colortab) return glb_host_fail(GLFER_EINVAL, "RGB output needs a 256-entry palette");
+  if (dc->autoscale && first_frame > 0 && !agc_state)
+    return glb_host_fail(GLFER_EINVAL, "autoscale from frame > 0 needs the carried AGC state");
+  if (nframes == 0) return 0;
+  ITRY(glb_set_device(p->cfg.device));
+  long long lo, hi;
+  glfer_iq_required_span(p, first_frame, nframes, &lo, &hi);
+  if (lo < 0) lo = 0;
+  if (lo < origin || hi > origin + count)
+    return glb_host_fail(GLFER_EINVAL, "samples do not cover the requested frames (see glfer_iq_required_span)");
+  const int n = p->cfg.n;
+  glb_display_run dr;
+  ITRY(glb_display_begin(&p->disp, &dr, dc, agc_state, nframes, range_out != NULL, p->slot[0].stream));
+  /* fixed range without RGB: the spectrogram kernel writes the levels itself */
+  const int fuse = glb_host_fused_levels() && !dc->autoscale && !rgb;
+  const long long cf = iq_chunk_frames(p);
+  int rc = 0, ci = 0;
+  long long done = 0;
+  while (done < nframes && rc == 0) {
+    islot *s = &p->slot[ci % ISLOT];
+    const long long c0 = first_frame + done;
+    const long long cn = (nframes - done < cf) ? nframes - done : cf;
+    rc = glb_host_shim(glb_stream_sync(s->stream));
+    if (rc == 0) rc = glb_display_reserve(&s->disp, cn, n, rgb != NULL);
+    if (rc == 0) rc = iq_chunk(p, s, src, pcm16, origin, c0, cn, fuse ? &dr : NULL);
+    if (rc == 0 && !fuse)
+      rc = glb_display_map(&p->disp, &dr, &s->disp, ci > 0 ? &p->slot[(ci - 1) % ISLOT].disp : NULL, s->d_rows, s->d_rows,
+                           n, c0, cn, done, p->cfg.overlap, rgb != NULL, s->stream);
+    if (rc == 0) rc = glb_display_fetch(&s->disp, cn, n, done, levels, rgb, s->stream);
+    done += cn;
+    ci++;
+  }
+  for (int i = 0; i < ISLOT; i++) {
+    const int r2 = glb_host_shim(glb_stream_sync(p->slot[i].stream));
+    if (rc == 0) rc = r2;
+  }
+  if (rc == 0) rc = glb_display_end(&p->disp, &dr, nframes, agc_state, range_out);
+  return rc;
+}
+
+int glfer_iq_run_display(glfer_iq_plan *p, const float *iq, long long origin, long long count, long long first_frame,
+                         long long nframes, const glfer_display_config *dc, float *agc_state, unsigned char *levels,
+                         unsigned char *rgb, float *display_range)
+{
+  return iq_run_display_impl(p, iq, 0, origin, count, first_frame, nframes, dc, agc_state, levels, rgb, display_range);
+}
+
+int glfer_iq_run_display_pcm16(glfer_iq_plan *p, const short *iq, long long origin, long long count,
+                               long long first_frame, long long nframes, const glfer_display_config *dc,
+                               float *agc_state, unsigned char *levels, unsigned char *rgb, float *display_range)
+{
+  return iq_run_display_impl(p, iq, 1, origin, count, first_frame, nframes, dc, agc_state, levels, rgb, display_range);
 }

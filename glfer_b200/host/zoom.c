@@ -13,6 +13,9 @@
  *
  * I/Q plans (glfer_zoom_plan_create_iq) take complex input, interleaved (I, Q), through the complex decimator
  * (glb_launch_zoom_decim_iq) and accept a signed centre; everything after the decimator is the same.
+ *
+ * The display entries (glfer_zoom_run_display*) keep each chunk's rows on the device and map them through the
+ * display chain of host/display.c: only the 8-bit levels (or RGB) come back.
  */
 #include <math.h>
 #include <stdlib.h>
@@ -34,6 +37,7 @@ typedef struct {
   size_t spec_cap;            /* floats */
   float *d_rows;
   size_t rows_cap;            /* floats */
+  glb_display_slot disp;      /* display mapping */
 } zslot;
 
 struct glfer_zoom_plan {
@@ -47,6 +51,7 @@ struct glfer_zoom_plan {
   int iq;                     /* 1: complex (I, Q) input (glfer_zoom_plan_create_iq), signed centre */
   void *tables;               /* FFT tables of the 2n-point real transform */
   zslot slot[ZSLOT];
+  glb_display disp;
 };
 
 /* I0 by its power series, in double (converges quickly for the beta of the design) */
@@ -133,8 +138,10 @@ void glfer_zoom_plan_destroy(glfer_zoom_plan *p)
     if (s->stream) glb_stream_sync(s->stream);
     glb_free(s->d_in); glb_free(s->d_y); glb_free(s->d_spec); glb_free(s->d_rows);
     glb_event_destroy(s->ev_dec);
+    glb_display_slot_free(&s->disp);
     glb_stream_destroy(s->stream);
   }
+  glb_display_free(&p->disp);
   glb_free(p->d_taps);
   glb_free(p->d_taper);
   glb_tables_destroy(p->tables);
@@ -214,6 +221,7 @@ static int zoom_plan_create(const glfer_zoom_config *cfg, int iq, glfer_zoom_pla
   for (int i = 0; i < ZSLOT && rc == 0; i++) {
     rc = glb_host_shim(glb_stream_create(&p->slot[i].stream));
     if (rc == 0) rc = glb_host_shim(glb_event_create(&p->slot[i].ev_dec));
+    if (rc == 0) rc = glb_host_shim(glb_event_create(&p->slot[i].disp.ev_agc));
   }
   if (rc != 0) {
     char keep[512];
@@ -257,9 +265,9 @@ static long long zoom_chunk_frames(const glfer_zoom_plan *p)
   return f < 1 ? 1 : f;
 }
 
-/* frames [c0, c0 + cn) on slot s; prev: the slot of the previous chunk of this run, or NULL */
+/* rows of frames [c0, c0 + cn) into s->d_rows; prev: the slot of the previous chunk of this run, or NULL */
 static int zoom_chunk(glfer_zoom_plan *p, zslot *s, const zslot *prev, const void *src, int pcm16,
-                      long long origin, long long c0, long long cn, float *rows)
+                      long long origin, long long c0, long long cn)
 {
   const glfer_zoom_config *c = &p->cfg;
   const long long D = c->decim, n = c->n, hop = p->hop;
@@ -316,7 +324,6 @@ static int zoom_chunk(glfer_zoom_plan *p, zslot *s, const zslot *prev, const voi
   g.tables = p->tables;
   g.scratch = s->d_spec;
   ZTRY(glb_launch_iq_gram_general(&g, s->stream));
-  ZTRY(glb_memcpy_d2h(rows, s->d_rows, sizeof(float) * (size_t) cn * n, s->stream));
   return 0;
 }
 
@@ -346,7 +353,10 @@ static int zoom_run_impl(glfer_zoom_plan *p, int iq, const void *src, int pcm16,
     const long long cn = (nframes - done < cf) ? nframes - done : cf;
     rc = glb_host_shim(glb_stream_sync(s->stream));
     if (rc) break;
-    rc = zoom_chunk(p, s, prev, src, pcm16, origin, first_frame + done, cn, rows + (size_t) done * p->cfg.n);
+    rc = zoom_chunk(p, s, prev, src, pcm16, origin, first_frame + done, cn);
+    if (rc == 0)
+      rc = glb_host_shim(glb_memcpy_d2h(rows + (size_t) done * p->cfg.n, s->d_rows, sizeof(float) * (size_t) cn * p->cfg.n,
+                                        s->stream));
     prev = s;
     done += cn;
     ci++;
@@ -380,4 +390,89 @@ int glfer_zoom_run_iq_pcm16(glfer_zoom_plan *p, const short *iq, long long origi
                             long long first_frame, long long nframes, float *rows)
 {
   return zoom_run_impl(p, 1, iq, 1, origin, count, first_frame, nframes, rows);
+}
+
+/* main_window_draw's mapping of the plan's own rows (include/glfer_b200.h, glfer_zoom_run_display) */
+static int zoom_run_display_impl(glfer_zoom_plan *p, int iq, const void *src, int pcm16, long long origin,
+                                 long long count, long long first_frame, long long nframes,
+                                 const glfer_display_config *dc, float *agc_state, unsigned char *levels,
+                                 unsigned char *rgb, float *range_out)
+{
+  glb_host_clear_error();
+  if (!p || !src || !dc) return glb_host_fail(GLFER_EINVAL, "null argument");
+  if (iq != p->iq)
+    return glb_host_fail(GLFER_EINVAL, iq ? "glfer_zoom_run_display_iq needs a plan from glfer_zoom_plan_create_iq"
+                                          : "an I/Q zoom plan runs through glfer_zoom_run_display_iq / _iq_pcm16");
+  if (nframes < 0 || first_frame < 0) return glb_host_fail(GLFER_EINVAL, "negative frame range");
+  if (origin < 0 || count < 0) return glb_host_fail(GLFER_EINVAL, "negative origin or sample count");
+  if (rgb && !dc->colortab) return glb_host_fail(GLFER_EINVAL, "RGB output needs a 256-entry palette");
+  if (dc->autoscale && first_frame > 0 && !agc_state)
+    return glb_host_fail(GLFER_EINVAL, "autoscale from frame > 0 needs the carried AGC state");
+  if (nframes == 0) return 0;
+  ZTRY(glb_set_device(p->cfg.device));
+  long long lo, hi;
+  glfer_zoom_required_span(p, first_frame, nframes, &lo, &hi);
+  if (lo < 0) lo = 0;
+  if (lo < origin || hi > origin + count)
+    return glb_host_fail(GLFER_EINVAL, "samples do not cover the requested frames (see glfer_zoom_required_span)");
+  const int n = p->cfg.n;
+  glb_display_run dr;
+  ZTRY(glb_display_begin(&p->disp, &dr, dc, agc_state, nframes, range_out != NULL, p->slot[0].stream));
+  const long long cf = zoom_chunk_frames(p);
+  int rc = 0, ci = 0;
+  long long done = 0;
+  const zslot *prev = NULL;
+  while (done < nframes && rc == 0) {
+    zslot *s = &p->slot[ci % ZSLOT];
+    const long long c0 = first_frame + done;
+    const long long cn = (nframes - done < cf) ? nframes - done : cf;
+    rc = glb_host_shim(glb_stream_sync(s->stream));
+    if (rc == 0) rc = glb_display_reserve(&s->disp, cn, n, rgb != NULL);
+    if (rc == 0) rc = zoom_chunk(p, s, prev, src, pcm16, origin, c0, cn);
+    if (rc == 0)
+      rc = glb_display_map(&p->disp, &dr, &s->disp, prev ? &prev->disp : NULL, s->d_rows, s->d_rows, n, c0, cn, done,
+                           p->cfg.overlap, rgb != NULL, s->stream);
+    if (rc == 0) rc = glb_display_fetch(&s->disp, cn, n, done, levels, rgb, s->stream);
+    prev = s;
+    done += cn;
+    ci++;
+  }
+  for (int i = 0; i < ZSLOT; i++) {
+    const int r2 = glb_host_shim(glb_stream_sync(p->slot[i].stream));
+    if (rc == 0) rc = r2;
+  }
+  if (rc == 0) rc = glb_display_end(&p->disp, &dr, nframes, agc_state, range_out);
+  return rc;
+}
+
+int glfer_zoom_run_display(glfer_zoom_plan *p, const float *samples, long long origin, long long count,
+                           long long first_frame, long long nframes, const glfer_display_config *dc,
+                           float *agc_state, unsigned char *levels, unsigned char *rgb, float *display_range)
+{
+  return zoom_run_display_impl(p, 0, samples, 0, origin, count, first_frame, nframes, dc, agc_state, levels, rgb,
+                               display_range);
+}
+
+int glfer_zoom_run_display_pcm16(glfer_zoom_plan *p, const short *pcm, long long origin, long long count,
+                                 long long first_frame, long long nframes, const glfer_display_config *dc,
+                                 float *agc_state, unsigned char *levels, unsigned char *rgb, float *display_range)
+{
+  return zoom_run_display_impl(p, 0, pcm, 1, origin, count, first_frame, nframes, dc, agc_state, levels, rgb,
+                               display_range);
+}
+
+int glfer_zoom_run_display_iq(glfer_zoom_plan *p, const float *iq, long long origin, long long count,
+                              long long first_frame, long long nframes, const glfer_display_config *dc,
+                              float *agc_state, unsigned char *levels, unsigned char *rgb, float *display_range)
+{
+  return zoom_run_display_impl(p, 1, iq, 0, origin, count, first_frame, nframes, dc, agc_state, levels, rgb,
+                               display_range);
+}
+
+int glfer_zoom_run_display_iq_pcm16(glfer_zoom_plan *p, const short *iq, long long origin, long long count,
+                                    long long first_frame, long long nframes, const glfer_display_config *dc,
+                                    float *agc_state, unsigned char *levels, unsigned char *rgb, float *display_range)
+{
+  return zoom_run_display_impl(p, 1, iq, 1, origin, count, first_frame, nframes, dc, agc_state, levels, rgb,
+                               display_range);
 }

@@ -228,13 +228,25 @@ typedef struct {
   float *rows;                 /* device out: [nframes][n] */
   const void *tables;          /* glb_tables_create(2 n) */
   void *scratch;               /* device: glb_iq_gram_scratch_bytes() bytes, or NULL when that is 0 */
+  /* display levels of a fixed range instead of rows (main_window_draw, g_main.c:1186-1229; fields as glb_gram_args):
+     pixel i of a row shows row position n - 1 - i.  Exactly one of rows and levels is set. */
+  unsigned char *levels;       /* device out: [nframes][levels_stride], levels_stride = n */
+  long long levels_stride;
+  const void *level_tables;    /* from glb_level_tables_create() */
+  int levels_log;              /* 1: integer-truncated dB, 0: linear */
+  const unsigned char *level_lut;   /* device: level of every integer dB value (log scales) or NULL */
+  float level_min, level_max;  /* display_min / display_max (dB in the log scales) */
+  float level_thr;             /* opt.thr_level / 100 */
 } glb_iq_gram_args;
 /* The one entry of the I/Q spectrogram: the fused kernel (iq.cu, regular geometry n = 32..8192, hop = (n/16) << s
  * with n - hop a multiple of hop; needs an even origin, a 16-byte aligned samples pointer and samples that cover
- * every frame's blocks) or, for any other launch or under glb_force_generic_kernel(1), the general path below. */
+ * every frame's blocks) or, for any other launch or under glb_force_generic_kernel(1), the general path below.
+ * With levels the fused kernel maps the powers in its epilogue; the general path writes rows into scratch and
+ * maps them with glb_launch_levels. */
 int glb_launch_iq_gram(const glb_iq_gram_args *a, void *stream);
-/* device scratch glb_launch_iq_gram needs for nframes frames (0 when the fused kernel serves the geometry) */
-long long glb_iq_gram_scratch_bytes(int n, int hop, long long nframes);
+/* device scratch glb_launch_iq_gram needs for nframes frames (0 when the fused kernel serves the geometry);
+ * levels: 1 when the launch writes levels (the general path then also holds the float rows) */
+long long glb_iq_gram_scratch_bytes(int n, int hop, long long nframes, int levels);
 /* the general path: the general spectrogram kernel's spectrum output on the 2n-float frames (into scratch, at
  * least nframes (n + 1) (re, im) pairs), then glb_launch_zoom_split */
 int glb_launch_iq_gram_general(const glb_iq_gram_args *a, void *stream);

@@ -173,8 +173,8 @@ void glfer_b200_set_zero_copy(int on);
  * can be (avg_band_only plans, N = 4096 / 8192, regular overlap, band history <= 2 KB): bit-identical rows, but
  * measured slower on B200 (1.31 ms against 0.82 + 0.20 ms on BASELINE config C2), so it is opt-in */
 void glfer_b200_set_fused_avg(int on);
-/* testing aid: 0 = glfer_gram_run_display always maps the levels in a second pass over float rows; 1 (default) =
- * with a fixed display range and no averaging the spectrogram kernel writes the 8-bit levels itself */
+/* testing aid: 0 = glfer_gram_run_display and glfer_iq_run_display always map the levels in a second pass over float
+ * rows; 1 (default) = with a fixed display range and no averaging the spectrogram kernel writes the 8-bit levels itself */
 void glfer_b200_set_fused_levels(int on);
 /* the palettes of set_palette (g_main.c:649-762; glfer.h:47: 0 HSV, 1 THRESH, 2 COOL, 3 HOT, 4 BW, 5 BONE,
  * 6 COPPER, 7 OTD): 256 RGB triplets into tab[768] */
@@ -272,7 +272,7 @@ int glfer_zoom_run_iq_pcm16(glfer_zoom_plan *plan, const short *iq, long long or
  * [f hop - (n - hop), f hop + hop) (samples before index 0 are zero) and its row is
  *     P[f][j] = |sum_i w[i] z[f hop - (n - hop) + i] e^{-2 pi i (j - n/2) i / n}|^2 / n,   j = 0..n-1,
  * so bin j lies at (j - n/2) sample_rate / n and DC is at j = n/2.  No block-mean removal, RA9MB or limiter;
- * glfer_b200_map_levels turns the rows into pixels. */
+ * glfer_iq_run_display gives the waterfall's pixels directly. */
 typedef struct {
   int n;               /* complex FFT size: power of two, 32..16384 */
   int window_type;     /* fft.h window enum (rectangular: all ones, as the zoom) */
@@ -297,6 +297,37 @@ int glfer_iq_run(glfer_iq_plan *plan, const float *iq, long long origin, long lo
                  long long first_frame, long long nframes, float *rows);
 int glfer_iq_run_pcm16(glfer_iq_plan *plan, const short *iq, long long origin, long long count,
                        long long first_frame, long long nframes, float *rows);
+
+/* ---- display output of I/Q and zoom plans ----
+ * The waterfall of the plan's own rows, as glfer_gram_run_display gives it for real audio: levels, rgb, agc_state
+ * and display_range as there, and exactly main_window_draw's mapping (g_main.c:1109-1229) of the rows that
+ * glfer_iq_run / glfer_zoom_run* compute.  Both the floor statistics and the row shown are the plan's row (these
+ * plans do not average); pixel i of a row is row position n - 1 - i, the highest frequency first; the AGC's first
+ * frame divides by the plan's overlap.  agc_state chains the recurrence between calls and time shards.  GLFER_EINVAL
+ * for autoscale from first_frame > 0 without agc_state, RGB without a palette, input that does not cover the
+ * plan's required span, and (zoom) a real entry point with an I/Q plan or the reverse.
+ * The I/Q centre -- the receiver's LO leakage, at row position n/2 -- is a bin like any other: a strong spike there
+ * can be the row's largest bin and so set the AGC's upper level, as it would in the reference's mapping.
+ * I/Q plans with a fixed range and no RGB compute the levels in the spectrogram kernel itself (no float row is
+ * stored); the other cases map device rows, and only the levels (or RGB) and the range cross PCIe. */
+int glfer_iq_run_display(glfer_iq_plan *plan, const float *iq, long long origin, long long count,
+                         long long first_frame, long long nframes, const glfer_display_config *dc,
+                         float *agc_state, unsigned char *levels, unsigned char *rgb, float *display_range);
+int glfer_iq_run_display_pcm16(glfer_iq_plan *plan, const short *iq, long long origin, long long count,
+                               long long first_frame, long long nframes, const glfer_display_config *dc,
+                               float *agc_state, unsigned char *levels, unsigned char *rgb, float *display_range);
+int glfer_zoom_run_display(glfer_zoom_plan *plan, const float *samples, long long origin, long long count,
+                           long long first_frame, long long nframes, const glfer_display_config *dc,
+                           float *agc_state, unsigned char *levels, unsigned char *rgb, float *display_range);
+int glfer_zoom_run_display_pcm16(glfer_zoom_plan *plan, const short *pcm, long long origin, long long count,
+                                 long long first_frame, long long nframes, const glfer_display_config *dc,
+                                 float *agc_state, unsigned char *levels, unsigned char *rgb, float *display_range);
+int glfer_zoom_run_display_iq(glfer_zoom_plan *plan, const float *iq, long long origin, long long count,
+                              long long first_frame, long long nframes, const glfer_display_config *dc,
+                              float *agc_state, unsigned char *levels, unsigned char *rgb, float *display_range);
+int glfer_zoom_run_display_iq_pcm16(glfer_zoom_plan *plan, const short *iq, long long origin, long long count,
+                                    long long first_frame, long long nframes, const glfer_display_config *dc,
+                                    float *agc_state, unsigned char *levels, unsigned char *rgb, float *display_range);
 
 /* ---- hidden inputs of the per-call interface (fft.c:99,186: globals `glfer`, `opt`) ----
  * When the host program defines `opt` and `glfer` (as glfer.c:56-62 does) the per-call
