@@ -156,6 +156,11 @@ def lib() -> C.CDLL:
         l.glfer_iq_required_span.argtypes = [C.c_void_p, C.c_longlong, C.c_longlong, C.POINTER(C.c_longlong),
                                              C.POINTER(C.c_longlong)]
         l.glfer_iq_required_span.restype = None
+        l.glfer_iq_plan_create_mtm.argtypes = [C.POINTER(IqConfig), C.c_float, C.c_int, C.POINTER(C.c_void_p)]
+        l.glfer_zoom_plan_create_mtm.argtypes = [C.POINTER(ZoomConfig), C.c_float, C.c_int, C.POINTER(C.c_void_p)]
+        l.glfer_zoom_plan_create_iq_mtm.argtypes = [C.POINTER(ZoomConfig), C.c_float, C.c_int, C.POINTER(C.c_void_p)]
+        l.glfer_iq_tapers.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
+        l.glfer_zoom_tapers.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         l.glfer_iq_run.argtypes = zoom_args
         l.glfer_iq_run_pcm16.argtypes = zoom_args
         for name in ("glfer_iq_run_display", "glfer_iq_run_display_pcm16", "glfer_zoom_run_display",
@@ -458,18 +463,34 @@ def _iq_samples(iq: np.ndarray):
     return iq.ctypes.data, iq.shape[0], iq.dtype == np.int16
 
 
+def _tapers(fn, h, k, n):
+    k = max(k, 1)
+    t = np.empty((k, n), dtype=np.float64)
+    lam = np.empty(k, dtype=np.float64)
+    _check(fn(h, t.ctypes.data, lam.ctypes.data))
+    return t, lam
+
+
 class ZoomPlan:
     """glfer_zoom_plan: mix center_hz to DC, low-pass and decimate by `decim`, complex FFT frames of n points.
     Rows hold n bins in frequency order, bin j at center_hz() + (j - n/2) * sample_rate / (decim * n).
-    iq=True: complex (I/Q) input (glfer_zoom_plan_create_iq), centre in [-sample_rate/2, sample_rate/2]."""
+    iq=True: complex (I/Q) input (glfer_zoom_plan_create_iq), centre in [-sample_rate/2, sample_rate/2].
+    multitaper=True: rows of K' = mtm_kmax + 1 DPSS tapers of NW = mtm_w (glfer_zoom_plan_create[_iq]_mtm; window_type
+    is ignored)."""
 
     def __init__(self, n=4096, decim=256, window_type=HANNING, overlap=0.0, center_hz=800.0, sample_rate=48000.0,
-                 device=0, iq=False):
+                 device=0, iq=False, multitaper=False, mtm_w=4.0, mtm_kmax=7):
         self.cfg = ZoomConfig(n, decim, window_type, overlap, center_hz, sample_rate, device)
         self._h = C.c_void_p()
         self.iq = iq
-        create = lib().glfer_zoom_plan_create_iq if iq else lib().glfer_zoom_plan_create
-        _check(create(C.byref(self.cfg), C.byref(self._h)))
+        self.multitaper = multitaper
+        self.mtm_kmax = mtm_kmax
+        if multitaper:
+            create = lib().glfer_zoom_plan_create_iq_mtm if iq else lib().glfer_zoom_plan_create_mtm
+            _check(create(C.byref(self.cfg), mtm_w, mtm_kmax, C.byref(self._h)))
+        else:
+            create = lib().glfer_zoom_plan_create_iq if iq else lib().glfer_zoom_plan_create
+            _check(create(C.byref(self.cfg), C.byref(self._h)))
         self.n = n
         self.decim = decim
         self.hop = lib().glfer_zoom_hop(self._h)
@@ -500,6 +521,10 @@ class ZoomPlan:
 
     def taps(self) -> np.ndarray:
         return zoom_taps(self.decim)
+
+    def tapers(self):
+        """glfer_zoom_tapers: (tapers [K'][n], lambda [K']) as float64, before scaling (multitaper plans only)"""
+        return _tapers(lib().glfer_zoom_tapers, self._h, self.mtm_kmax + 1 if self.multitaper else 1, self.n)
 
     def run(self, samples: np.ndarray, origin: int = 0, first_frame: int = 0, nframes: int | None = None,
             out: np.ndarray | None = None) -> np.ndarray:
@@ -546,12 +571,19 @@ class ZoomPlan:
 
 class IqPlan:
     """glfer_iq_plan: two-sided spectrogram of complex (I/Q) input.  Rows hold n bins, bin j at
-    (j - n/2) * sample_rate / n (DC at n/2): |FFT(w z_f)|^2 / n, fft-shifted."""
+    (j - n/2) * sample_rate / n (DC at n/2): |FFT(w z_f)|^2 / n, fft-shifted.
+    multitaper=True: rows of K' = mtm_kmax + 1 DPSS tapers of NW = mtm_w (glfer_iq_plan_create_mtm; window_type is
+    ignored)."""
 
-    def __init__(self, n=4096, window_type=HANNING, overlap=0.5, device=0):
+    def __init__(self, n=4096, window_type=HANNING, overlap=0.5, device=0, multitaper=False, mtm_w=4.0, mtm_kmax=7):
         self.cfg = IqConfig(n, window_type, overlap, device)
         self._h = C.c_void_p()
-        _check(lib().glfer_iq_plan_create(C.byref(self.cfg), C.byref(self._h)))
+        self.multitaper = multitaper
+        self.mtm_kmax = mtm_kmax
+        if multitaper:
+            _check(lib().glfer_iq_plan_create_mtm(C.byref(self.cfg), mtm_w, mtm_kmax, C.byref(self._h)))
+        else:
+            _check(lib().glfer_iq_plan_create(C.byref(self.cfg), C.byref(self._h)))
         self.n = n
         self.hop = lib().glfer_iq_hop(self._h)
         self.bins = lib().glfer_iq_bins(self._h)
@@ -574,6 +606,10 @@ class IqPlan:
         lo, hi = C.c_longlong(), C.c_longlong()
         lib().glfer_iq_required_span(self._h, first_frame, nframes, C.byref(lo), C.byref(hi))
         return lo.value, hi.value
+
+    def tapers(self):
+        """glfer_iq_tapers: (tapers [K'][n], lambda [K']) as float64, before scaling (multitaper plans only)"""
+        return _tapers(lib().glfer_iq_tapers, self._h, self.mtm_kmax + 1 if self.multitaper else 1, self.n)
 
     def run(self, iq: np.ndarray, origin: int = 0, first_frame: int = 0, nframes: int | None = None,
             out: np.ndarray | None = None) -> np.ndarray:

@@ -12,6 +12,10 @@
 //   everything else         the general spectrogram kernel's spectrum output on the 2n-float frames, then
 //                           zoom_split_kernel (glb_launch_iq_gram_general, zoom.cu): the zoom's frame stage.
 //
+//   gram_iq_mtm_kernel<M, QSC>  multitaper rows on the same geometry: the frame stays in registers while each of
+//                           the K' tapers runs the transform, and the powers are summed before the one row store.
+//                           Multitaper launches of any other geometry take the general path once per taper.
+//
 // LEV instantiations write 8-bit display levels (levels.cuh) instead of the float row: pixel n - 1 - j shows row
 // position j (iq_core.cuh).  Separate instantiations, for the reason the real ring kernel has them (store_levels,
 // gram_common.cuh): as a run-time branch the level mapping would cost the float-row path registers.  Launches with
@@ -187,12 +191,173 @@ __global__ void __launch_bounds__(Geo<M>::THREADS, (RingGeo<M, false>::MINB)) gr
   }
 }
 
+// CTAs per SM the multitaper kernel is compiled for: RingGeo<M, true>::MINB (4 CTAs of 128 threads) where that is
+// spill-free (n <= 256); one CTA less from n = 512 on, where the frame x[], the sums acc[] and the transform's
+// registers no longer fit 128 registers (at 4 CTAs n = 512 ... 4096 spill 4 ... 484 bytes): 3 CTAs for n = 512 ... 2048
+// (134 - 144 registers), 2 for n = 4096 (256 threads, 120 registers), 1 for n = 8192 (512 threads, 118 - 120)
+template <int M> struct IqMtmGeo {
+  static constexpr int MINB = M <= 256 ? RingGeo<M, true>::MINB : (M <= 2048 ? 3 : (M == 4096 ? 2 : 1));
+};
+// Multitaper rows: the frame loop of gram_iq_kernel with the multitaper loop of gram_ring_kernel.  The frame is
+// fetched from the ring once and kept in registers (x) while each of the p.ntapers tapers ([2M] floats each at
+// p.tapers) runs the multiply, the passes and the power epilogue; the powers are summed per slot in taper order
+// (acc) and stored once per frame, with the stores of the periodogram's float rows.  A kernel of its own rather than
+// a template flag of gram_iq_kernel, which keeps the periodogram kernels' instructions as they are.
+template <int M, int QSC>
+__global__ void __launch_bounds__(Geo<M>::THREADS, (IqMtmGeo<M>::MINB)) gram_iq_mtm_kernel(const KParams p) {
+  using GeoM = Geo<M>;
+  constexpr int T = GeoM::T, G = GeoM::G;
+  constexpr bool RT = RingGeo<M, true>::RT;
+  extern __shared__ __align__(16) unsigned char smem_raw[];
+  const int g = threadIdx.x / T;
+  const int t = threadIdx.x % T;
+  const int qs = QSC >= 0 ? QSC : p.qs;
+  const int hop = QSC >= 0 ? ((2 * T) << (QSC >= 0 ? QSC : 0)) : p.hop;   // floats: 2 complex hops
+  const int nb = kPoints >> qs;
+  const RingLayout L = ring_layout<M>(hop, nb);                  // the real kernel's layout (the mean slots stay unused)
+  const int slots = L.slots;
+  unsigned char *gbase = smem_raw + (size_t) g * L.group_bytes;
+  float2 *buf = reinterpret_cast<float2 *>(gbase);
+  float *ring = reinterpret_cast<float *>(gbase + L.ring_off);
+  float *red = reinterpret_cast<float *>(gbase + L.red_off);
+  float *mu = reinterpret_cast<float *>(gbase + L.mu_off);
+  unsigned long long *mbar = reinterpret_cast<unsigned long long *>(gbase + L.mbar_off);
+  const long long gid = (long long) blockIdx.x * G + g;
+  const long long fb = gid * p.frames_per_group;
+  const bool group_active = fb < p.nframes;
+  const long long f_first = p.first_frame + fb;
+  const long long b0 = f_first - (nb - 1);                       // oldest block of the first frame
+  const unsigned blk_bytes = (unsigned) hop * 4u;
+  unsigned phase_bits = 0;
+
+  TwRegs tr;
+  if constexpr (RT) load_tw_regs<M>(tr, t, p.tw, p.vtab);
+  if (t == 0) {
+    for (int sl = 0; sl < slots; sl++) mbar_init(&mbar[sl], 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  const float2 *tw_mid = p.tw;
+  if constexpr (!RT) {
+    float2 *tws = reinterpret_cast<float2 *>(smem_raw + (size_t) G * L.group_bytes);
+    constexpr int kMid = TwOffset<M, Plan<M>::NP - 1>::value;
+    for (int i = threadIdx.x; i < kMid; i += GeoM::THREADS) tws[i] = p.tw[i];
+    tw_mid = tws;
+  }
+  group_sync<M>(g);
+
+  // prologue: the nb blocks of the first frame, zeros before the stream start
+  for (int lb = 0; lb < nb; lb++) {
+    const long long blk = b0 + lb;
+    if (group_active) {
+      if (blk < 0) {
+        float2 *z = reinterpret_cast<float2 *>(ring + (size_t) lb * hop);
+        for (int i = 0; i < (1 << qs); i++) z[t + T * i] = make_float2(0.f, 0.f);
+      } else if (t == 0) {
+        GLB_CHECK_SRC(p, p.samples + (blk * hop - p.origin), hop);
+        mbar_expect_tx(&mbar[lb], blk_bytes);
+        tma_load_1d(ring + (size_t) lb * hop, p.samples + (blk * hop - p.origin), blk_bytes, &mbar[lb]);
+      }
+    }
+  }
+  for (int lb = 0; lb < nb; lb++) {
+    if (group_active && b0 + lb >= 0) {
+      mbar_wait(&mbar[lb], 0);
+      phase_bits ^= 1u << lb;
+    }
+  }
+  group_sync<M>(g);                                               // zero fill visible
+
+  int slot_new = nb - 1;
+  const int nact = group_active ? (int) ((p.nframes - fb < p.frames_per_group) ? p.nframes - fb : p.frames_per_group) : 0;
+  float *row_ptr = p.rows + fb * p.row_stride;                   // (never dereferenced past nact)
+  const float *next_src = p.samples + ((f_first + 1) * (long long) hop - p.origin);
+  int ob[4];
+  iq_row_bases<M>(t, ob);
+  float mu_new = 0.f;
+  for (int it = 0; it < p.frames_per_group; ++it, row_ptr += p.row_stride, next_src += hop) {
+    const bool active = it < nact;
+    const bool next_there = it + 1 < nact;
+    const int slot_next = (slot_new + 1 == slots) ? 0 : slot_new + 1;
+    if (it > 0 && active) {
+      mbar_wait(&mbar[slot_new], (phase_bits >> slot_new) & 1u);
+      phase_bits ^= 1u << slot_new;
+    }
+    auto request_next = [&]() {
+      GLB_CHECK_SRC(p, next_src, hop);
+      asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+      mbar_expect_tx(&mbar[slot_next], blk_bytes);
+      tma_load_1d(ring + (size_t) slot_next * hop, next_src, blk_bytes, &mbar[slot_next]);
+    };
+    if (GLB_RING_EXTRA && next_there && t == 0) request_next();
+    const int slot_oldest = GLB_RING_EXTRA ? ((slot_next + 1 == slots) ? 0 : slot_next + 1) : slot_next;
+    {
+      float2 x[kPoints];
+      if constexpr (QSC >= 0) {
+        ring_fetch<M, (QSC >= 0 ? QSC : 0)>(x, t, ring, hop, slot_oldest, slots, mu, mu_new, false, false, red, 0.f, g);
+      } else {
+        switch (qs) {
+          case 4: ring_fetch<M, 4>(x, t, ring, hop, slot_oldest, slots, mu, mu_new, false, false, red, 0.f, g); break;
+          case 3: ring_fetch<M, 3>(x, t, ring, hop, slot_oldest, slots, mu, mu_new, false, false, red, 0.f, g); break;
+          case 2: ring_fetch<M, 2>(x, t, ring, hop, slot_oldest, slots, mu, mu_new, false, false, red, 0.f, g); break;
+          case 1: ring_fetch<M, 1>(x, t, ring, hop, slot_oldest, slots, mu, mu_new, false, false, red, 0.f, g); break;
+          default: ring_fetch<M, 0>(x, t, ring, hop, slot_oldest, slots, mu, mu_new, false, false, red, 0.f, g); break;
+        }
+      }
+      float acc[17];
+#pragma unroll
+      for (int i = 0; i < 17; i++) acc[i] = 0.f;
+      for (int j = 0; j < p.ntapers; ++j) {
+        float2 v[kPoints];
+        apply_taper<M, true>(v, x, t, p, p.tapers + (size_t) j * GeoM::N);
+        if constexpr (RT) {
+          pass_compute_rt<M, 0>(v, tr);
+          group_sync<M>(g);            // (A) the previous transform's last pass has been read by all
+          pass_scatter<M, 0>(v, t, buf);
+        } else {
+          group_sync<M>(g);
+          pass_store<M, 0>(v, t, buf, p.tw);
+        }
+        // the frame is in registers: past the first (A) nobody reads the oldest ring slot any more
+        if (!GLB_RING_EXTRA && next_there && j == 0 && t == 0) request_next();
+        group_sync<M>(g);
+        RingMidPasses<M, 1, RT>::run(v, t, buf, tw_mid, tr, g);
+        const bool w0 = t < 32;
+        if constexpr (RT) {
+          last_pass_rt<M>(v, t, buf, p.tw, tr);
+        } else {
+          TwRegs tl;
+          load_last_regs<M>(tl, t, p.tw, p.vtab);
+          last_pass_load<M>(v, t, buf);
+          last_pass_compute_rt<M>(v, t, tl);
+        }
+        if (w0) iq_add_power<M, true>(v, t, kIqPowerScale, acc);
+        else iq_add_power<M, false>(v, t, kIqPowerScale, acc);
+      }
+      if (active) {
+        GLB_CHECK_ROW(p, row_ptr);
+        GLB_CHECK_ROW(p, row_ptr + M - 1);
+#pragma unroll
+        for (int slot = 0; slot < 17; slot++) {
+          if (slot == 16) {
+            if (t == 0) st_row(row_ptr, acc[16]);
+          } else if (slot != 1 || t != 0) {
+            st_row(row_ptr + iq_slot_offset<M>(ob, slot), acc[slot]);
+          }
+        }
+      }
+    }
+    slot_new = slot_next;
+    // no barrier here: (A) of the next transform orders these reads of `buf` before its stores
+  }
+}
+
 // regular geometry, staged span covers every block of the launch, 16-byte aligned blocks: fused kernel.
 // Returns 1 when launched, 0 when the launch is not served, < 0 on error.
 template <int M>
 static int launch_iq_fused(const KParams &kp, cudaStream_t st) {
   using GeoM = Geo<M>;
-  constexpr bool RT = RingGeo<M, false>::RT;
+  const bool multi = kp.ntapers > 1;
+  const bool rt = multi ? RingGeo<M, true>::RT : RingGeo<M, false>::RT;
   const int unit = 2 * GeoM::T;
   int qs = -1;
   for (int s2 = 0; s2 <= 4; s2++)
@@ -204,16 +369,18 @@ static int launch_iq_fused(const KParams &kp, cudaStream_t st) {
   const long long blk_hi = (kp.first_frame + kp.nframes) * (long long) kp.hop;
   if (!(kp.origin <= (blk_lo > 0 ? blk_lo : 0) && blk_hi <= kp.origin + kp.count)) return 0;
   const RingLayout L = ring_layout<M>(kp.hop, kPoints >> qs);
-  const size_t smem = (size_t) GeoM::G * L.group_bytes + (RT ? 0 : Geo<M>::TWS_BYTES);
+  const size_t smem = (size_t) GeoM::G * L.group_bytes + (rt ? 0 : Geo<M>::TWS_BYTES);
   if (smem > 227 * 1024) return 0;
   const bool lev = kp.levels != nullptr;
-  void (*rk)(const KParams) = lev ? (qs == 3 ? gram_iq_kernel<M, 3, true> : (qs == 2 ? gram_iq_kernel<M, 2, true> : gram_iq_kernel<M, -1, true>))
-                                  : (qs == 3 ? gram_iq_kernel<M, 3> : (qs == 2 ? gram_iq_kernel<M, 2> : gram_iq_kernel<M, -1>));
+  void (*rk)(const KParams) =
+      multi ? (qs == 3 ? gram_iq_mtm_kernel<M, 3> : (qs == 2 ? gram_iq_mtm_kernel<M, 2> : gram_iq_mtm_kernel<M, -1>))
+      : lev ? (qs == 3 ? gram_iq_kernel<M, 3, true> : (qs == 2 ? gram_iq_kernel<M, 2, true> : gram_iq_kernel<M, -1, true>))
+            : (qs == 3 ? gram_iq_kernel<M, 3> : (qs == 2 ? gram_iq_kernel<M, 2> : gram_iq_kernel<M, -1>));
   int dev = 0, sms = 0;
   CU(cudaGetDevice(&dev));
   CU(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
-  static thread_local int occ_iq[2][5][64];
-  int &occ = occ_iq[lev][qs][dev & 63];
+  static thread_local int occ_iq[3][5][64];
+  int &occ = occ_iq[multi ? 2 : lev][qs][dev & 63];
   if (occ == 0) {
     CU(cudaFuncSetAttribute(rk, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
     CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, rk, GeoM::THREADS, smem));
@@ -242,6 +409,8 @@ static int launch_iq_fused(const KParams &kp, cudaStream_t st) {
   return 1;
 }
 
+// (the multitaper kernel serves the same n as the periodogram's, n = 8192 included: 3.6x faster than the general
+// path there, DESIGN §7.5)
 static int iq_fused_n(int n) { return n >= 32 && n <= 8192 && (n & (n - 1)) == 0; }
 
 static bool iq_fused_geometry(int n, int hop) {
@@ -254,8 +423,10 @@ static bool iq_fused_geometry(int n, int hop) {
 static bool iq_fused_allowed() { return g_force_generic == 0 && g_kernel_pref != 1; }
 
 // general path: the spectrum [nframes][n + 1] (re, im) pairs, then, for a launch with levels, the float rows
-// [nframes][n] that levels_kernel maps
-extern "C" long long glb_iq_gram_scratch_bytes(int n, int hop, long long nframes, int levels) {
+// [nframes][n] that levels_kernel maps.  A multitaper launch reuses the one spectrum plane for every taper and the
+// fused kernel serves it wherever it serves the periodogram, so the size does not depend on ntapers.
+extern "C" long long glb_iq_gram_scratch_bytes(int n, int hop, long long nframes, int levels, int ntapers) {
+  (void) ntapers;
   if (nframes <= 0 || (iq_fused_allowed() && iq_fused_geometry(n, hop))) return 0;
   return nframes * ((long long) (n + 1) * 2 + (levels ? n : 0)) * (long long) sizeof(float);
 }
@@ -264,6 +435,14 @@ extern "C" int glb_launch_iq_gram(const glb_iq_gram_args *a, void *stream) {
   if (!a || !a->tables || !a->samples || !a->taper || !a->rows == !a->levels || a->n < 32 || a->n > 16384 ||
       (a->n & (a->n - 1)) != 0 || a->hop < 1 || a->hop > a->n || a->origin < 0 || a->count < 0 || a->first_frame < 0) {
     glb_set_error("glb_launch_iq_gram: invalid arguments (exactly one of rows and levels)");
+    return GLB_EINVAL;
+  }
+  if (a->ntapers < 0 || a->ntapers > 32) {
+    glb_set_error("glb_launch_iq_gram: ntapers must be in 0..32");
+    return GLB_EINVAL;
+  }
+  if (a->levels && a->ntapers > 1) {
+    glb_set_error("glb_launch_iq_gram: multitaper rows have no level output (map them with glb_launch_levels)");
     return GLB_EINVAL;
   }
   if (a->levels && (!a->level_tables || a->levels_stride != a->n)) {
@@ -284,7 +463,7 @@ extern "C" int glb_launch_iq_gram(const glb_iq_gram_args *a, void *stream) {
     k.origin = 2 * a->origin;
     k.count = 2 * a->count;
     k.tapers = a->taper;
-    k.ntapers = 1;
+    k.ntapers = a->ntapers > 1 ? a->ntapers : 1;
     k.hop = 2 * a->hop;
     k.n_ov = 2 * (a->n - a->hop);
     k.first_frame = a->first_frame;

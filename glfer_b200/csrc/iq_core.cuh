@@ -29,6 +29,20 @@ GLB_HD void iq_emit_power(float2 *v, int t, float scale, float (&yv)[17]) {
   }
 }
 
+// The same powers added to a multitaper row's per-slot sums (acc[slot] += scale |Z|^2, the order of iq_emit_power)
+template <int M, bool T0 = true>
+GLB_HD void iq_add_power(float2 *v, int t, float scale, float (&acc)[17]) {
+  if (T0 && t == 0) {
+    const float2 z = thread0_fixup(v);
+    acc[16] += scale * norm2(z);
+  }
+#pragma unroll
+  for (int rp = 0; rp < 8; rp++) {
+    acc[2 * rp] += scale * norm2(v[rp]);
+    acc[2 * rp + 1] += scale * norm2(v[15 - rp]);
+  }
+}
+
 template <int M> GLB_HD bool iq_slot_stored(int t, int slot) { return slot == 16 ? t == 0 : !(t == 0 && slot == 1); }
 
 // Row positions as four per-thread bases plus compile-time offsets (the stores of a warp cover 32

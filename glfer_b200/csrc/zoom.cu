@@ -18,6 +18,8 @@
 //                         rounds exactly as the real kernel's when Q = 0.
 //   zoom_split_kernel     X[k], k = 0..Nz, of the interleaved (re, im) stream seen as 2 Nz real points ->
 //                         Z[k] = E + iO of the complex frame -> |Z|^2 / Nz in fft-shifted bin order.
+//   iq_mtm_split_kernel   the same split for one taper of a multitaper row: taper 0 stores |Z_0|^2 / Nz, taper
+//                         k > 0 adds |Z_k|^2 / Nz to the row, so the tapers are summed in the order k = 0..K'-1.
 #include <cuda_runtime.h>
 #include <atomic>
 #include <cstdio>
@@ -158,6 +160,28 @@ __global__ void zoom_split_kernel(const float2 *__restrict__ spec, int nz, long 
   }
 }
 
+// zoom_split_kernel's arithmetic, kept apart so that the periodogram's kernel keeps its exact instructions
+__global__ void iq_mtm_split_kernel(const float2 *__restrict__ spec, int nz, long long nframes, float inv_nz, int add,
+                                    float *__restrict__ rows) {
+  const long long total = nframes * nz;
+  const long long stride = (long long) gridDim.x * blockDim.x;
+  for (long long idx = (long long) blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += stride) {
+    const long long f = idx / nz;
+    const int j = (int) (idx - f * nz);
+    const int k = (j + nz / 2) & (nz - 1);
+    const float2 *X = spec + f * (nz + 1);
+    const float2 a = X[k], c = X[nz - k];
+    const float er = 0.5f * (a.x + c.x), ei = 0.5f * (a.y - c.y);
+    const float dr = 0.5f * (a.x - c.x), di = 0.5f * (a.y + c.y);
+    float sn, cs;
+    sincospif((float) k / (float) nz, &sn, &cs);
+    const float orr = dr * cs - di * sn, oi = dr * sn + di * cs;
+    const float zr = er - oi, zi = ei + orr;
+    const float pw = (zr * zr + zi * zi) * inv_nz;
+    rows[idx] = add ? rows[idx] + pw : pw;
+  }
+}
+
 static int sm_count() {
   int dev = 0, sms = 148;
   if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -223,9 +247,10 @@ extern "C" int glb_launch_zoom_split(const void *spec, int nz, long long nframes
 
 // The general path of complex frames: the interleaved stream seen as a real stream of 2n floats per frame at hop
 // 2 hop, the general spectrogram kernel's spectrum output X[k], k = 0..n, then zoom_split_kernel.  The zoom's frame
-// stage (host/zoom.c) and the I/Q spectrogram's non-fused launches (iq.cu).
+// stage (host/zoom.c) and the I/Q spectrogram's non-fused launches (iq.cu).  Multitaper (ntapers > 1): one spectrum
+// per taper into the same scratch plane, each followed by iq_mtm_split_kernel, which sums the tapers into the rows.
 extern "C" int glb_launch_iq_gram_general(const glb_iq_gram_args *a, void *stream) {
-  if (!a || !a->rows || a->nframes < 0) {
+  if (!a || !a->rows || a->nframes < 0 || a->ntapers < 0 || a->ntapers > 32) {
     glb_set_error("glb_launch_iq_gram_general: invalid arguments");
     return GLB_EINVAL;
   }
@@ -250,7 +275,25 @@ extern "C" int glb_launch_iq_gram_general(const glb_iq_gram_args *a, void *strea
   g.spectrum = (float *) a->scratch;
   g.tables = a->tables;
   g.general_only = 1;
-  int rc = glb_launch_gram(&g, stream);
-  if (rc != GLB_OK) return rc;
-  return glb_launch_zoom_split(a->scratch, a->n, a->nframes, a->rows, stream);
+  if (a->ntapers <= 1) {
+    int rc = glb_launch_gram(&g, stream);
+    if (rc != GLB_OK) return rc;
+    return glb_launch_zoom_split(a->scratch, a->n, a->nframes, a->rows, stream);
+  }
+  const int nz = a->n;
+  const long long total = a->nframes * nz;
+  long long ctas = (total + 255) / 256;
+  const long long cap = (long long) sm_count() * 16;
+  if (ctas > cap) ctas = cap;
+  for (int k = 0; k < a->ntapers; k++) {
+    g.tapers = a->taper + (size_t) k * 2 * nz;
+    g.taper_symmetric = (int) (((unsigned) a->taper_symmetric >> k) & 1u);
+    int rc = glb_launch_gram(&g, stream);
+    if (rc != GLB_OK) return rc;
+    iq_mtm_split_kernel<<<(int) ctas, 256, 0, (cudaStream_t) stream>>>((const float2 *) a->scratch, nz, a->nframes,
+                                                                         (float) (1.0 / nz), k > 0, a->rows);
+    ZCU(cudaGetLastError());
+    g_launches++;
+  }
+  return GLB_OK;
 }

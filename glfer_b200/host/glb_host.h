@@ -12,6 +12,9 @@
 double glb_bessel_i0(double x);
 void glb_window_table(int n, int window_type, float *w);
 int glb_dpss(int n, double nw, int kmax, double *tapers, double *lambda);
+/* host/iq.c: DPSS and [K'][2n] taper table of a complex multitaper plan (I/Q or zoom); sym: bit k = taper k mirror-symmetric */
+int glb_iq_mtm_tapers(int n, float mtm_w, int mtm_kmax, float taper_scale, double **h_tapers, double **h_lambda,
+                      float **table, int *sym);
 int glb_hop(int n, float overlap);
 /* the message slot of glfer_b200_last_error() (gram.c), for the other host units */
 int glb_host_fail(int code, const char *msg);

@@ -10,6 +10,10 @@
  * The display entries (glfer_iq_run_display*) bring back 8-bit levels instead of rows.  With a fixed range and no
  * RGB the spectrogram kernel maps its own powers (glb_iq_gram_args.levels) and no float row is ever stored;
  * otherwise each chunk's rows stay on the device and go through the display chain of host/display.c.
+ *
+ * Multitaper plans (glfer_iq_plan_create_mtm, and the zoom's) upload K' DPSS tapers, [K'][2n] floats, each scaled as
+ * the real multitaper plan scales its own (host/gram.c); the row sums the K' eigen-spectra.  They always bring float
+ * rows to the device: their waterfall goes through the display chain, for a fixed range too.
  */
 #include <math.h>
 #include <stdlib.h>
@@ -36,9 +40,12 @@ typedef struct {
 struct glfer_iq_plan {
   glfer_iq_config cfg;
   int hop;
-  float *d_taper;             /* [2n]: w[i] on both halves of complex sample i, times taper_scale */
-  int taper_sym;
+  float *d_taper;             /* [ntapers][2n]: w[i] (or v_k[i] / sqrt(lambda_k)) on both halves of complex sample i,
+                                 times taper_scale */
+  int taper_sym;              /* bit k: taper k is mirror-symmetric bit for bit */
   float taper_scale;
+  int ntapers;                /* 1: periodogram, K' = mtm_kmax + 1: multitaper */
+  double *h_tapers, *h_lambda;  /* multitaper: the unscaled DPSS [K'][n] and eigenvalues (glfer_iq_tapers) */
   void *tables;               /* FFT tables of the 2n-float frames */
   islot slot[ISLOT];
   glb_display disp;
@@ -82,20 +89,58 @@ void glfer_iq_plan_destroy(glfer_iq_plan *p)
   glb_display_free(&p->disp);
   glb_free(p->d_taper);
   glb_tables_destroy(p->tables);
+  free(p->h_tapers); free(p->h_lambda);
   free(p);
 }
 
-static int build_taper(glfer_iq_plan *p)
+/* The DPSS of a complex multitaper plan (I/Q or zoom) and its taper table, built as host/gram.c builds the real
+ * plan's: h_tapers [K'][n] and h_lambda [K'] from glb_dpss, table [K'][2n] floats with
+ * v_k[i] taper_scale / sqrt(lambda_k) on both floats of complex sample i, sym: bit k when taper k reads the same
+ * backwards bit for bit.  Validation as glfer_gram_plan_create; needs no device. */
+int glb_iq_mtm_tapers(int n, float mtm_w, int mtm_kmax, float taper_scale, double **h_tapers, double **h_lambda,
+                      float **table, int *sym)
+{
+  *h_tapers = NULL; *h_lambda = NULL; *table = NULL; *sym = 0;
+  if (mtm_kmax < 0 || mtm_kmax > 31) return glb_host_fail(GLFER_EINVAL, "mtm_kmax must be in 0..31 (32 eigenvectors exist)");
+  if (!(mtm_w > 0.0f)) return glb_host_fail(GLFER_EINVAL, "mtm_w must be > 0");
+  const int K = mtm_kmax + 1;
+  double *tap = malloc(sizeof(double) * (size_t) K * n);
+  double *lam = malloc(sizeof(double) * K);
+  float *tab = malloc(sizeof(float) * (size_t) K * 2 * n);
+  if (!tap || !lam || !tab) { free(tap); free(lam); free(tab); return glb_host_fail(GLFER_ENOMEM, "out of memory"); }
+  /* the real plan's call: mtm_params_t.w is a float promoted to double */
+  if (glb_dpss(n, (double) mtm_w, mtm_kmax, tap, lam) != 0) {
+    free(tap); free(lam); free(tab);
+    return glb_host_fail(GLFER_EINVAL, "DPSS computation failed");
+  }
+  for (int k = 0; k < K; k++) {
+    if (!(lam[k] > 0.0)) {
+      free(tap); free(lam); free(tab);
+      return glb_host_fail(GLFER_EINVAL, "DPSS eigenvalue not positive: reduce mtm_kmax or raise mtm_w");
+    }
+    const double g = (double) taper_scale / sqrt(lam[k]);
+    float *t = tab + (size_t) k * 2 * n;
+    for (int i = 0; i < n; i++) t[2 * i] = t[2 * i + 1] = (float) (tap[(size_t) k * n + i] * g);
+    int s = 1;
+    for (int i = 0; i < n && s; i++)
+      if (memcmp(&t[i], &t[2 * n - 1 - i], sizeof(float)) != 0) s = 0;
+    *sym |= s << k;
+  }
+  *h_tapers = tap; *h_lambda = lam; *table = tab;
+  return 0;
+}
+
+/* tab: NULL (periodogram: the window), or the multitaper table of glb_iq_mtm_tapers */
+static int build_taper(glfer_iq_plan *p, const float *tab)
 {
   const int n = p->cfg.n;
   float *w = malloc(sizeof(float) * n);
   float *taper = malloc(sizeof(float) * 2 * n);
   int rc = 0;
   if (!w || !taper) rc = glb_host_fail(GLFER_ENOMEM, "out of memory");
-  if (rc == 0) {
+  if (rc == 0 && !tab) {
     /* as the zoom (host/zoom.c): the window on both floats of a complex sample, times 1 / (2 sqrt(2n)) */
     glb_window_table(n, p->cfg.window_type, w);
-    p->taper_scale = (float) (1.0 / (2.0 * sqrt(2.0 * n)));
     for (int i = 0; i < n; i++) {
       const double wi = p->cfg.window_type == RECTANGULAR_WINDOW ? 1.0 : (double) w[i];
       taper[2 * i] = taper[2 * i + 1] = (float) (wi * (double) p->taper_scale);
@@ -103,15 +148,17 @@ static int build_taper(glfer_iq_plan *p)
     p->taper_sym = 1;
     for (int i = 0; i < n; i++)
       if (memcmp(&taper[i], &taper[2 * n - 1 - i], sizeof(float)) != 0) { p->taper_sym = 0; break; }
-    rc = glb_host_shim(glb_malloc((void **) &p->d_taper, sizeof(float) * 2 * (size_t) n));
-    if (rc == 0) rc = glb_host_shim(glb_memcpy_h2d(p->d_taper, taper, sizeof(float) * 2 * (size_t) n, NULL));
-    if (rc == 0) rc = glb_host_shim(glb_tables_create(2 * n, &p->tables));
+    tab = taper;
   }
+  const size_t bytes = sizeof(float) * 2 * (size_t) n * p->ntapers;
+  if (rc == 0) rc = glb_host_shim(glb_malloc((void **) &p->d_taper, bytes));
+  if (rc == 0) rc = glb_host_shim(glb_memcpy_h2d(p->d_taper, tab, bytes, NULL));
+  if (rc == 0) rc = glb_host_shim(glb_tables_create(2 * n, &p->tables));
   free(w); free(taper);
   return rc;
 }
 
-int glfer_iq_plan_create(const glfer_iq_config *cfg, glfer_iq_plan **out)
+static int iq_plan_create(const glfer_iq_config *cfg, int mtm, float mtm_w, int mtm_kmax, glfer_iq_plan **out)
 {
   glb_host_clear_error();
   if (!cfg || !out) return glb_host_fail(GLFER_EINVAL, "null argument");
@@ -121,17 +168,37 @@ int glfer_iq_plan_create(const glfer_iq_config *cfg, glfer_iq_plan **out)
   if (cfg->window_type < 0 || cfg->window_type > 7) return glb_host_fail(GLFER_EINVAL, "unknown window type");
   const int hop = glb_hop(cfg->n, cfg->overlap);
   if (hop < 1 || hop > cfg->n) return glb_host_fail(GLFER_EINVAL, "overlap leaves no new samples per block");
+  const float taper_scale = (float) (1.0 / (2.0 * sqrt(2.0 * cfg->n)));
+  double *h_tapers = NULL, *h_lambda = NULL;
+  float *tab = NULL;
+  int sym = 0;
+  if (mtm) {
+    const int rc = glb_iq_mtm_tapers(cfg->n, mtm_w, mtm_kmax, taper_scale, &h_tapers, &h_lambda, &tab, &sym);
+    if (rc != 0) return rc;
+  }
   int ndev = 0;
+  int rc = 0;
   if (glb_device_count(&ndev) != GLB_OK || ndev < 1)
-    return glb_host_fail(GLFER_ENODEV, "no CUDA device (libglfer_b200 has no CPU fallback)");
-  if (cfg->device < 0 || cfg->device >= ndev) return glb_host_fail(GLFER_EINVAL, "device ordinal out of range");
-  ITRY(glb_set_device(cfg->device));
-
-  glfer_iq_plan *p = calloc(1, sizeof *p);
-  if (!p) return glb_host_fail(GLFER_ENOMEM, "out of memory");
+    rc = glb_host_fail(GLFER_ENODEV, "no CUDA device (libglfer_b200 has no CPU fallback)");
+  else if (cfg->device < 0 || cfg->device >= ndev)
+    rc = glb_host_fail(GLFER_EINVAL, "device ordinal out of range");
+  else
+    rc = glb_host_shim(glb_set_device(cfg->device));
+  glfer_iq_plan *p = rc == 0 ? calloc(1, sizeof *p) : NULL;
+  if (rc == 0 && !p) rc = glb_host_fail(GLFER_ENOMEM, "out of memory");
+  if (rc != 0) {
+    free(h_tapers); free(h_lambda); free(tab);
+    return rc;
+  }
   p->cfg = *cfg;
   p->hop = hop;
-  int rc = build_taper(p);
+  p->taper_scale = taper_scale;
+  p->ntapers = mtm ? mtm_kmax + 1 : 1;
+  p->h_tapers = h_tapers;
+  p->h_lambda = h_lambda;
+  p->taper_sym = sym;
+  rc = build_taper(p, tab);
+  free(tab);
   for (int i = 0; i < ISLOT && rc == 0; i++) {
     rc = glb_host_shim(glb_stream_create(&p->slot[i].stream));
     if (rc == 0) rc = glb_host_shim(glb_event_create(&p->slot[i].disp.ev_agc));
@@ -146,6 +213,25 @@ int glfer_iq_plan_create(const glfer_iq_config *cfg, glfer_iq_plan **out)
   }
   *out = p;
   return GLFER_OK;
+}
+
+int glfer_iq_plan_create(const glfer_iq_config *cfg, glfer_iq_plan **out)
+{
+  return iq_plan_create(cfg, 0, 0.0f, 0, out);
+}
+
+int glfer_iq_plan_create_mtm(const glfer_iq_config *cfg, float mtm_w, int mtm_kmax, glfer_iq_plan **out)
+{
+  return iq_plan_create(cfg, 1, mtm_w, mtm_kmax, out);
+}
+
+int glfer_iq_tapers(const glfer_iq_plan *p, double *tapers, double *lambda)
+{
+  if (!p || !tapers || !lambda) return glb_host_fail(GLFER_EINVAL, "null argument");
+  if (!p->h_tapers) return glb_host_fail(GLFER_EINVAL, "plan is not a multitaper plan");
+  memcpy(tapers, p->h_tapers, sizeof(double) * (size_t) p->ntapers * p->cfg.n);
+  memcpy(lambda, p->h_lambda, sizeof(double) * p->ntapers);
+  return 0;
 }
 
 /* grow-only device buffers */
@@ -188,7 +274,7 @@ static int iq_chunk(glfer_iq_plan *p, islot *s, const void *src, int pcm16, long
     ITRY(glb_memcpy_h2d(s->d_in, (const float *) src + 2 * (lo - origin), sizeof(float) * 2 * (size_t) cnt, s->stream));
   }
   if (!fl) ITRY(iensure((void **) &s->d_rows, &s->rows_cap, (size_t) (cn * n), sizeof(float)));
-  const long long sb = glb_iq_gram_scratch_bytes((int) n, (int) hop, cn, fl != NULL);
+  const long long sb = glb_iq_gram_scratch_bytes((int) n, (int) hop, cn, fl != NULL, p->ntapers);
   if (sb > 0) ITRY(iensure(&s->d_scratch, &s->scratch_cap, (size_t) sb, 1));
   glb_iq_gram_args g;
   memset(&g, 0, sizeof g);
@@ -200,6 +286,7 @@ static int iq_chunk(glfer_iq_plan *p, islot *s, const void *src, int pcm16, long
   g.taper = p->d_taper;
   g.taper_symmetric = p->taper_sym;
   g.taper_scale = p->taper_scale;
+  g.ntapers = p->ntapers;
   g.first_frame = c0;
   g.nframes = cn;
   g.rows = fl ? NULL : s->d_rows;
@@ -289,8 +376,8 @@ static int iq_run_display_impl(glfer_iq_plan *p, const void *src, int pcm16, lon
   const int n = p->cfg.n;
   glb_display_run dr;
   ITRY(glb_display_begin(&p->disp, &dr, dc, agc_state, nframes, range_out != NULL, p->slot[0].stream));
-  /* fixed range without RGB: the spectrogram kernel writes the levels itself */
-  const int fuse = glb_host_fused_levels() && !dc->autoscale && !rgb;
+  /* fixed range without RGB: the spectrogram kernel writes the levels itself (periodogram plans only) */
+  const int fuse = glb_host_fused_levels() && !dc->autoscale && !rgb && p->ntapers == 1;
   const long long cf = iq_chunk_frames(p);
   int rc = 0, ci = 0;
   long long done = 0;

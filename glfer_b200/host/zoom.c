@@ -16,6 +16,9 @@
  *
  * The display entries (glfer_zoom_run_display*) keep each chunk's rows on the device and map them through the
  * display chain of host/display.c: only the 8-bit levels (or RGB) come back.
+ *
+ * Multitaper plans (glfer_zoom_plan_create_mtm / _create_iq_mtm) replace the window by K' DPSS tapers
+ * (glb_iq_mtm_tapers, host/iq.c); the frame stage then runs one spectrum per taper into the same scratch plane.
  */
 #include <math.h>
 #include <stdlib.h>
@@ -45,9 +48,12 @@ struct glfer_zoom_plan {
   int hop, K;
   unsigned step;
   float *d_taps;              /* [33 D] (re, im) pairs: g[j] = h[K - j] e^{+2 pi i phi(K - j)}, zero past 2K */
-  float *d_taper;             /* [2n]: w[i] on both halves of complex sample i, times taper_scale */
-  int taper_sym;
+  float *d_taper;             /* [ntapers][2n]: w[i] (or v_k[i] / sqrt(lambda_k)) on both halves of complex sample i,
+                                 times taper_scale */
+  int taper_sym;              /* bit k: taper k is mirror-symmetric bit for bit */
   float taper_scale;
+  int ntapers;                /* 1: periodogram, K' = mtm_kmax + 1: multitaper */
+  double *h_tapers, *h_lambda;  /* multitaper: the unscaled DPSS [K'][n] and eigenvalues (glfer_zoom_tapers) */
   int iq;                     /* 1: complex (I, Q) input (glfer_zoom_plan_create_iq), signed centre */
   void *tables;               /* FFT tables of the 2n-point real transform */
   zslot slot[ZSLOT];
@@ -145,10 +151,12 @@ void glfer_zoom_plan_destroy(glfer_zoom_plan *p)
   glb_free(p->d_taps);
   glb_free(p->d_taper);
   glb_tables_destroy(p->tables);
+  free(p->h_tapers); free(p->h_lambda);
   free(p);
 }
 
-static int build_tables(glfer_zoom_plan *p)
+/* mtab: NULL (periodogram: the window), or the multitaper table of glb_iq_mtm_tapers */
+static int build_tables(glfer_zoom_plan *p, const float *mtab)
 {
   const glfer_zoom_config *c = &p->cfg;
   const int D = c->decim, K = p->K, n = c->n;
@@ -167,27 +175,31 @@ static int build_tables(glfer_zoom_plan *p)
       g[2 * j] = (float) ((double) h[j] * cos(a));
       g[2 * j + 1] = (float) ((double) h[j] * sin(a));
     }
-    glb_window_table(n, c->window_type, w);
-    p->taper_scale = (float) (1.0 / (2.0 * sqrt(2.0 * n)));
-    for (int i = 0; i < n; i++) {
-      /* as the spectrogram: a rectangular window is not applied (weight 1) */
-      const double wi = c->window_type == RECTANGULAR_WINDOW ? 1.0 : (double) w[i];
-      taper[2 * i] = taper[2 * i + 1] = (float) (wi * (double) p->taper_scale);
+    if (!mtab) {
+      glb_window_table(n, c->window_type, w);
+      for (int i = 0; i < n; i++) {
+        /* as the spectrogram: a rectangular window is not applied (weight 1) */
+        const double wi = c->window_type == RECTANGULAR_WINDOW ? 1.0 : (double) w[i];
+        taper[2 * i] = taper[2 * i + 1] = (float) (wi * (double) p->taper_scale);
+      }
+      p->taper_sym = 1;
+      for (int i = 0; i < n; i++)
+        if (memcmp(&taper[i], &taper[2 * n - 1 - i], sizeof(float)) != 0) { p->taper_sym = 0; break; }
+      mtab = taper;
     }
-    p->taper_sym = 1;
-    for (int i = 0; i < n; i++)
-      if (memcmp(&taper[i], &taper[2 * n - 1 - i], sizeof(float)) != 0) { p->taper_sym = 0; break; }
+    const size_t tbytes = sizeof(float) * 2 * (size_t) n * p->ntapers;
     rc = glb_host_shim(glb_malloc((void **) &p->d_taps, sizeof(float) * 66 * (size_t) D));
     if (rc == 0) rc = glb_host_shim(glb_memcpy_h2d(p->d_taps, g, sizeof(float) * 66 * (size_t) D, NULL));
-    if (rc == 0) rc = glb_host_shim(glb_malloc((void **) &p->d_taper, sizeof(float) * 2 * (size_t) n));
-    if (rc == 0) rc = glb_host_shim(glb_memcpy_h2d(p->d_taper, taper, sizeof(float) * 2 * (size_t) n, NULL));
+    if (rc == 0) rc = glb_host_shim(glb_malloc((void **) &p->d_taper, tbytes));
+    if (rc == 0) rc = glb_host_shim(glb_memcpy_h2d(p->d_taper, mtab, tbytes, NULL));
     if (rc == 0) rc = glb_host_shim(glb_tables_create(2 * n, &p->tables));
   }
   free(h); free(g); free(w); free(taper);
   return rc;
 }
 
-static int zoom_plan_create(const glfer_zoom_config *cfg, int iq, glfer_zoom_plan **out)
+static int zoom_plan_create(const glfer_zoom_config *cfg, int iq, int mtm, float mtm_w, int mtm_kmax,
+                            glfer_zoom_plan **out)
 {
   glb_host_clear_error();
   if (!cfg || !out) return glb_host_fail(GLFER_EINVAL, "null argument");
@@ -203,21 +215,41 @@ static int zoom_plan_create(const glfer_zoom_config *cfg, int iq, glfer_zoom_pla
     return glb_host_fail(GLFER_EINVAL, "centre frequency must be in [0, sample_rate / 2]");
   if (iq && !(cfg->center_hz >= -0.5 * cfg->sample_rate && cfg->center_hz <= 0.5 * cfg->sample_rate))
     return glb_host_fail(GLFER_EINVAL, "I/Q centre frequency must be in [-sample_rate / 2, sample_rate / 2]");
+  const float taper_scale = (float) (1.0 / (2.0 * sqrt(2.0 * cfg->n)));
+  double *h_tapers = NULL, *h_lambda = NULL;
+  float *mtab = NULL;
+  int sym = 0;
+  if (mtm) {
+    const int rc = glb_iq_mtm_tapers(cfg->n, mtm_w, mtm_kmax, taper_scale, &h_tapers, &h_lambda, &mtab, &sym);
+    if (rc != 0) return rc;
+  }
   int ndev = 0;
+  int rc = 0;
   if (glb_device_count(&ndev) != GLB_OK || ndev < 1)
-    return glb_host_fail(GLFER_ENODEV, "no CUDA device (libglfer_b200 has no CPU fallback)");
-  if (cfg->device < 0 || cfg->device >= ndev) return glb_host_fail(GLFER_EINVAL, "device ordinal out of range");
-  ZTRY(glb_set_device(cfg->device));
-
-  glfer_zoom_plan *p = calloc(1, sizeof *p);
-  if (!p) return glb_host_fail(GLFER_ENOMEM, "out of memory");
+    rc = glb_host_fail(GLFER_ENODEV, "no CUDA device (libglfer_b200 has no CPU fallback)");
+  else if (cfg->device < 0 || cfg->device >= ndev)
+    rc = glb_host_fail(GLFER_EINVAL, "device ordinal out of range");
+  else
+    rc = glb_host_shim(glb_set_device(cfg->device));
+  glfer_zoom_plan *p = rc == 0 ? calloc(1, sizeof *p) : NULL;
+  if (rc == 0 && !p) rc = glb_host_fail(GLFER_ENOMEM, "out of memory");
+  if (rc != 0) {
+    free(h_tapers); free(h_lambda); free(mtab);
+    return rc;
+  }
   p->cfg = *cfg;
   p->hop = hop;
   p->K = 16 * cfg->decim;
   p->iq = iq;
   /* modulo 2^32: a negative I/Q centre is a step above 2^31 */
   p->step = (unsigned) (unsigned long long) llround(cfg->center_hz / cfg->sample_rate * 4294967296.0);
-  int rc = build_tables(p);
+  p->taper_scale = taper_scale;
+  p->ntapers = mtm ? mtm_kmax + 1 : 1;
+  p->h_tapers = h_tapers;
+  p->h_lambda = h_lambda;
+  p->taper_sym = sym;
+  rc = build_tables(p, mtab);
+  free(mtab);
   for (int i = 0; i < ZSLOT && rc == 0; i++) {
     rc = glb_host_shim(glb_stream_create(&p->slot[i].stream));
     if (rc == 0) rc = glb_host_shim(glb_event_create(&p->slot[i].ev_dec));
@@ -237,12 +269,31 @@ static int zoom_plan_create(const glfer_zoom_config *cfg, int iq, glfer_zoom_pla
 
 int glfer_zoom_plan_create(const glfer_zoom_config *cfg, glfer_zoom_plan **out)
 {
-  return zoom_plan_create(cfg, 0, out);
+  return zoom_plan_create(cfg, 0, 0, 0.0f, 0, out);
 }
 
 int glfer_zoom_plan_create_iq(const glfer_zoom_config *cfg, glfer_zoom_plan **out)
 {
-  return zoom_plan_create(cfg, 1, out);
+  return zoom_plan_create(cfg, 1, 0, 0.0f, 0, out);
+}
+
+int glfer_zoom_plan_create_mtm(const glfer_zoom_config *cfg, float mtm_w, int mtm_kmax, glfer_zoom_plan **out)
+{
+  return zoom_plan_create(cfg, 0, 1, mtm_w, mtm_kmax, out);
+}
+
+int glfer_zoom_plan_create_iq_mtm(const glfer_zoom_config *cfg, float mtm_w, int mtm_kmax, glfer_zoom_plan **out)
+{
+  return zoom_plan_create(cfg, 1, 1, mtm_w, mtm_kmax, out);
+}
+
+int glfer_zoom_tapers(const glfer_zoom_plan *p, double *tapers, double *lambda)
+{
+  if (!p || !tapers || !lambda) return glb_host_fail(GLFER_EINVAL, "null argument");
+  if (!p->h_tapers) return glb_host_fail(GLFER_EINVAL, "plan is not a multitaper plan");
+  memcpy(tapers, p->h_tapers, sizeof(double) * (size_t) p->ntapers * p->cfg.n);
+  memcpy(lambda, p->h_lambda, sizeof(double) * p->ntapers);
+  return 0;
 }
 
 /* grow-only device buffers */
@@ -318,6 +369,7 @@ static int zoom_chunk(glfer_zoom_plan *p, zslot *s, const zslot *prev, const voi
   g.taper = p->d_taper;
   g.taper_symmetric = p->taper_sym;
   g.taper_scale = p->taper_scale;
+  g.ntapers = p->ntapers;
   g.first_frame = c0;
   g.nframes = cn;
   g.rows = s->d_rows;

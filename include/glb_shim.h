@@ -215,14 +215,16 @@ int glb_launch_zoom_decim_iq(const void *x, int pcm16, long long origin, long lo
 /* Rows of complex frames (I/Q spectrogram, zoom frame stage) of an interleaved (I, Q) stream z:
  *     rows[f - first_frame][j] = |sum_i w[i] z[f hop - (n - hop) + i] e^{-2 pi i (j - n/2) i / n}|^2 / n
  * The taper holds w[i] taper_scale on both floats of complex sample i, with taper_scale = (float) (1 / (2 sqrt(2 n)))
- * (the fused kernel folds 1 / (n taper_scale^2) = 8 into its epilogue). */
+ * (the fused kernel folds 1 / (n taper_scale^2) = 8 into its epilogue).
+ * Multitaper (ntapers = K' > 1): taper points at [K'][2n] floats, taper k holding v_k[i] taper_scale / sqrt(lambda_k) on
+ * both floats of complex sample i, and the row is the sum over k = 0..K'-1, in that order, of the rows of each taper. */
 typedef struct {
   int n;                       /* complex frame length: power of two, 32..16384 */
   int hop;                     /* complex samples per frame */
   const float *samples;        /* device: interleaved (I, Q) of complex samples [origin, origin + count) */
   long long origin, count;     /* complex samples; indices < 0 read as 0 */
-  const float *taper;          /* device: [2n] floats */
-  int taper_symmetric;         /* taper[i] == taper[2n - 1 - i] bit for bit */
+  const float *taper;          /* device: [2n] floats, or [ntapers][2n] */
+  int taper_symmetric;         /* bit k: taper k satisfies taper[i] == taper[2n - 1 - i] bit for bit (one taper: 0 or 1) */
   float taper_scale;
   long long first_frame, nframes;
   float *rows;                 /* device out: [nframes][n] */
@@ -237,6 +239,7 @@ typedef struct {
   const unsigned char *level_lut;   /* device: level of every integer dB value (log scales) or NULL */
   float level_min, level_max;  /* display_min / display_max (dB in the log scales) */
   float level_thr;             /* opt.thr_level / 100 */
+  int ntapers;                 /* 0 or 1: periodogram; K' = 2..32: multitaper (no levels: GLB_EINVAL) */
 } glb_iq_gram_args;
 /* The one entry of the I/Q spectrogram: the fused kernel (iq.cu, regular geometry n = 32..8192, hop = (n/16) << s
  * with n - hop a multiple of hop; needs an even origin, a 16-byte aligned samples pointer and samples that cover
@@ -245,10 +248,12 @@ typedef struct {
  * maps them with glb_launch_levels. */
 int glb_launch_iq_gram(const glb_iq_gram_args *a, void *stream);
 /* device scratch glb_launch_iq_gram needs for nframes frames (0 when the fused kernel serves the geometry);
- * levels: 1 when the launch writes levels (the general path then also holds the float rows) */
-long long glb_iq_gram_scratch_bytes(int n, int hop, long long nframes, int levels);
+ * levels: 1 when the launch writes levels (the general path then also holds the float rows); ntapers as in the
+ * arguments (the general path reuses one spectrum plane for all tapers, so the size does not grow with it) */
+long long glb_iq_gram_scratch_bytes(int n, int hop, long long nframes, int levels, int ntapers);
 /* the general path: the general spectrogram kernel's spectrum output on the 2n-float frames (into scratch, at
- * least nframes (n + 1) (re, im) pairs), then glb_launch_zoom_split */
+ * least nframes (n + 1) (re, im) pairs), then glb_launch_zoom_split; multitaper: that spectrum once per taper, each
+ * followed by a split that stores (taper 0) or adds (the others) its powers into the rows */
 int glb_launch_iq_gram_general(const glb_iq_gram_args *a, void *stream);
 
 /* counters */

@@ -298,6 +298,31 @@ int glfer_iq_run(glfer_iq_plan *plan, const float *iq, long long origin, long lo
 int glfer_iq_run_pcm16(glfer_iq_plan *plan, const short *iq, long long origin, long long count,
                        long long first_frame, long long nframes, float *rows);
 
+/* ---- multitaper I/Q and zoom plans ----
+ * Thomson's multitaper estimator on the complex frames of an I/Q or zoom plan.  Frame f is the plan's frame above
+ * (complex samples [f hop - (n - hop), f hop + hop) of z, or of the decimated y for a zoom, zeros before index 0),
+ * and its row is
+ *     P[f][j] = sum_{k=0..K'-1} |sum_i v_k[i] z_f[i] e^{-2 pi i (j - n/2) i / n}|^2 / (n lambda_k),   j = 0..n-1,
+ * K' = mtm_kmax + 1, with v_k, lambda_k = glb_dpss(n, mtm_w, mtm_kmax): the unit-energy DPSS tapers and eigenvalues
+ * that a real GLFER_MODE_MTM plan of the same n uses (NW = mtm_w as gl_dpss takes it).  The weights are 1 / lambda_k,
+ * not normalised, as mtm_do weighs them (mtm.c:214-219): an I/Q multitaper row of (x, 0) is the real multitaper row
+ * of x on its positive half.  So on white noise a multitaper row sits about 10 log10(sum_k 1 / lambda_k) dB above the
+ * periodogram row of the same n (the tapers and the spectrogram windows all have unit energy; the rectangular window,
+ * all ones, has energy n instead): +9.3 dB at NW = 4, K' = 8 (sum_k 1 / lambda_k = 8.51), +23.8 dB at NW = 2.5,
+ * K' = 8, where the last tapers have small eigenvalues.  A fixed display range chosen for periodogram rows must move
+ * up by that much.
+ * Rows are fft-shifted as before (DC at n/2; zoom bin j at centre + (j - n/2) sample_rate / (D n)); window_type is
+ * ignored, everything else in the config means what it means above.  GLFER_EINVAL for mtm_kmax outside 0..31, mtm_w
+ * not > 0, or a DPSS eigenvalue that is not positive.  Every run, run_display and query entry point serves these
+ * plans unchanged (run_display maps the multitaper rows), and the zoom's real and I/Q entry points keep rejecting
+ * each other's plans. */
+int glfer_iq_plan_create_mtm(const glfer_iq_config *cfg, float mtm_w, int mtm_kmax, glfer_iq_plan **plan);
+int glfer_zoom_plan_create_mtm(const glfer_zoom_config *cfg, float mtm_w, int mtm_kmax, glfer_zoom_plan **plan);
+int glfer_zoom_plan_create_iq_mtm(const glfer_zoom_config *cfg, float mtm_w, int mtm_kmax, glfer_zoom_plan **plan);
+/* the plan's tapers [mtm_kmax + 1][n] and eigenvalues [mtm_kmax + 1] before scaling; GLFER_EINVAL on a periodogram plan */
+int glfer_iq_tapers(const glfer_iq_plan *plan, double *tapers, double *lambda);
+int glfer_zoom_tapers(const glfer_zoom_plan *plan, double *tapers, double *lambda);
+
 /* ---- display output of I/Q and zoom plans ----
  * The waterfall of the plan's own rows, as glfer_gram_run_display gives it for real audio: levels, rgb, agc_state
  * and display_range as there, and exactly main_window_draw's mapping (g_main.c:1109-1229) of the rows that
@@ -308,8 +333,9 @@ int glfer_iq_run_pcm16(glfer_iq_plan *plan, const short *iq, long long origin, l
  * plan's required span, and (zoom) a real entry point with an I/Q plan or the reverse.
  * The I/Q centre -- the receiver's LO leakage, at row position n/2 -- is a bin like any other: a strong spike there
  * can be the row's largest bin and so set the AGC's upper level, as it would in the reference's mapping.
- * I/Q plans with a fixed range and no RGB compute the levels in the spectrogram kernel itself (no float row is
- * stored); the other cases map device rows, and only the levels (or RGB) and the range cross PCIe. */
+ * Periodogram I/Q plans with a fixed range and no RGB compute the levels in the spectrogram kernel itself (no float
+ * row is stored); the other cases, multitaper plans always, map device rows, and only the levels (or RGB) and the
+ * range cross PCIe. */
 int glfer_iq_run_display(glfer_iq_plan *plan, const float *iq, long long origin, long long count,
                          long long first_frame, long long nframes, const glfer_display_config *dc,
                          float *agc_state, unsigned char *levels, unsigned char *rgb, float *display_range);
