@@ -163,6 +163,9 @@ def lib() -> C.CDLL:
         l.glfer_zoom_tapers.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p]
         l.glfer_iq_run.argtypes = zoom_args
         l.glfer_iq_run_pcm16.argtypes = zoom_args
+        for name in ("glfer_iq_run_mtm_ftest", "glfer_iq_run_mtm_ftest_pcm16", "glfer_zoom_run_mtm_ftest",
+                     "glfer_zoom_run_mtm_ftest_pcm16", "glfer_zoom_run_iq_mtm_ftest", "glfer_zoom_run_iq_mtm_ftest_pcm16"):
+            getattr(l, name).argtypes = zoom_args + [C.c_void_p]
         for name in ("glfer_iq_run_display", "glfer_iq_run_display_pcm16", "glfer_zoom_run_display",
                      "glfer_zoom_run_display_pcm16", "glfer_zoom_run_display_iq", "glfer_zoom_run_display_iq_pcm16"):
             getattr(l, name).argtypes = disp_args
@@ -549,6 +552,22 @@ class ZoomPlan:
         _check(fn(self._h, samples.ctypes.data, origin, len(samples), first_frame, nframes, rows.ctypes.data))
         return rows
 
+    def run_mtm_ftest(self, samples: np.ndarray, origin: int = 0, first_frame: int = 0, nframes: int | None = None,
+                      want_psd: bool = True, want_ftest: bool = True):
+        """glfer_zoom_run[_iq]_mtm_ftest[_pcm16]: the multitaper rows and the harmonic F-test rows, [nframes][n] each
+        (None when not wanted), of a multitaper plan.  Input formats of run."""
+        if self.iq:
+            ptr, count, pcm = _iq_samples(samples)
+            fn = lib().glfer_zoom_run_iq_mtm_ftest_pcm16 if pcm else lib().glfer_zoom_run_iq_mtm_ftest
+        else:
+            pcm = samples.dtype == np.int16
+            assert samples.flags["C_CONTIGUOUS"] and (pcm or samples.dtype == np.float32)
+            ptr, count = samples.ctypes.data, len(samples)
+            fn = lib().glfer_zoom_run_mtm_ftest_pcm16 if pcm else lib().glfer_zoom_run_mtm_ftest
+        if nframes is None:
+            nframes = self.num_frames(origin + count) - first_frame
+        return _run_ftest(fn, self._h, ptr, origin, count, first_frame, nframes, self.bins, want_psd, want_ftest)
+
     def run_display(self, samples: np.ndarray, log_scale=True, autoscale=True, max_level_db=-20.0, min_level_db=-80.0,
                     thr_level=0.0, colortab: np.ndarray | None = None, origin: int = 0, first_frame: int = 0,
                     nframes: int | None = None, agc_state: np.ndarray | None = None, want_rgb: bool = False,
@@ -625,6 +644,16 @@ class IqPlan:
         _check(fn(self._h, ptr, origin, count, first_frame, nframes, rows.ctypes.data))
         return rows
 
+    def run_mtm_ftest(self, iq: np.ndarray, origin: int = 0, first_frame: int = 0, nframes: int | None = None,
+                      want_psd: bool = True, want_ftest: bool = True):
+        """glfer_iq_run_mtm_ftest / _pcm16: the multitaper rows and the harmonic F-test rows, [nframes][n] each (None
+        when not wanted), of a multitaper plan.  Input formats of run."""
+        ptr, count, pcm = _iq_samples(iq)
+        if nframes is None:
+            nframes = self.num_frames(origin + count) - first_frame
+        fn = lib().glfer_iq_run_mtm_ftest_pcm16 if pcm else lib().glfer_iq_run_mtm_ftest
+        return _run_ftest(fn, self._h, ptr, origin, count, first_frame, nframes, self.bins, want_psd, want_ftest)
+
     def run_display(self, iq: np.ndarray, log_scale=True, autoscale=True, max_level_db=-20.0, min_level_db=-80.0,
                     thr_level=0.0, colortab: np.ndarray | None = None, origin: int = 0, first_frame: int = 0,
                     nframes: int | None = None, agc_state: np.ndarray | None = None, want_rgb: bool = False,
@@ -637,6 +666,13 @@ class IqPlan:
         fn = lib().glfer_iq_run_display_pcm16 if pcm else lib().glfer_iq_run_display
         return _run_display(fn, self._h, ptr, count, self.bins, nframes, log_scale, autoscale, max_level_db, min_level_db,
                             thr_level, colortab, origin, first_frame, agc_state, want_rgb, out, want_range)
+
+
+def _run_ftest(fn, h, ptr, origin, count, first_frame, nframes, bins, want_psd, want_ftest):
+    psd = np.empty((nframes, bins), np.float32) if want_psd else None
+    ft = np.empty((nframes, bins), np.float32) if want_ftest else None
+    _check(fn(h, ptr, origin, count, first_frame, nframes, _ptr(psd), _ptr(ft)))
+    return dict(psd=psd, ftest=ft)
 
 
 def zoom_taps(decim: int) -> np.ndarray:

@@ -43,6 +43,46 @@ GLB_HD void iq_add_power(float2 *v, int t, float scale, float (&acc)[17]) {
   }
 }
 
+// Harmonic F-test (gram_iq_ftest_kernel, iq.cu; the general path's split kernels, zoom.cu).  The hn transform leaves
+// mu by slot (the slots of iq_emit_power) at mu[slot * stride]: stride 1 for an array in registers, the thread count
+// for a per-thread column of shared memory.  Each taper's transform then adds its power to acc exactly as
+// iq_add_power does, and its residual to den.  The uploaded taper carries taper_scale / sqrt(lambda_k): sl = sqrt(lambda_k)
+// undoes the per-taper factor, the common taper_scale cancels in F.  The residual is formed directly: the expanded
+// sum |y_k|^2 - |sum U0_k y_k|^2 / S needs no mu but cancels in FP32 on exactly the bins where F is large.
+GLB_HD float iq_ftest_resid(float2 z, float2 mu, float u0, float sl) {
+  const float rr = z.x * sl - mu.x * u0, ri = z.y * sl - mu.y * u0;
+  return rr * rr + ri * ri;
+}
+// fnum = (K' - 1) S; IEEE division (0 / 0 is NaN, as on an all-zero frame)
+GLB_HD float iq_ftest_value(float2 mu, float den, float fnum) { return fnum * norm2(mu) / den; }
+
+template <int M, bool T0 = true>
+GLB_HD void iq_emit_mu(float2 *v, int t, float2 *mu, int stride) {
+  if (T0 && t == 0) mu[16 * stride] = thread0_fixup(v);
+#pragma unroll
+  for (int rp = 0; rp < 8; rp++) {
+    mu[2 * rp * stride] = v[rp];
+    mu[(2 * rp + 1) * stride] = v[15 - rp];
+  }
+}
+
+template <int M, bool T0 = true>
+GLB_HD void iq_add_ftest(float2 *v, int t, float scale, float u0, float sl, const float2 *mu, int stride,
+                         float (&acc)[17], float (&den)[17]) {
+  if (T0 && t == 0) {
+    const float2 z = thread0_fixup(v);
+    acc[16] += scale * norm2(z);
+    den[16] += iq_ftest_resid(z, mu[16 * stride], u0, sl);
+  }
+#pragma unroll
+  for (int rp = 0; rp < 8; rp++) {
+    acc[2 * rp] += scale * norm2(v[rp]);
+    acc[2 * rp + 1] += scale * norm2(v[15 - rp]);
+    den[2 * rp] += iq_ftest_resid(v[rp], mu[2 * rp * stride], u0, sl);
+    den[2 * rp + 1] += iq_ftest_resid(v[15 - rp], mu[(2 * rp + 1) * stride], u0, sl);
+  }
+}
+
 template <int M> GLB_HD bool iq_slot_stored(int t, int slot) { return slot == 16 ? t == 0 : !(t == 0 && slot == 1); }
 
 // Row positions as four per-thread bases plus compile-time offsets (the stores of a warp cover 32

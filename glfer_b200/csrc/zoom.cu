@@ -20,11 +20,14 @@
 //                         Z[k] = E + iO of the complex frame -> |Z|^2 / Nz in fft-shifted bin order.
 //   iq_mtm_split_kernel   the same split for one taper of a multitaper row: taper 0 stores |Z_0|^2 / Nz, taper
 //                         k > 0 adds |Z_k|^2 / Nz to the row, so the tapers are summed in the order k = 0..K'-1.
+//   iq_ftest_*_kernel     the harmonic F-test on the general path: the hn spectrum split into the mu plane, each
+//                         taper's split adding its power to the row and its residual to the den plane, the quotient.
 #include <cuda_runtime.h>
 #include <atomic>
 #include <cstdio>
 #include <cstring>
 #include "../../include/glb_shim.h"
+#include "iq_core.cuh"
 
 extern std::atomic<unsigned long long> g_launches;   // gram_kernels.cu
 
@@ -182,6 +185,57 @@ __global__ void iq_mtm_split_kernel(const float2 *__restrict__ spec, int nz, lon
   }
 }
 
+// The harmonic F-test on the general path (glb_launch_iq_gram_general with ftest).  Z[k] of a frame as the splits above
+// form it; the kernels below are the complex-output split of the hn spectrum (the mu plane), the split of one taper's
+// spectrum that adds its power to the rows as iq_mtm_split_kernel does and its residual to the den plane, and the
+// quotient.  The residual and F are the fused kernel's (iq_core.cuh).
+static __device__ __forceinline__ float2 iq_split_z(const float2 *X, int nz, int k) {
+  const float2 a = X[k], c = X[nz - k];
+  const float er = 0.5f * (a.x + c.x), ei = 0.5f * (a.y - c.y);
+  const float dr = 0.5f * (a.x - c.x), di = 0.5f * (a.y + c.y);
+  float sn, cs;
+  sincospif((float) k / (float) nz, &sn, &cs);
+  const float orr = dr * cs - di * sn, oi = dr * sn + di * cs;
+  return make_float2(er - oi, ei + orr);
+}
+
+__global__ void iq_ftest_mu_kernel(const float2 *__restrict__ spec, int nz, long long nframes, float2 *__restrict__ mu) {
+  const long long total = nframes * nz;
+  const long long stride = (long long) gridDim.x * blockDim.x;
+  for (long long idx = (long long) blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += stride) {
+    const long long f = idx / nz;
+    const int j = (int) (idx - f * nz);
+    mu[idx] = iq_split_z(spec + f * (nz + 1), nz, (j + nz / 2) & (nz - 1));
+  }
+}
+
+// taper k: u0k = (U0_k, sqrt(lambda_k)); add = 0 stores (taper 0), 1 adds; rows may be nullptr
+__global__ void iq_ftest_split_kernel(const float2 *__restrict__ spec, int nz, long long nframes, float inv_nz, int add,
+                                      const float2 *__restrict__ u0, int k, const float2 *__restrict__ mu,
+                                      float *__restrict__ rows, float *__restrict__ den) {
+  const long long total = nframes * nz;
+  const long long stride = (long long) gridDim.x * blockDim.x;
+  const float2 w = u0[k];
+  for (long long idx = (long long) blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += stride) {
+    const long long f = idx / nz;
+    const int j = (int) (idx - f * nz);
+    const float2 z = iq_split_z(spec + f * (nz + 1), nz, (j + nz / 2) & (nz - 1));
+    if (rows) {
+      const float pw = (z.x * z.x + z.y * z.y) * inv_nz;
+      rows[idx] = add ? rows[idx] + pw : pw;
+    }
+    const float r = glb::iq_ftest_resid(z, mu[idx], w.x, w.y);
+    den[idx] = add ? den[idx] + r : r;
+  }
+}
+
+__global__ void iq_ftest_f_kernel(const float2 *__restrict__ mu, const float *__restrict__ den, long long total, float fnum,
+                                  float *__restrict__ ftest) {
+  const long long stride = (long long) gridDim.x * blockDim.x;
+  for (long long idx = (long long) blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += stride)
+    ftest[idx] = glb::iq_ftest_value(mu[idx], den[idx], fnum);
+}
+
 static int sm_count() {
   int dev = 0, sms = 148;
   if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
@@ -250,7 +304,8 @@ extern "C" int glb_launch_zoom_split(const void *spec, int nz, long long nframes
 // stage (host/zoom.c) and the I/Q spectrogram's non-fused launches (iq.cu).  Multitaper (ntapers > 1): one spectrum
 // per taper into the same scratch plane, each followed by iq_mtm_split_kernel, which sums the tapers into the rows.
 extern "C" int glb_launch_iq_gram_general(const glb_iq_gram_args *a, void *stream) {
-  if (!a || !a->rows || a->nframes < 0 || a->ntapers < 0 || a->ntapers > 32) {
+  if (!a || (!a->rows && !a->ftest) || a->nframes < 0 || a->ntapers < 0 || a->ntapers > 32 ||
+      (a->ftest && (a->ntapers < 2 || !a->ftest_taper || !a->ftest_u0))) {
     glb_set_error("glb_launch_iq_gram_general: invalid arguments");
     return GLB_EINVAL;
   }
@@ -285,6 +340,33 @@ extern "C" int glb_launch_iq_gram_general(const glb_iq_gram_args *a, void *strea
   long long ctas = (total + 255) / 256;
   const long long cap = (long long) sm_count() * 16;
   if (ctas > cap) ctas = cap;
+  if (a->ftest) {
+    float2 *mu = reinterpret_cast<float2 *>((float *) a->scratch + a->nframes * (long long) (nz + 1) * 2);
+    float *den = reinterpret_cast<float *>(mu + total);
+    g.tapers = a->ftest_taper;
+    g.taper_symmetric = 0;
+    int rc = glb_launch_gram(&g, stream);
+    if (rc != GLB_OK) return rc;
+    iq_ftest_mu_kernel<<<(int) ctas, 256, 0, (cudaStream_t) stream>>>((const float2 *) a->scratch, nz, a->nframes, mu);
+    ZCU(cudaGetLastError());
+    g_launches++;
+    for (int k = 0; k < a->ntapers; k++) {
+      g.tapers = a->taper + (size_t) k * 2 * nz;
+      g.taper_symmetric = (int) (((unsigned) a->taper_symmetric >> k) & 1u);
+      rc = glb_launch_gram(&g, stream);
+      if (rc != GLB_OK) return rc;
+      iq_ftest_split_kernel<<<(int) ctas, 256, 0, (cudaStream_t) stream>>>(
+          (const float2 *) a->scratch, nz, a->nframes, (float) (1.0 / nz), k > 0, (const float2 *) a->ftest_u0, k, mu,
+          a->rows, den);
+      ZCU(cudaGetLastError());
+      g_launches++;
+    }
+    const float fnum = (float) ((double) (a->ntapers - 1) * (double) a->ftest_s);
+    iq_ftest_f_kernel<<<(int) ctas, 256, 0, (cudaStream_t) stream>>>(mu, den, total, fnum, a->ftest);
+    ZCU(cudaGetLastError());
+    g_launches++;
+    return GLB_OK;
+  }
   for (int k = 0; k < a->ntapers; k++) {
     g.tapers = a->taper + (size_t) k * 2 * nz;
     g.taper_symmetric = (int) (((unsigned) a->taper_symmetric >> k) & 1u);

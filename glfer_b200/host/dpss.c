@@ -158,3 +158,23 @@ int gl_dpss(int nmax, int kmax, int n, double w, double **v, double *sig, int *t
   free(lam);
   return rc;
 }
+
+/* The harmonic F-test's weights of K unit-energy tapers [K][n] (mtm_init, mtm.c:78-84,123-136): u0[k] = sum_i v_k[i] in
+ * double, s = sum_k u0[k]^2 and hn[i] = sum_k u0[k] v_k[i] / s through float accumulators, as the reference rounds them.
+ * Shared by the real multitaper plan (host/gram.c) and the complex ones (host/iq.c, host/zoom.c). */
+void glb_mtm_ftest_weights(int n, int K, const double *tapers, double *u0, float *hn, float *s)
+{
+  float s2 = 0.0f;
+  for (int k = 0; k < K; k++) {
+    double acc = 0.0;
+    for (int i = 0; i < n; i++) acc += tapers[(size_t) k * n + i];
+    u0[k] = acc;
+    s2 += u0[k] * u0[k];
+  }
+  for (int i = 0; i < n; i++) {
+    float h = 0.0f;
+    for (int k = 0; k < K; k++) h += u0[k] * tapers[(size_t) k * n + i];
+    hn[i] = h / s2;
+  }
+  *s = s2;
+}

@@ -12,9 +12,14 @@
 double glb_bessel_i0(double x);
 void glb_window_table(int n, int window_type, float *w);
 int glb_dpss(int n, double nw, int kmax, double *tapers, double *lambda);
+/* host/dpss.c: U0 (double), S and hn (float) of the harmonic F-test from K unit-energy tapers [K][n] */
+void glb_mtm_ftest_weights(int n, int K, const double *tapers, double *u0, float *hn, float *s);
 /* host/iq.c: DPSS and [K'][2n] taper table of a complex multitaper plan (I/Q or zoom); sym: bit k = taper k mirror-symmetric */
 int glb_iq_mtm_tapers(int n, float mtm_w, int mtm_kmax, float taper_scale, double **h_tapers, double **h_lambda,
                       float **table, int *sym);
+/* host/iq.c: the F-test's device table of a complex multitaper plan, hn [2n] then (U0_k, sqrt(lambda_k)) [K'], and S */
+int glb_iq_ftest_table(int n, int K, const double *h_tapers, const double *h_lambda, float taper_scale, float **d_ftab,
+                       float *s);
 int glb_hop(int n, float overlap);
 /* the message slot of glfer_b200_last_error() (gram.c), for the other host units */
 int glb_host_fail(int code, const char *msg);

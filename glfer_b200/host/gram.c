@@ -289,17 +289,9 @@ int glfer_gram_plan_create(const glfer_gram_config *cfg, glfer_gram_plan **out)
       double *u0 = malloc(sizeof(double) * K);
       float *ft = malloc(sizeof(float) * (size_t) (K + 1) * n);
       float s2 = 0.0f;
-      for (int k = 0; k < K; k++) {
-        double s = 0.0;
-        for (int i = 0; i < n; i++) s += p->h_tapers[(size_t) k * n + i];
-        u0[k] = s;
-        s2 += u0[k] * u0[k];
-      }
+      glb_mtm_ftest_weights(n, K, p->h_tapers, u0, ft, &s2);
       for (int i = 0; i < n; i++) {
-        float h = 0.0f;
-        for (int k = 0; k < K; k++) h += u0[k] * p->h_tapers[(size_t) k * n + i];
-        h /= s2;
-        ft[i] = (float) ((double) h * (double) p->taper_scale);
+        ft[i] = (float) ((double) ft[i] * (double) p->taper_scale);
         for (int k = 0; k < K; k++) ft[(size_t) (k + 1) * n + i] = (float) (p->h_tapers[(size_t) k * n + i] * (double) p->taper_scale);
       }
       p->sum_u0_sqr = (double) s2;

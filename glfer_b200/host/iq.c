@@ -13,7 +13,9 @@
  *
  * Multitaper plans (glfer_iq_plan_create_mtm, and the zoom's) upload K' DPSS tapers, [K'][2n] floats, each scaled as
  * the real multitaper plan scales its own (host/gram.c); the row sums the K' eigen-spectra.  They always bring float
- * rows to the device: their waterfall goes through the display chain, for a fixed range too.
+ * rows to the device: their waterfall goes through the display chain, for a fixed range too.  They also upload the
+ * harmonic F-test's hn taper and U0 values (glb_iq_ftest_table), n + K' values: every multitaper plan serves
+ * glfer_iq_run_mtm_ftest, whose chunks bring back F rows beside or instead of the rows.
  */
 #include <math.h>
 #include <stdlib.h>
@@ -32,6 +34,8 @@ typedef struct {
   size_t in_cap;              /* floats */
   float *d_rows;
   size_t rows_cap;            /* floats */
+  float *d_ftest;             /* F rows (glfer_iq_run_mtm_ftest) */
+  size_t ftest_cap;           /* floats */
   void *d_scratch;
   size_t scratch_cap;         /* bytes */
   glb_display_slot disp;      /* display mapping */
@@ -46,6 +50,8 @@ struct glfer_iq_plan {
   float taper_scale;
   int ntapers;                /* 1: periodogram, K' = mtm_kmax + 1: multitaper */
   double *h_tapers, *h_lambda;  /* multitaper: the unscaled DPSS [K'][n] and eigenvalues (glfer_iq_tapers) */
+  float *d_ftab;              /* multitaper: the F-test's table (glb_iq_ftest_table): hn [2n], then (U0_k, sqrt(lambda_k)) */
+  float ftest_s;              /* S = sum_k U0_k^2 */
   void *tables;               /* FFT tables of the 2n-float frames */
   islot slot[ISLOT];
   glb_display disp;
@@ -82,12 +88,13 @@ void glfer_iq_plan_destroy(glfer_iq_plan *p)
   for (int i = 0; i < ISLOT; i++) {
     islot *s = &p->slot[i];
     if (s->stream) glb_stream_sync(s->stream);
-    glb_free(s->d_pcm); glb_free(s->d_in); glb_free(s->d_rows); glb_free(s->d_scratch);
+    glb_free(s->d_pcm); glb_free(s->d_in); glb_free(s->d_rows); glb_free(s->d_ftest); glb_free(s->d_scratch);
     glb_display_slot_free(&s->disp);
     glb_stream_destroy(s->stream);
   }
   glb_display_free(&p->disp);
   glb_free(p->d_taper);
+  glb_free(p->d_ftab);
   glb_tables_destroy(p->tables);
   free(p->h_tapers); free(p->h_lambda);
   free(p);
@@ -128,6 +135,32 @@ int glb_iq_mtm_tapers(int n, float mtm_w, int mtm_kmax, float taper_scale, doubl
   }
   *h_tapers = tap; *h_lambda = lam; *table = tab;
   return 0;
+}
+
+/* The harmonic F-test's table of a complex multitaper plan, uploaded to *d_ftab: hn (glb_mtm_ftest_weights, as the real
+ * plan builds it) times taper_scale on both floats of complex sample i, [2n] floats, then the K' pairs
+ * (U0_k, sqrt(lambda_k)) that undo the per-taper weight of the taper table in the residual (glb_iq_gram_args). */
+int glb_iq_ftest_table(int n, int K, const double *h_tapers, const double *h_lambda, float taper_scale, float **d_ftab,
+                       float *s)
+{
+  double *u0 = malloc(sizeof(double) * K);
+  float *hn = malloc(sizeof(float) * n);
+  float *tab = malloc(sizeof(float) * (2 * (size_t) n + 2 * (size_t) K));
+  int rc = 0;
+  if (!u0 || !hn || !tab) rc = glb_host_fail(GLFER_ENOMEM, "out of memory");
+  if (rc == 0) {
+    glb_mtm_ftest_weights(n, K, h_tapers, u0, hn, s);
+    for (int i = 0; i < n; i++) tab[2 * i] = tab[2 * i + 1] = (float) ((double) hn[i] * (double) taper_scale);
+    for (int k = 0; k < K; k++) {
+      tab[2 * n + 2 * k] = (float) u0[k];
+      tab[2 * n + 2 * k + 1] = (float) sqrt(h_lambda[k]);
+    }
+    const size_t bytes = sizeof(float) * (2 * (size_t) n + 2 * (size_t) K);
+    rc = glb_host_shim(glb_malloc((void **) d_ftab, bytes));
+    if (rc == 0) rc = glb_host_shim(glb_memcpy_h2d(*d_ftab, tab, bytes, NULL));
+  }
+  free(u0); free(hn); free(tab);
+  return rc;
 }
 
 /* tab: NULL (periodogram: the window), or the multitaper table of glb_iq_mtm_tapers */
@@ -199,6 +232,8 @@ static int iq_plan_create(const glfer_iq_config *cfg, int mtm, float mtm_w, int 
   p->taper_sym = sym;
   rc = build_taper(p, tab);
   free(tab);
+  if (rc == 0 && mtm)
+    rc = glb_iq_ftest_table(cfg->n, p->ntapers, h_tapers, h_lambda, taper_scale, &p->d_ftab, &p->ftest_s);
   for (int i = 0; i < ISLOT && rc == 0; i++) {
     rc = glb_host_shim(glb_stream_create(&p->slot[i].stream));
     if (rc == 0) rc = glb_host_shim(glb_event_create(&p->slot[i].disp.ev_agc));
@@ -253,9 +288,10 @@ static long long iq_chunk_frames(const glfer_iq_plan *p)
   return f < 1 ? 1 : f;
 }
 
-/* frames [c0, c0 + cn) on slot s: rows into s->d_rows, or with fl the fixed-range levels into s->disp.d_levels */
+/* frames [c0, c0 + cn) on slot s: with fl the fixed-range levels into s->disp.d_levels, otherwise rows into s->d_rows
+ * (rows_on) and F rows into s->d_ftest (ftest_on) */
 static int iq_chunk(glfer_iq_plan *p, islot *s, const void *src, int pcm16, long long origin, long long c0,
-                    long long cn, const glb_display_run *fl)
+                    long long cn, const glb_display_run *fl, int rows_on, int ftest_on)
 {
   const long long n = p->cfg.n, hop = p->hop;
   long long lo = c0 * hop - (n - hop);
@@ -273,8 +309,9 @@ static int iq_chunk(glfer_iq_plan *p, islot *s, const void *src, int pcm16, long
   } else {
     ITRY(glb_memcpy_h2d(s->d_in, (const float *) src + 2 * (lo - origin), sizeof(float) * 2 * (size_t) cnt, s->stream));
   }
-  if (!fl) ITRY(iensure((void **) &s->d_rows, &s->rows_cap, (size_t) (cn * n), sizeof(float)));
-  const long long sb = glb_iq_gram_scratch_bytes((int) n, (int) hop, cn, fl != NULL, p->ntapers);
+  if (!fl && rows_on) ITRY(iensure((void **) &s->d_rows, &s->rows_cap, (size_t) (cn * n), sizeof(float)));
+  if (ftest_on) ITRY(iensure((void **) &s->d_ftest, &s->ftest_cap, (size_t) (cn * n), sizeof(float)));
+  const long long sb = glb_iq_gram_scratch_bytes((int) n, (int) hop, cn, fl != NULL, p->ntapers, ftest_on);
   if (sb > 0) ITRY(iensure(&s->d_scratch, &s->scratch_cap, (size_t) sb, 1));
   glb_iq_gram_args g;
   memset(&g, 0, sizeof g);
@@ -289,7 +326,7 @@ static int iq_chunk(glfer_iq_plan *p, islot *s, const void *src, int pcm16, long
   g.ntapers = p->ntapers;
   g.first_frame = c0;
   g.nframes = cn;
-  g.rows = fl ? NULL : s->d_rows;
+  g.rows = (fl || !rows_on) ? NULL : s->d_rows;
   g.tables = p->tables;
   g.scratch = sb > 0 ? s->d_scratch : NULL;
   if (fl) {
@@ -302,15 +339,27 @@ static int iq_chunk(glfer_iq_plan *p, islot *s, const void *src, int pcm16, long
     g.level_max = fl->fixed[0];
     g.level_thr = fl->thr;
   }
+  if (ftest_on) {
+    g.ftest = s->d_ftest;
+    g.ftest_taper = p->d_ftab;
+    g.ftest_u0 = p->d_ftab + 2 * n;
+    g.ftest_s = p->ftest_s;
+  }
   ITRY(glb_launch_iq_gram(&g, s->stream));
   return 0;
 }
 
+/* rows and/or F rows (ftest_on: glfer_iq_run_mtm_ftest; rows or ftest may then be NULL) */
 static int iq_run_impl(glfer_iq_plan *p, const void *src, int pcm16, long long origin, long long count,
-                       long long first_frame, long long nframes, float *rows)
+                       long long first_frame, long long nframes, float *rows, int ftest_on, float *ftest)
 {
   glb_host_clear_error();
-  if (!p || !src || !rows) return glb_host_fail(GLFER_EINVAL, "null argument");
+  if (!p || !src || (!ftest_on && !rows)) return glb_host_fail(GLFER_EINVAL, "null argument");
+  if (ftest_on) {
+    if (!p->h_tapers) return glb_host_fail(GLFER_EINVAL, "the F-test needs a multitaper plan (glfer_iq_plan_create_mtm)");
+    if (p->ntapers < 2) return glb_host_fail(GLFER_EINVAL, "the F-test needs mtm_kmax >= 1 (K' - 1 degrees of freedom)");
+    if (!rows && !ftest) return glb_host_fail(GLFER_EINVAL, "null argument: rows and ftest are both NULL");
+  }
   if (nframes < 0 || first_frame < 0) return glb_host_fail(GLFER_EINVAL, "negative frame range");
   if (origin < 0 || count < 0) return glb_host_fail(GLFER_EINVAL, "negative origin or sample count");
   if (nframes == 0) return 0;
@@ -328,10 +377,13 @@ static int iq_run_impl(glfer_iq_plan *p, const void *src, int pcm16, long long o
     const long long cn = (nframes - done < cf) ? nframes - done : cf;
     rc = glb_host_shim(glb_stream_sync(s->stream));
     if (rc) break;
-    rc = iq_chunk(p, s, src, pcm16, origin, first_frame + done, cn, NULL);
-    if (rc == 0)
+    rc = iq_chunk(p, s, src, pcm16, origin, first_frame + done, cn, NULL, rows != NULL, ftest != NULL);
+    if (rc == 0 && rows)
       rc = glb_host_shim(glb_memcpy_d2h(rows + (size_t) done * p->cfg.n, s->d_rows, sizeof(float) * (size_t) (cn * p->cfg.n),
                                         s->stream));
+    if (rc == 0 && ftest)
+      rc = glb_host_shim(glb_memcpy_d2h(ftest + (size_t) done * p->cfg.n, s->d_ftest,
+                                        sizeof(float) * (size_t) (cn * p->cfg.n), s->stream));
     done += cn;
     ci++;
   }
@@ -345,13 +397,25 @@ static int iq_run_impl(glfer_iq_plan *p, const void *src, int pcm16, long long o
 int glfer_iq_run(glfer_iq_plan *p, const float *iq, long long origin, long long count, long long first_frame,
                  long long nframes, float *rows)
 {
-  return iq_run_impl(p, iq, 0, origin, count, first_frame, nframes, rows);
+  return iq_run_impl(p, iq, 0, origin, count, first_frame, nframes, rows, 0, NULL);
 }
 
 int glfer_iq_run_pcm16(glfer_iq_plan *p, const short *iq, long long origin, long long count, long long first_frame,
                        long long nframes, float *rows)
 {
-  return iq_run_impl(p, iq, 1, origin, count, first_frame, nframes, rows);
+  return iq_run_impl(p, iq, 1, origin, count, first_frame, nframes, rows, 0, NULL);
+}
+
+int glfer_iq_run_mtm_ftest(glfer_iq_plan *p, const float *iq, long long origin, long long count, long long first_frame,
+                           long long nframes, float *rows, float *ftest)
+{
+  return iq_run_impl(p, iq, 0, origin, count, first_frame, nframes, rows, 1, ftest);
+}
+
+int glfer_iq_run_mtm_ftest_pcm16(glfer_iq_plan *p, const short *iq, long long origin, long long count,
+                                 long long first_frame, long long nframes, float *rows, float *ftest)
+{
+  return iq_run_impl(p, iq, 1, origin, count, first_frame, nframes, rows, 1, ftest);
 }
 
 /* main_window_draw's mapping of the plan's own rows (include/glfer_b200.h, glfer_iq_run_display) */
@@ -387,7 +451,7 @@ static int iq_run_display_impl(glfer_iq_plan *p, const void *src, int pcm16, lon
     const long long cn = (nframes - done < cf) ? nframes - done : cf;
     rc = glb_host_shim(glb_stream_sync(s->stream));
     if (rc == 0) rc = glb_display_reserve(&s->disp, cn, n, rgb != NULL);
-    if (rc == 0) rc = iq_chunk(p, s, src, pcm16, origin, c0, cn, fuse ? &dr : NULL);
+    if (rc == 0) rc = iq_chunk(p, s, src, pcm16, origin, c0, cn, fuse ? &dr : NULL, !fuse, 0);
     if (rc == 0 && !fuse)
       rc = glb_display_map(&p->disp, &dr, &s->disp, ci > 0 ? &p->slot[(ci - 1) % ISLOT].disp : NULL, s->d_rows, s->d_rows,
                            n, c0, cn, done, p->cfg.overlap, rgb != NULL, s->stream);

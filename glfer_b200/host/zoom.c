@@ -19,6 +19,8 @@
  *
  * Multitaper plans (glfer_zoom_plan_create_mtm / _create_iq_mtm) replace the window by K' DPSS tapers
  * (glb_iq_mtm_tapers, host/iq.c); the frame stage then runs one spectrum per taper into the same scratch plane.
+ * They also hold the harmonic F-test's table (glb_iq_ftest_table): glfer_zoom_run[_iq]_mtm_ftest add the hn spectrum
+ * and the mu and den planes to that scratch and bring back F rows beside or instead of the rows.
  */
 #include <math.h>
 #include <stdlib.h>
@@ -40,6 +42,8 @@ typedef struct {
   size_t spec_cap;            /* floats */
   float *d_rows;
   size_t rows_cap;            /* floats */
+  float *d_ftest;             /* F rows (glfer_zoom_run[_iq]_mtm_ftest) */
+  size_t ftest_cap;           /* floats */
   glb_display_slot disp;      /* display mapping */
 } zslot;
 
@@ -54,6 +58,8 @@ struct glfer_zoom_plan {
   float taper_scale;
   int ntapers;                /* 1: periodogram, K' = mtm_kmax + 1: multitaper */
   double *h_tapers, *h_lambda;  /* multitaper: the unscaled DPSS [K'][n] and eigenvalues (glfer_zoom_tapers) */
+  float *d_ftab;              /* multitaper: the F-test's table (glb_iq_ftest_table): hn [2n], then (U0_k, sqrt(lambda_k)) */
+  float ftest_s;              /* S = sum_k U0_k^2 */
   int iq;                     /* 1: complex (I, Q) input (glfer_zoom_plan_create_iq), signed centre */
   void *tables;               /* FFT tables of the 2n-point real transform */
   zslot slot[ZSLOT];
@@ -142,7 +148,7 @@ void glfer_zoom_plan_destroy(glfer_zoom_plan *p)
   for (int i = 0; i < ZSLOT; i++) {
     zslot *s = &p->slot[i];
     if (s->stream) glb_stream_sync(s->stream);
-    glb_free(s->d_in); glb_free(s->d_y); glb_free(s->d_spec); glb_free(s->d_rows);
+    glb_free(s->d_in); glb_free(s->d_y); glb_free(s->d_spec); glb_free(s->d_rows); glb_free(s->d_ftest);
     glb_event_destroy(s->ev_dec);
     glb_display_slot_free(&s->disp);
     glb_stream_destroy(s->stream);
@@ -150,6 +156,7 @@ void glfer_zoom_plan_destroy(glfer_zoom_plan *p)
   glb_display_free(&p->disp);
   glb_free(p->d_taps);
   glb_free(p->d_taper);
+  glb_free(p->d_ftab);
   glb_tables_destroy(p->tables);
   free(p->h_tapers); free(p->h_lambda);
   free(p);
@@ -250,6 +257,8 @@ static int zoom_plan_create(const glfer_zoom_config *cfg, int iq, int mtm, float
   p->taper_sym = sym;
   rc = build_tables(p, mtab);
   free(mtab);
+  if (rc == 0 && mtm)
+    rc = glb_iq_ftest_table(cfg->n, p->ntapers, h_tapers, h_lambda, taper_scale, &p->d_ftab, &p->ftest_s);
   for (int i = 0; i < ZSLOT && rc == 0; i++) {
     rc = glb_host_shim(glb_stream_create(&p->slot[i].stream));
     if (rc == 0) rc = glb_host_shim(glb_event_create(&p->slot[i].ev_dec));
@@ -316,9 +325,10 @@ static long long zoom_chunk_frames(const glfer_zoom_plan *p)
   return f < 1 ? 1 : f;
 }
 
-/* rows of frames [c0, c0 + cn) into s->d_rows; prev: the slot of the previous chunk of this run, or NULL */
+/* rows of frames [c0, c0 + cn) into s->d_rows (rows_on) and F rows into s->d_ftest (ftest_on); prev: the slot of the
+ * previous chunk of this run, or NULL */
 static int zoom_chunk(glfer_zoom_plan *p, zslot *s, const zslot *prev, const void *src, int pcm16,
-                      long long origin, long long c0, long long cn)
+                      long long origin, long long c0, long long cn, int rows_on, int ftest_on)
 {
   const glfer_zoom_config *c = &p->cfg;
   const long long D = c->decim, n = c->n, hop = p->hop;
@@ -357,8 +367,10 @@ static int zoom_chunk(glfer_zoom_plan *p, zslot *s, const zslot *prev, const voi
   s->y_base = base;
   s->y_end = m_hi;
 
-  ZTRY(zensure((void **) &s->d_spec, &s->spec_cap, (size_t) cn * (n + 1) * 2, sizeof(float)));
-  ZTRY(zensure((void **) &s->d_rows, &s->rows_cap, (size_t) cn * n, sizeof(float)));
+  /* the general path's scratch (glb_launch_iq_gram_general): the spectrum, and for the F-test the mu and den planes */
+  ZTRY(zensure((void **) &s->d_spec, &s->spec_cap, (size_t) cn * ((n + 1) * 2 + (ftest_on ? 3 * n : 0)), sizeof(float)));
+  if (rows_on) ZTRY(zensure((void **) &s->d_rows, &s->rows_cap, (size_t) cn * n, sizeof(float)));
+  if (ftest_on) ZTRY(zensure((void **) &s->d_ftest, &s->ftest_cap, (size_t) cn * n, sizeof(float)));
   glb_iq_gram_args g;
   memset(&g, 0, sizeof g);
   g.n = (int) n;
@@ -372,21 +384,33 @@ static int zoom_chunk(glfer_zoom_plan *p, zslot *s, const zslot *prev, const voi
   g.ntapers = p->ntapers;
   g.first_frame = c0;
   g.nframes = cn;
-  g.rows = s->d_rows;
+  g.rows = rows_on ? s->d_rows : NULL;
   g.tables = p->tables;
   g.scratch = s->d_spec;
+  if (ftest_on) {
+    g.ftest = s->d_ftest;
+    g.ftest_taper = p->d_ftab;
+    g.ftest_u0 = p->d_ftab + 2 * n;
+    g.ftest_s = p->ftest_s;
+  }
   ZTRY(glb_launch_iq_gram_general(&g, s->stream));
   return 0;
 }
 
+/* rows and/or F rows (ftest_on: glfer_zoom_run[_iq]_mtm_ftest; rows or ftest may then be NULL) */
 static int zoom_run_impl(glfer_zoom_plan *p, int iq, const void *src, int pcm16, long long origin, long long count,
-                         long long first_frame, long long nframes, float *rows)
+                         long long first_frame, long long nframes, float *rows, int ftest_on, float *ftest)
 {
   glb_host_clear_error();
-  if (!p || !src || !rows) return glb_host_fail(GLFER_EINVAL, "null argument");
+  if (!p || !src || (!ftest_on && !rows)) return glb_host_fail(GLFER_EINVAL, "null argument");
   if (iq != p->iq)
     return glb_host_fail(GLFER_EINVAL, iq ? "glfer_zoom_run_iq needs a plan from glfer_zoom_plan_create_iq"
                                           : "an I/Q zoom plan runs through glfer_zoom_run_iq / glfer_zoom_run_iq_pcm16");
+  if (ftest_on) {
+    if (!p->h_tapers) return glb_host_fail(GLFER_EINVAL, "the F-test needs a multitaper zoom plan");
+    if (p->ntapers < 2) return glb_host_fail(GLFER_EINVAL, "the F-test needs mtm_kmax >= 1 (K' - 1 degrees of freedom)");
+    if (!rows && !ftest) return glb_host_fail(GLFER_EINVAL, "null argument: rows and ftest are both NULL");
+  }
   if (nframes < 0 || first_frame < 0) return glb_host_fail(GLFER_EINVAL, "negative frame range");
   if (origin < 0 || count < 0) return glb_host_fail(GLFER_EINVAL, "negative origin or sample count");
   if (nframes == 0) return 0;
@@ -405,10 +429,13 @@ static int zoom_run_impl(glfer_zoom_plan *p, int iq, const void *src, int pcm16,
     const long long cn = (nframes - done < cf) ? nframes - done : cf;
     rc = glb_host_shim(glb_stream_sync(s->stream));
     if (rc) break;
-    rc = zoom_chunk(p, s, prev, src, pcm16, origin, first_frame + done, cn);
-    if (rc == 0)
+    rc = zoom_chunk(p, s, prev, src, pcm16, origin, first_frame + done, cn, rows != NULL, ftest != NULL);
+    if (rc == 0 && rows)
       rc = glb_host_shim(glb_memcpy_d2h(rows + (size_t) done * p->cfg.n, s->d_rows, sizeof(float) * (size_t) cn * p->cfg.n,
                                         s->stream));
+    if (rc == 0 && ftest)
+      rc = glb_host_shim(glb_memcpy_d2h(ftest + (size_t) done * p->cfg.n, s->d_ftest,
+                                        sizeof(float) * (size_t) cn * p->cfg.n, s->stream));
     prev = s;
     done += cn;
     ci++;
@@ -423,25 +450,49 @@ static int zoom_run_impl(glfer_zoom_plan *p, int iq, const void *src, int pcm16,
 int glfer_zoom_run(glfer_zoom_plan *p, const float *samples, long long origin, long long count,
                    long long first_frame, long long nframes, float *rows)
 {
-  return zoom_run_impl(p, 0, samples, 0, origin, count, first_frame, nframes, rows);
+  return zoom_run_impl(p, 0, samples, 0, origin, count, first_frame, nframes, rows, 0, NULL);
 }
 
 int glfer_zoom_run_pcm16(glfer_zoom_plan *p, const short *pcm, long long origin, long long count,
                          long long first_frame, long long nframes, float *rows)
 {
-  return zoom_run_impl(p, 0, pcm, 1, origin, count, first_frame, nframes, rows);
+  return zoom_run_impl(p, 0, pcm, 1, origin, count, first_frame, nframes, rows, 0, NULL);
 }
 
 int glfer_zoom_run_iq(glfer_zoom_plan *p, const float *iq, long long origin, long long count,
                       long long first_frame, long long nframes, float *rows)
 {
-  return zoom_run_impl(p, 1, iq, 0, origin, count, first_frame, nframes, rows);
+  return zoom_run_impl(p, 1, iq, 0, origin, count, first_frame, nframes, rows, 0, NULL);
 }
 
 int glfer_zoom_run_iq_pcm16(glfer_zoom_plan *p, const short *iq, long long origin, long long count,
                             long long first_frame, long long nframes, float *rows)
 {
-  return zoom_run_impl(p, 1, iq, 1, origin, count, first_frame, nframes, rows);
+  return zoom_run_impl(p, 1, iq, 1, origin, count, first_frame, nframes, rows, 0, NULL);
+}
+
+int glfer_zoom_run_mtm_ftest(glfer_zoom_plan *p, const float *samples, long long origin, long long count,
+                             long long first_frame, long long nframes, float *rows, float *ftest)
+{
+  return zoom_run_impl(p, 0, samples, 0, origin, count, first_frame, nframes, rows, 1, ftest);
+}
+
+int glfer_zoom_run_mtm_ftest_pcm16(glfer_zoom_plan *p, const short *pcm, long long origin, long long count,
+                                   long long first_frame, long long nframes, float *rows, float *ftest)
+{
+  return zoom_run_impl(p, 0, pcm, 1, origin, count, first_frame, nframes, rows, 1, ftest);
+}
+
+int glfer_zoom_run_iq_mtm_ftest(glfer_zoom_plan *p, const float *iq, long long origin, long long count,
+                                long long first_frame, long long nframes, float *rows, float *ftest)
+{
+  return zoom_run_impl(p, 1, iq, 0, origin, count, first_frame, nframes, rows, 1, ftest);
+}
+
+int glfer_zoom_run_iq_mtm_ftest_pcm16(glfer_zoom_plan *p, const short *iq, long long origin, long long count,
+                                      long long first_frame, long long nframes, float *rows, float *ftest)
+{
+  return zoom_run_impl(p, 1, iq, 1, origin, count, first_frame, nframes, rows, 1, ftest);
 }
 
 /* main_window_draw's mapping of the plan's own rows (include/glfer_b200.h, glfer_zoom_run_display) */
@@ -480,7 +531,7 @@ static int zoom_run_display_impl(glfer_zoom_plan *p, int iq, const void *src, in
     const long long cn = (nframes - done < cf) ? nframes - done : cf;
     rc = glb_host_shim(glb_stream_sync(s->stream));
     if (rc == 0) rc = glb_display_reserve(&s->disp, cn, n, rgb != NULL);
-    if (rc == 0) rc = zoom_chunk(p, s, prev, src, pcm16, origin, c0, cn);
+    if (rc == 0) rc = zoom_chunk(p, s, prev, src, pcm16, origin, c0, cn, 1, 0);
     if (rc == 0)
       rc = glb_display_map(&p->disp, &dr, &s->disp, prev ? &prev->disp : NULL, s->d_rows, s->d_rows, n, c0, cn, done,
                            p->cfg.overlap, rgb != NULL, s->stream);

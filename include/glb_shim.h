@@ -240,6 +240,13 @@ typedef struct {
   float level_min, level_max;  /* display_min / display_max (dB in the log scales) */
   float level_thr;             /* opt.thr_level / 100 */
   int ntapers;                 /* 0 or 1: periodogram; K' = 2..32: multitaper (no levels: GLB_EINVAL) */
+  /* Thomson's harmonic F-test of a multitaper launch (include/glfer_b200.h, glfer_iq_run_mtm_ftest):
+       F[f][j] = (K' - 1) |mu(j)|^2 S / sum_k |y_k(j) - mu(j) U0_k|^2
+     with mu the transform of the frame under hn and y_k under the unit-energy taper v_k.  Rows may then be NULL. */
+  float *ftest;                /* device out: [nframes][n] F rows, or NULL */
+  const float *ftest_taper;    /* device: [2n] floats, hn[i] taper_scale on both floats of complex sample i */
+  const float *ftest_u0;       /* device: [ntapers] float pairs (U0_k, sqrt(lambda_k)) */
+  float ftest_s;               /* S = sum_k U0_k^2 */
 } glb_iq_gram_args;
 /* The one entry of the I/Q spectrogram: the fused kernel (iq.cu, regular geometry n = 32..8192, hop = (n/16) << s
  * with n - hop a multiple of hop; needs an even origin, a 16-byte aligned samples pointer and samples that cover
@@ -249,11 +256,15 @@ typedef struct {
 int glb_launch_iq_gram(const glb_iq_gram_args *a, void *stream);
 /* device scratch glb_launch_iq_gram needs for nframes frames (0 when the fused kernel serves the geometry);
  * levels: 1 when the launch writes levels (the general path then also holds the float rows); ntapers as in the
- * arguments (the general path reuses one spectrum plane for all tapers, so the size does not grow with it) */
-long long glb_iq_gram_scratch_bytes(int n, int hop, long long nframes, int levels, int ntapers);
+ * arguments (the general path reuses one spectrum plane for all tapers, so the size does not grow with it);
+ * ftest: 1 when the launch writes F rows (the general path then also holds the mu and den planes) */
+long long glb_iq_gram_scratch_bytes(int n, int hop, long long nframes, int levels, int ntapers, int ftest);
 /* the general path: the general spectrogram kernel's spectrum output on the 2n-float frames (into scratch, at
  * least nframes (n + 1) (re, im) pairs), then glb_launch_zoom_split; multitaper: that spectrum once per taper, each
- * followed by a split that stores (taper 0) or adds (the others) its powers into the rows */
+ * followed by a split that stores (taper 0) or adds (the others) its powers into the rows.  F-test: scratch holds
+ * nframes 3 n more floats; the hn spectrum is split first into the mu plane ([nframes][n] (re, im) pairs behind
+ * the spectrum), each taper's split also adds its residual to the den plane ([nframes][n] floats behind mu), and a
+ * last kernel forms F */
 int glb_launch_iq_gram_general(const glb_iq_gram_args *a, void *stream);
 
 /* counters */

@@ -323,6 +323,36 @@ int glfer_zoom_plan_create_iq_mtm(const glfer_zoom_config *cfg, float mtm_w, int
 int glfer_iq_tapers(const glfer_iq_plan *plan, double *tapers, double *lambda);
 int glfer_zoom_tapers(const glfer_zoom_plan *plan, double *tapers, double *lambda);
 
+/* Thomson's harmonic F-test of multitaper I/Q and zoom plans (real and I/Q zoom).  Frame f is the plan's complex frame
+ * z_f above (I/Q samples, or the decimated y of a zoom), v_k and lambda_k the plan's tapers (glfer_iq_tapers /
+ * glfer_zoom_tapers), K' = mtm_kmax + 1, and
+ *     U0_k = sum_i v_k[i],   S = sum_k U0_k^2,   hn[i] = sum_k U0_k v_k[i] / S
+ * built exactly as a real GLFER_MODE_MTM plan with mtm_ftest = 1 builds them (U0 in double, S and hn through float
+ * accumulators, mtm.c:78-84,123-136).  For every row position j = 0..n-1 (fft-shifted, DC at n/2, as the rows):
+ *     y_k(j) = sum_i v_k[i] z_f[i] e^{-2 pi i (j - n/2) i / n}     (the unit-energy taper, not weighted by 1 / lambda_k)
+ *     mu(j)  = sum_i hn[i] z_f[i] e^{-2 pi i (j - n/2) i / n}
+ *     F[f][j] = (K' - 1) |mu(j)|^2 S / sum_k |y_k(j) - mu(j) U0_k|^2
+ * Every bin of a complex frame is complex: none of the real F-test's DC and Nyquist special cases, the denominator is
+ * accumulated at every position.  For I/Q input (x, 0), F at row position n/2 + j is the real plan's F-test of x at bin
+ * j, 1 <= j < n/2.  On white complex Gaussian noise F follows the F(2, 2K' - 2) distribution, so a threshold has a
+ * stated false-alarm rate.  The division follows IEEE rules: an all-zero frame gives 0 / 0 = NaN.
+ * Each call returns the rows (bit-identical to glfer_iq_run / glfer_zoom_run* of the same frames) and/or the F rows,
+ * [nframes][n] each; either pointer may be NULL, not both.  Every multitaper I/Q or zoom plan serves them.  GLFER_EINVAL
+ * for a periodogram plan, K' < 2 (no degrees of freedom), both outputs NULL, input that does not cover the plan's
+ * required span, and (zoom) a real entry point with an I/Q plan or the reverse. */
+int glfer_iq_run_mtm_ftest(glfer_iq_plan *plan, const float *iq, long long origin, long long count,
+                           long long first_frame, long long nframes, float *rows, float *ftest);
+int glfer_iq_run_mtm_ftest_pcm16(glfer_iq_plan *plan, const short *iq, long long origin, long long count,
+                                 long long first_frame, long long nframes, float *rows, float *ftest);
+int glfer_zoom_run_mtm_ftest(glfer_zoom_plan *plan, const float *samples, long long origin, long long count,
+                             long long first_frame, long long nframes, float *rows, float *ftest);
+int glfer_zoom_run_mtm_ftest_pcm16(glfer_zoom_plan *plan, const short *pcm, long long origin, long long count,
+                                   long long first_frame, long long nframes, float *rows, float *ftest);
+int glfer_zoom_run_iq_mtm_ftest(glfer_zoom_plan *plan, const float *iq, long long origin, long long count,
+                                long long first_frame, long long nframes, float *rows, float *ftest);
+int glfer_zoom_run_iq_mtm_ftest_pcm16(glfer_zoom_plan *plan, const short *iq, long long origin, long long count,
+                                      long long first_frame, long long nframes, float *rows, float *ftest);
+
 /* ---- display output of I/Q and zoom plans ----
  * The waterfall of the plan's own rows, as glfer_gram_run_display gives it for real audio: levels, rgb, agc_state
  * and display_range as there, and exactly main_window_draw's mapping (g_main.c:1109-1229) of the rows that

@@ -35,7 +35,8 @@ class IqGramArgs(C.Structure):         # include/glb_shim.h glb_iq_gram_args
                 ("first_frame", C.c_longlong), ("nframes", C.c_longlong), ("rows", C.c_void_p), ("tables", C.c_void_p),
                 ("scratch", C.c_void_p), ("levels", C.c_void_p), ("levels_stride", C.c_longlong),
                 ("level_tables", C.c_void_p), ("levels_log", C.c_int), ("level_lut", C.c_void_p), ("level_min", C.c_float),
-                ("level_max", C.c_float), ("level_thr", C.c_float), ("ntapers", C.c_int)]
+                ("level_max", C.c_float), ("level_thr", C.c_float), ("ntapers", C.c_int),
+                ("ftest", C.c_void_p), ("ftest_taper", C.c_void_p), ("ftest_u0", C.c_void_p), ("ftest_s", C.c_float)]
 
 
 def gpu_info():
@@ -75,7 +76,7 @@ def main():
         raise SystemExit("iq_bench needs a CUDA device")
     L = api.lib()
     L.glb_launch_iq_gram.argtypes = [C.POINTER(IqGramArgs), C.c_void_p]
-    L.glb_iq_gram_scratch_bytes.argtypes = [C.c_int, C.c_int, C.c_longlong, C.c_int]
+    L.glb_iq_gram_scratch_bytes.argtypes = [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_int]
     L.glb_iq_gram_scratch_bytes.restype = C.c_longlong
     L.glb_tables_create.argtypes = [C.c_int, C.POINTER(C.c_void_p)]
     L.glb_tables_destroy.argtypes = [C.c_void_p]
@@ -138,7 +139,7 @@ def main():
             rows2 = torch.empty((nf2, n), dtype=torch.float32, device="cuda") if ov != 0.5 else rows
             api.force_generic_kernel(ov == 0.5)
             try:
-                sb = L.glb_iq_gram_scratch_bytes(n, h2, nf2, 0)
+                sb = L.glb_iq_gram_scratch_bytes(n, h2, nf2, 0, 1, 0)
                 scratch = torch.empty(sb, dtype=torch.uint8, device="cuda")
                 fg = lambda: iq_launch(n, h2, rows2, taper, tables, scratch.data_ptr())   # noqa: E731
                 fg(); torch.cuda.synchronize()

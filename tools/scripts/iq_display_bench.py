@@ -33,7 +33,8 @@ class IqGramArgs(C.Structure):         # include/glb_shim.h glb_iq_gram_args
                 ("first_frame", C.c_longlong), ("nframes", C.c_longlong), ("rows", C.c_void_p), ("tables", C.c_void_p),
                 ("scratch", C.c_void_p), ("levels", C.c_void_p), ("levels_stride", C.c_longlong),
                 ("level_tables", C.c_void_p), ("levels_log", C.c_int), ("level_lut", C.c_void_p), ("level_min", C.c_float),
-                ("level_max", C.c_float), ("level_thr", C.c_float), ("ntapers", C.c_int)]
+                ("level_max", C.c_float), ("level_thr", C.c_float), ("ntapers", C.c_int),
+                ("ftest", C.c_void_p), ("ftest_taper", C.c_void_p), ("ftest_u0", C.c_void_p), ("ftest_s", C.c_float)]
 
 
 def gpu_info():

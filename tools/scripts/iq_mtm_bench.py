@@ -40,7 +40,8 @@ class IqGramArgs(C.Structure):         # include/glb_shim.h glb_iq_gram_args
                 ("first_frame", C.c_longlong), ("nframes", C.c_longlong), ("rows", C.c_void_p), ("tables", C.c_void_p),
                 ("scratch", C.c_void_p), ("levels", C.c_void_p), ("levels_stride", C.c_longlong),
                 ("level_tables", C.c_void_p), ("levels_log", C.c_int), ("level_lut", C.c_void_p), ("level_min", C.c_float),
-                ("level_max", C.c_float), ("level_thr", C.c_float), ("ntapers", C.c_int)]
+                ("level_max", C.c_float), ("level_thr", C.c_float), ("ntapers", C.c_int),
+                ("ftest", C.c_void_p), ("ftest_taper", C.c_void_p), ("ftest_u0", C.c_void_p), ("ftest_s", C.c_float)]
 
 
 def gpu_info():
@@ -84,7 +85,7 @@ def main():
         raise SystemExit("iq_mtm_bench needs a CUDA device")
     L = api.lib()
     L.glb_launch_iq_gram.argtypes = [C.POINTER(IqGramArgs), C.c_void_p]
-    L.glb_iq_gram_scratch_bytes.argtypes = [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int]
+    L.glb_iq_gram_scratch_bytes.argtypes = [C.c_int, C.c_int, C.c_longlong, C.c_int, C.c_int, C.c_int]
     L.glb_iq_gram_scratch_bytes.restype = C.c_longlong
     L.glb_tables_create.argtypes = [C.c_int, C.POINTER(C.c_void_p)]
     L.glb_tables_destroy.argtypes = [C.c_void_p]
@@ -118,7 +119,7 @@ def main():
         tables = C.c_void_p()
         api._check(L.glb_tables_create(2 * n, C.byref(tables)))
         api.force_generic_kernel(generic)
-        sb = L.glb_iq_gram_scratch_bytes(n, hop, nf, 0, k)
+        sb = L.glb_iq_gram_scratch_bytes(n, hop, nf, 0, k, 0)
         api.force_generic_kernel(False)
         scratch = torch.empty(max(sb, 4), dtype=torch.uint8, device="cuda")
         g = IqGramArgs(n, hop, dev.data_ptr(), 0, ns, tab.data_ptr(), sym, ts, 0, nf, rows.data_ptr(), tables,
