@@ -208,6 +208,9 @@ def lib() -> C.CDLL:
         l.glb_force_generic_kernel.restype = None
         l.glb_set_kernel_preference.argtypes = [C.c_int]
         l.glb_set_kernel_preference.restype = None
+        l.glb_set_ring_groups.argtypes = [C.c_int]
+        l.glb_set_ring_groups.restype = None
+        l.glb_last_frames_per_group.restype = C.c_int
         _lib = l
     return _lib
 
@@ -755,6 +758,17 @@ def palette(p: int) -> np.ndarray:
 def force_generic_kernel(on: bool) -> None:
     """testing aid: run the general kernel where the TMA ring kernel would be chosen"""
     lib().glb_force_generic_kernel(int(on))
+
+
+def set_ring_groups(groups: int) -> None:
+    """testing aid: groups > 0 replaces the frame-group count of fused I/Q launches (at most one group per frame), so
+    that a short run holds several frames per group; 0 (the default) restores the launch policy"""
+    lib().glb_set_ring_groups(int(groups))
+
+
+def last_frames_per_group() -> int:
+    """testing aid: frames per group of the last fused I/Q launch"""
+    return int(lib().glb_last_frames_per_group())
 
 
 def set_kernel_preference(pref: int) -> None:

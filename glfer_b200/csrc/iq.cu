@@ -34,6 +34,13 @@ int glb_tables_get(const void *tables, int *n, const float2 **tw, const float2 *
 // the contract's |Z|^2 / n divided by 8: the epilogue multiplies by 8, exactly.
 constexpr float kIqPowerScale = 8.f;
 
+// testing aid (glb_set_ring_groups): > 0 replaces the frame-group count of the fused launch policy, so that short runs
+// put several frames into every group and reach the ring's steady state
+static int g_ring_groups = 0;
+static int g_last_frames_per_group = 0;
+extern "C" void glb_set_ring_groups(int groups) { g_ring_groups = groups > 0 ? groups : 0; }
+extern "C" int glb_last_frames_per_group(void) { return g_last_frames_per_group; }
+
 template <int M, int QSC, bool LEV = false>
 __global__ void __launch_bounds__(Geo<M>::THREADS, (RingGeo<M, false>::MINB)) gram_iq_kernel(const KParams p) {
   using GeoM = Geo<M>;
@@ -595,11 +602,13 @@ static int launch_iq_fused(const KParams &kp, const IqFtestParams *fp, cudaStrea
     while (waves > 1 && kp.nframes < groups * waves * kRingMinRun) waves--;
     groups *= waves;
   }
+  if (g_ring_groups > 0) groups = g_ring_groups;
   if (groups > kp.nframes) groups = kp.nframes;
   if (groups < 1) groups = 1;
   KParams k = kp;
   k.qs = qs;
   k.frames_per_group = (int) ((kp.nframes + groups - 1) / groups);
+  g_last_frames_per_group = k.frames_per_group;
   const long long used = (kp.nframes + k.frames_per_group - 1) / k.frames_per_group;
   const int ctas = (int) ((used + GeoM::G - 1) / GeoM::G);
   if (fp) fk<<<ctas, GeoM::THREADS, smem, st>>>(k, *fp);

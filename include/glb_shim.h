@@ -259,6 +259,12 @@ int glb_launch_iq_gram(const glb_iq_gram_args *a, void *stream);
  * arguments (the general path reuses one spectrum plane for all tapers, so the size does not grow with it);
  * ftest: 1 when the launch writes F rows (the general path then also holds the mu and den planes) */
 long long glb_iq_gram_scratch_bytes(int n, int hop, long long nframes, int levels, int ntapers, int ftest);
+/* testing aids of the fused I/Q kernels: groups > 0 replaces the number of frame groups the launch policy picks
+ * (still at most one per frame), so that a short run puts several frames into each group and exercises the ring's
+ * steady state; 0, the default, restores the policy.  Occupancy, shared memory and the kernel choice are unchanged. */
+void glb_set_ring_groups(int groups);
+/* frames per group of the last fused I/Q launch */
+int glb_last_frames_per_group(void);
 /* the general path: the general spectrogram kernel's spectrum output on the 2n-float frames (into scratch, at
  * least nframes (n + 1) (re, im) pairs), then glb_launch_zoom_split; multitaper: that spectrum once per taper, each
  * followed by a split that stores (taper 0) or adds (the others) its powers into the rows.  F-test: scratch holds
