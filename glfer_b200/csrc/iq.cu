@@ -632,14 +632,13 @@ static bool iq_fused_geometry(int n, int hop) {
 
 static bool iq_fused_allowed() { return g_force_generic == 0 && g_kernel_pref != 1; }
 
-// general path: the spectrum [nframes][n + 1] (re, im) pairs, then, for a launch with levels, the float rows
-// [nframes][n] that levels_kernel maps, or, for an F-test launch, the mu plane [nframes][n] (re, im) pairs and the den
-// plane [nframes][n] floats.  A multitaper launch reuses the one spectrum plane for every taper and the fused kernel
-// serves it wherever it serves the periodogram, so the size does not depend on ntapers.
+// the general path's scratch (glb_iq_gram_general_scratch_bytes, zoom.cu).  A multitaper launch reuses the one spectrum
+// plane for every taper and the fused kernel serves it wherever it serves the periodogram, so the size does not depend
+// on ntapers.
 extern "C" long long glb_iq_gram_scratch_bytes(int n, int hop, long long nframes, int levels, int ntapers, int ftest) {
   (void) ntapers;
   if (nframes <= 0 || (iq_fused_allowed() && iq_fused_geometry(n, hop))) return 0;
-  return nframes * ((long long) (n + 1) * 2 + (levels ? n : 0) + (ftest ? 3LL * n : 0)) * (long long) sizeof(float);
+  return glb_iq_gram_general_scratch_bytes(n, nframes, levels, ftest);
 }
 
 extern "C" int glb_launch_iq_gram(const glb_iq_gram_args *a, void *stream) {

@@ -1,6 +1,6 @@
 // zoom.cu -- kernels of the zoom spectrogram (host/zoom.c): mix a centre frequency to DC, low-pass and
-// decimate by D, then turn the general spectrogram kernel's real-FFT output of the decimated stream into
-// complex-FFT rows.
+// decimate by D; and the general path of complex frames (glb_launch_iq_gram_general, the zoom's and the I/Q plans'
+// frame stage, host/cframe.c), which turns the general spectrogram kernel's real-FFT output into complex-FFT rows.
 //
 //   zoom_decim_kernel<T>  the hot path.  y[m] = e^{-2 pi i phi(mD)} sum_j g[j] x[mD - K + j], j = 0..2K,
 //                         with the complex taps g[j] = h[K - j] e^{+2 pi i phi(K - j)} built on the host.
@@ -16,8 +16,9 @@
 //                         output falls in a launch or chunk.  int16 input is converted in registers.
 //                         T = float2 / short2: complex (I, Q) input, four FMAs per tap in an order that
 //                         rounds exactly as the real kernel's when Q = 0.
-//   zoom_split_kernel     X[k], k = 0..Nz, of the interleaved (re, im) stream seen as 2 Nz real points ->
-//                         Z[k] = E + iO of the complex frame -> |Z|^2 / Nz in fft-shifted bin order.
+//   iq_split_z            X[k], k = 0..Nz, of the interleaved (re, im) stream seen as 2 Nz real points ->
+//                         Z[k] = E + iO of the complex frame; every split kernel below forms Z with it.
+//   zoom_split_kernel     |Z|^2 / Nz in fft-shifted bin order.
 //   iq_mtm_split_kernel   the same split for one taper of a multitaper row: taper 0 stores |Z_0|^2 / Nz, taper
 //                         k > 0 adds |Z_k|^2 / Nz to the row, so the tapers are summed in the order k = 0..K'-1.
 //   iq_ftest_*_kernel     the harmonic F-test on the general path: the hn spectrum split into the mu plane, each
@@ -142,53 +143,8 @@ zoom_decim_kernel(const T *__restrict__ x, long long origin, long long count, in
   }
 }
 
-__global__ void zoom_split_kernel(const float2 *__restrict__ spec, int nz, long long nframes, float inv_nz,
-                                  float *__restrict__ rows) {
-  const long long total = nframes * nz;
-  const long long stride = (long long) gridDim.x * blockDim.x;
-  for (long long idx = (long long) blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += stride) {
-    const long long f = idx / nz;
-    const int j = (int) (idx - f * nz);
-    const int k = (j + nz / 2) & (nz - 1);
-    const float2 *X = spec + f * (nz + 1);
-    const float2 a = X[k], c = X[nz - k];
-    // E = (X[k] + conj X[Nz-k]) / 2,  O = (X[k] - conj X[Nz-k]) / (2 W^k),  W = e^{-i pi / Nz}
-    const float er = 0.5f * (a.x + c.x), ei = 0.5f * (a.y - c.y);
-    const float dr = 0.5f * (a.x - c.x), di = 0.5f * (a.y + c.y);
-    float sn, cs;
-    sincospif((float) k / (float) nz, &sn, &cs);
-    const float orr = dr * cs - di * sn, oi = dr * sn + di * cs;
-    const float zr = er - oi, zi = ei + orr;          // Z = E + i O
-    rows[idx] = (zr * zr + zi * zi) * inv_nz;
-  }
-}
-
-// zoom_split_kernel's arithmetic, kept apart so that the periodogram's kernel keeps its exact instructions
-__global__ void iq_mtm_split_kernel(const float2 *__restrict__ spec, int nz, long long nframes, float inv_nz, int add,
-                                    float *__restrict__ rows) {
-  const long long total = nframes * nz;
-  const long long stride = (long long) gridDim.x * blockDim.x;
-  for (long long idx = (long long) blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += stride) {
-    const long long f = idx / nz;
-    const int j = (int) (idx - f * nz);
-    const int k = (j + nz / 2) & (nz - 1);
-    const float2 *X = spec + f * (nz + 1);
-    const float2 a = X[k], c = X[nz - k];
-    const float er = 0.5f * (a.x + c.x), ei = 0.5f * (a.y - c.y);
-    const float dr = 0.5f * (a.x - c.x), di = 0.5f * (a.y + c.y);
-    float sn, cs;
-    sincospif((float) k / (float) nz, &sn, &cs);
-    const float orr = dr * cs - di * sn, oi = dr * sn + di * cs;
-    const float zr = er - oi, zi = ei + orr;
-    const float pw = (zr * zr + zi * zi) * inv_nz;
-    rows[idx] = add ? rows[idx] + pw : pw;
-  }
-}
-
-// The harmonic F-test on the general path (glb_launch_iq_gram_general with ftest).  Z[k] of a frame as the splits above
-// form it; the kernels below are the complex-output split of the hn spectrum (the mu plane), the split of one taper's
-// spectrum that adds its power to the rows as iq_mtm_split_kernel does and its residual to the den plane, and the
-// quotient.  The residual and F are the fused kernel's (iq_core.cuh).
+// Z[k] = E + iO of the complex frame from X[k], k = 0..Nz, the real FFT of its interleaved (re, im) samples seen as
+// 2 Nz real points: E = (X[k] + conj X[Nz-k]) / 2,  O = (X[k] - conj X[Nz-k]) / (2 W^k),  W = e^{-i pi / Nz}
 static __device__ __forceinline__ float2 iq_split_z(const float2 *X, int nz, int k) {
   const float2 a = X[k], c = X[nz - k];
   const float er = 0.5f * (a.x + c.x), ei = 0.5f * (a.y - c.y);
@@ -199,6 +155,36 @@ static __device__ __forceinline__ float2 iq_split_z(const float2 *X, int nz, int
   return make_float2(er - oi, ei + orr);
 }
 
+__global__ void zoom_split_kernel(const float2 *__restrict__ spec, int nz, long long nframes, float inv_nz,
+                                  float *__restrict__ rows) {
+  const long long total = nframes * nz;
+  const long long stride = (long long) gridDim.x * blockDim.x;
+  for (long long idx = (long long) blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += stride) {
+    const long long f = idx / nz;
+    const int j = (int) (idx - f * nz);
+    const float2 z = iq_split_z(spec + f * (nz + 1), nz, (j + nz / 2) & (nz - 1));
+    rows[idx] = (z.x * z.x + z.y * z.y) * inv_nz;
+  }
+}
+
+// zoom_split_kernel for one taper of a multitaper row, kept a kernel of its own so that the periodogram's kernel has
+// no `add` branch
+__global__ void iq_mtm_split_kernel(const float2 *__restrict__ spec, int nz, long long nframes, float inv_nz, int add,
+                                    float *__restrict__ rows) {
+  const long long total = nframes * nz;
+  const long long stride = (long long) gridDim.x * blockDim.x;
+  for (long long idx = (long long) blockIdx.x * blockDim.x + threadIdx.x; idx < total; idx += stride) {
+    const long long f = idx / nz;
+    const int j = (int) (idx - f * nz);
+    const float2 z = iq_split_z(spec + f * (nz + 1), nz, (j + nz / 2) & (nz - 1));
+    const float pw = (z.x * z.x + z.y * z.y) * inv_nz;
+    rows[idx] = add ? rows[idx] + pw : pw;
+  }
+}
+
+// The harmonic F-test on the general path (glb_launch_iq_gram_general with ftest): the complex-output split of the hn
+// spectrum (the mu plane), the split of one taper's spectrum that adds its power to the rows as iq_mtm_split_kernel
+// does and its residual to the den plane, and the quotient.  The residual and F are the fused kernel's (iq_core.cuh).
 __global__ void iq_ftest_mu_kernel(const float2 *__restrict__ spec, int nz, long long nframes, float2 *__restrict__ mu) {
   const long long total = nframes * nz;
   const long long stride = (long long) gridDim.x * blockDim.x;
@@ -299,9 +285,17 @@ extern "C" int glb_launch_zoom_split(const void *spec, int nz, long long nframes
   return GLB_OK;
 }
 
+// The general path's scratch: the spectrum [nframes][n + 1] (re, im) pairs, then, for a launch with levels, the float
+// rows [nframes][n] that levels_kernel maps (their offset is taken in glb_launch_iq_gram, iq.cu), or, for an F-test
+// launch, the mu plane [nframes][n] (re, im) pairs and the den plane [nframes][n] floats (their offsets are taken in
+// glb_launch_iq_gram_general below).
+extern "C" long long glb_iq_gram_general_scratch_bytes(int n, long long nframes, int levels, int ftest) {
+  return nframes * ((long long) (n + 1) * 2 + (levels ? n : 0) + (ftest ? 3LL * n : 0)) * (long long) sizeof(float);
+}
+
 // The general path of complex frames: the interleaved stream seen as a real stream of 2n floats per frame at hop
 // 2 hop, the general spectrogram kernel's spectrum output X[k], k = 0..n, then zoom_split_kernel.  The zoom's frame
-// stage (host/zoom.c) and the I/Q spectrogram's non-fused launches (iq.cu).  Multitaper (ntapers > 1): one spectrum
+// stage (host/cframe.c) and the I/Q spectrogram's non-fused launches (iq.cu).  Multitaper (ntapers > 1): one spectrum
 // per taper into the same scratch plane, each followed by iq_mtm_split_kernel, which sums the tapers into the rows.
 extern "C" int glb_launch_iq_gram_general(const glb_iq_gram_args *a, void *stream) {
   if (!a || (!a->rows && !a->ftest) || a->nframes < 0 || a->ntapers < 0 || a->ntapers > 32 ||

@@ -14,17 +14,14 @@ void glb_window_table(int n, int window_type, float *w);
 int glb_dpss(int n, double nw, int kmax, double *tapers, double *lambda);
 /* host/dpss.c: U0 (double), S and hn (float) of the harmonic F-test from K unit-energy tapers [K][n] */
 void glb_mtm_ftest_weights(int n, int K, const double *tapers, double *u0, float *hn, float *s);
-/* host/iq.c: DPSS and [K'][2n] taper table of a complex multitaper plan (I/Q or zoom); sym: bit k = taper k mirror-symmetric */
-int glb_iq_mtm_tapers(int n, float mtm_w, int mtm_kmax, float taper_scale, double **h_tapers, double **h_lambda,
-                      float **table, int *sym);
-/* host/iq.c: the F-test's device table of a complex multitaper plan, hn [2n] then (U0_k, sqrt(lambda_k)) [K'], and S */
-int glb_iq_ftest_table(int n, int K, const double *h_tapers, const double *h_lambda, float taper_scale, float **d_ftab,
-                       float *s);
 int glb_hop(int n, float overlap);
 /* the message slot of glfer_b200_last_error() (gram.c), for the other host units */
 int glb_host_fail(int code, const char *msg);
 int glb_host_shim(int rc);
 void glb_host_clear_error(void);
+#define TRY(x) do { int rc_ = glb_host_shim(x); if (rc_ != 0) return rc_; } while (0)
+/* grow-only device buffer (gram.c): *ptr holds at least want elements of elem bytes, *cap counts elements */
+int glb_ensure(void **ptr, size_t *cap, size_t want, size_t elem);
 
 /* display mapping tables (host/levels.c) */
 #define GLB_DB_JMIN (-450)
@@ -79,6 +76,72 @@ int glb_display_end(const glb_display *d, const glb_display_run *r, long long nf
                     float *range_out);
 /* testing aid glfer_b200_set_fused_levels (gram.c): 0 = levels always in a second pass over float rows */
 int glb_host_fused_levels(void);
+
+/* the complex frame stage of the I/Q and zoom plans (host/cframe.c): everything after a chunk's complex samples are
+ * on the device.  Chunks in flight: three, as the real plan's (gram.c). */
+#define GLB_CSLOTS 3
+typedef struct {                /* per slot (stream); embedded in the plan's own slot */
+  void *stream;
+  float *d_rows;
+  size_t rows_cap;              /* floats */
+  float *d_ftest;               /* F rows (*_mtm_ftest) */
+  size_t ftest_cap;             /* floats */
+  void *d_scratch;              /* the general path's (glb_iq_gram_scratch_bytes) */
+  size_t scratch_cap;           /* bytes */
+  glb_display_slot disp;        /* display mapping */
+} glb_cslot;
+typedef struct {                /* per plan */
+  int n, hop, device;
+  float overlap;
+  float *d_taper;               /* [ntapers][2n]: w[i] (or v_k[i] / sqrt(lambda_k)) on both halves of complex sample i,
+                                   times taper_scale */
+  int taper_sym;                /* bit k: taper k is mirror-symmetric bit for bit */
+  float taper_scale;            /* 1 / (2 sqrt(2n)) */
+  int ntapers;                  /* 1: periodogram, K' = mtm_kmax + 1: multitaper */
+  double *h_tapers, *h_lambda;  /* multitaper: the unscaled DPSS [K'][n] and eigenvalues */
+  float *d_ftab;                /* multitaper: the F-test's table: hn [2n], then (U0_k, sqrt(lambda_k)) [K'] */
+  float ftest_s;                /* S = sum_k U0_k^2 */
+  void *tables;                 /* FFT tables of the 2n-float frames */
+  glb_display disp;
+  glb_cslot *slot[GLB_CSLOTS];  /* in the plan's slots */
+} glb_cframe;
+/* Validates n (size_msg: the plan's message), window_type, overlap and, for mtm, the DPSS parameters before any device
+ * call; then selects the device, uploads the taper table (the window, or the K' DPSS tapers) and the F-test's table,
+ * builds the FFT tables and creates the slots' streams.  On failure f owns nothing and the message is kept. */
+int glb_cframe_create(glb_cframe *f, glb_cslot *const slot[GLB_CSLOTS], int n, int window_type, float overlap,
+                      int device, int mtm, float mtm_w, int mtm_kmax, const char *size_msg);
+/* synchronises and frees the slots' buffers and streams and the plan's tables (not f itself) */
+void glb_cframe_destroy(glb_cframe *f);
+/* glfer_iq_tapers / glfer_zoom_tapers (f: NULL for a NULL plan) */
+int glb_cframe_tapers(const glb_cframe *f, double *tapers, double *lambda);
+typedef struct glb_cframe_call glb_cframe_call;
+/* the plan's stage of a chunk: the complex samples that frames [c0, c0 + cn) read, on the device of slot i (prev: the
+ * slot of the run's previous chunk, or -1), on that slot's stream; *z holds samples [*z_origin, *z_origin + *z_count) */
+typedef int (*glb_cframe_stage)(void *plan, const glb_cframe_call *c, int i, int prev, long long c0, long long cn,
+                                const float **z, long long *z_origin, long long *z_count);
+struct glb_cframe_call {        /* one run entry's call */
+  const void *src;              /* the caller's samples [origin, origin + count), float or int16 (pcm16) */
+  int pcm16;
+  long long origin, count, first_frame, nframes;
+  int ftest_on;                 /* a *_mtm_ftest entry: rows or ftest may be NULL */
+  float *rows, *ftest;
+  int display;                  /* a *_run_display entry: levels / RGB of dc's mapping */
+  const glfer_display_config *dc;
+  float *agc_state, *range_out;
+  unsigned char *levels, *rgb;
+  /* from the plan */
+  void *plan;
+  glb_cframe_stage stage;
+  long long chunk_frames;
+  long long lo, hi;             /* the plan's required span of the frames */
+  int general;                  /* 1: glb_launch_iq_gram_general (the zoom), 0: glb_launch_iq_gram */
+  int fuse;                     /* display: the spectrogram kernel writes fixed-range levels itself, no float rows */
+  const char *wrong_kind;       /* non-NULL: the entry does not serve this plan (checked after the null arguments) */
+  const char *no_mtm, *short_span;   /* the plan's messages: F-test without a multitaper plan, samples short */
+};
+/* checks the call, then walks its frames in chunks of chunk_frames on the slots in turn: the plan's stage, the launch,
+ * and the rows / F rows downloads or the display chain */
+int glb_cframe_run(glb_cframe *f, const glb_cframe_call *c);
 
 /* values of the hidden globals (weak `opt` / `glfer` when the host program has them) */
 int glb_autoscale(void);

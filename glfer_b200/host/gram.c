@@ -110,8 +110,6 @@ static int shim(int rc)
   return rc;   /* GLB_E* and GLFER_E* share values */
 }
 
-#define TRY(x) do { int rc_ = shim(x); if (rc_ != 0) return rc_; } while (0)
-
 int glb_host_fail(int code, const char *msg) { return fail(code, msg); }
 int glb_host_shim(int rc) { return shim(rc); }
 void glb_host_clear_error(void) { g_msg[0] = 0; }
@@ -344,8 +342,7 @@ int glfer_gram_plan_create(const glfer_gram_config *cfg, glfer_gram_plan **out)
   return GLFER_OK;
 }
 
-/* grow-only device buffers */
-static int ensure(void **ptr, size_t *cap, size_t want, size_t elem)
+int glb_ensure(void **ptr, size_t *cap, size_t want, size_t elem)
 {
   if (want <= *cap) return 0;
   if (*ptr) TRY(glb_free(*ptr));
@@ -360,9 +357,9 @@ static int stage_slot(glfer_gram_plan *p, slot_t *s, const float *samples, const
                       long long count)
 {
   if (count < 0) return fail(GLFER_EINVAL, "negative sample count");
-  TRY(ensure((void **) &s->d_samples, &s->samples_cap, (size_t) count + 2, sizeof(float)));
+  TRY(glb_ensure((void **) &s->d_samples, &s->samples_cap, (size_t) count + 2, sizeof(float)));
   if (pcm) {
-    TRY(ensure((void **) &s->d_pcm, &s->pcm_cap, (size_t) count, sizeof(short)));
+    TRY(glb_ensure((void **) &s->d_pcm, &s->pcm_cap, (size_t) count, sizeof(short)));
     TRY(glb_memcpy_h2d(s->d_pcm, pcm, sizeof(short) * (size_t) count, s->stream));
     TRY(glb_launch_pcm16_to_float(s->d_pcm, s->d_samples, count, s->stream));
   } else {
@@ -392,7 +389,7 @@ static int exec_slot(glfer_gram_plan *p, slot_t *s, long long first, long long n
   if (lo < 0) lo = 0;
   if (lo < s->s_origin || hi > s->s_origin + s->s_count)
     return fail(GLFER_EINVAL, "staged samples do not cover the requested frames (see glfer_gram_required_span)");
-  if (!fl) TRY(ensure((void **) &s->d_psd, &s->psd_cap, (size_t) nf * p->bins, sizeof(float)));
+  if (!fl) TRY(glb_ensure((void **) &s->d_psd, &s->psd_cap, (size_t) nf * p->bins, sizeof(float)));
 
   const float *d_means = NULL;
   long long means_first = 0;
@@ -400,7 +397,7 @@ static int exec_slot(glfer_gram_plan *p, slot_t *s, long long first, long long n
   if (c->sub_mean && !fused_mean) {
     /* irregular hop: block means from a pre-pass over the staged samples */
     const long long b_lo = lo / p->hop, b_hi = first + nframes;      /* blocks [b_lo, b_hi) */
-    TRY(ensure((void **) &s->d_means, &s->means_cap, (size_t) (b_hi - b_lo), sizeof(float)));
+    TRY(glb_ensure((void **) &s->d_means, &s->means_cap, (size_t) (b_hi - b_lo), sizeof(float)));
     TRY(glb_launch_block_means(s->d_samples, s->s_origin, s->s_count, p->hop, b_lo, b_hi - b_lo, s->d_means, s->stream));
     d_means = s->d_means;
     means_first = b_lo;
@@ -444,7 +441,7 @@ static int exec_slot(glfer_gram_plan *p, slot_t *s, long long first, long long n
   glb_avg_args a;
   memset(&a, 0, sizeof a);
   if (c->avg_mode != GLFER_NO_AVG) {
-    TRY(ensure((void **) &s->d_avg, &s->avg_cap, (size_t) nframes * p->avg_cols, sizeof(float)));
+    TRY(glb_ensure((void **) &s->d_avg, &s->avg_cap, (size_t) nframes * p->avg_cols, sizeof(float)));
     if ((size_t) nframes > s->scal_cap) {
       glb_free(s->d_ret); glb_free(s->d_var); glb_free(s->d_cand); glb_free(s->d_peak);
       s->d_ret = s->d_var = NULL; s->d_cand = s->d_peak = NULL; s->scal_cap = 0;
@@ -516,7 +513,7 @@ static int exec_slot(glfer_gram_plan *p, slot_t *s, long long first, long long n
   }
   if (c->mode == GLFER_MODE_LMP) {
     /* the rows handed out are the detector statistic over the ring of the last lmp_av PSD rows */
-    TRY(ensure((void **) &s->d_avg, &s->avg_cap, (size_t) nframes * p->bins, sizeof(float)));
+    TRY(glb_ensure((void **) &s->d_avg, &s->avg_cap, (size_t) nframes * p->bins, sizeof(float)));
     TRY(glb_launch_lmp(s->d_psd, f0, p->bins, 0, p->bins, first, nframes, c->lmp_av, c->scale_db, s->d_avg, p->bins, s->stream));
   }
   s->out_first = first;
@@ -607,8 +604,8 @@ static int ftest_slot(glfer_gram_plan *p, slot_t *s, long long first, long long 
 {
   const glfer_gram_config *c = &p->cfg;
   const size_t plane = (size_t) nframes * p->bins;
-  TRY(ensure((void **) &p->d_fspec, &p->fspec_cap, plane * 2 * (size_t) (p->ntapers + 1), sizeof(float)));
-  TRY(ensure((void **) &p->d_ftest, &p->ftest_cap, plane, sizeof(float)));
+  TRY(glb_ensure((void **) &p->d_fspec, &p->fspec_cap, plane * 2 * (size_t) (p->ntapers + 1), sizeof(float)));
+  TRY(glb_ensure((void **) &p->d_ftest, &p->ftest_cap, plane, sizeof(float)));
   long long lo, hi;
   glfer_gram_required_span(p, first, nframes, &lo, &hi);
   if (lo < 0) lo = 0;
@@ -617,7 +614,7 @@ static int ftest_slot(glfer_gram_plan *p, slot_t *s, long long first, long long 
   const int fused_mean = c->sub_mean && glb_gram_fused_mean_ok(c->n, p->hop);
   if (c->sub_mean && !fused_mean) {
     const long long b_lo = lo / p->hop, b_hi = first + nframes;
-    TRY(ensure((void **) &s->d_means, &s->means_cap, (size_t) (b_hi - b_lo), sizeof(float)));
+    TRY(glb_ensure((void **) &s->d_means, &s->means_cap, (size_t) (b_hi - b_lo), sizeof(float)));
     TRY(glb_launch_block_means(s->d_samples, s->s_origin, s->s_count, p->hop, b_lo, b_hi - b_lo, s->d_means, s->stream));
     d_means = s->d_means;
     means_first = b_lo;

@@ -272,6 +272,9 @@ int glb_last_frames_per_group(void);
  * the spectrum), each taper's split also adds its residual to the den plane ([nframes][n] floats behind mu), and a
  * last kernel forms F */
 int glb_launch_iq_gram_general(const glb_iq_gram_args *a, void *stream);
+/* device scratch glb_launch_iq_gram_general needs for nframes frames: the spectrum, then the float rows (levels = 1,
+ * the two-pass levels of glb_launch_iq_gram) or the mu and den planes (ftest = 1) */
+long long glb_iq_gram_general_scratch_bytes(int n, long long nframes, int levels, int ftest);
 
 /* counters */
 unsigned long long glb_kernel_launches(void);
