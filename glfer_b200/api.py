@@ -145,6 +145,13 @@ def lib() -> C.CDLL:
         l.glfer_zoom_taps.argtypes = [C.c_int, C.c_void_p]
         l.glfer_zoom_plan_create_iq.argtypes = [C.POINTER(ZoomConfig), C.POINTER(C.c_void_p)]
         l.glfer_zoom_run_iq.argtypes = zoom_args
+        l.glfer_zoom_plan_create_bank.argtypes = [C.POINTER(ZoomConfig), C.c_void_p, C.c_int, C.c_int,
+                                                  C.POINTER(C.c_void_p)]
+        l.glfer_zoom_plan_create_bank_mtm.argtypes = [C.POINTER(ZoomConfig), C.c_void_p, C.c_int, C.c_int, C.c_float,
+                                                      C.c_int, C.POINTER(C.c_void_p)]
+        l.glfer_zoom_channels.argtypes = [C.c_void_p]
+        l.glfer_zoom_channel_center_hz.argtypes = [C.c_void_p, C.c_int]
+        l.glfer_zoom_channel_center_hz.restype = C.c_double
         l.glfer_zoom_run_iq_pcm16.argtypes = zoom_args
         # I/Q spectrogram
         l.glfer_iq_plan_create.argtypes = [C.POINTER(IqConfig), C.POINTER(C.c_void_p)]
@@ -438,21 +445,23 @@ class GramPlan:
 
 
 def _run_display(fn, handle, ptr, count, bins, nframes, log_scale, autoscale, max_level_db, min_level_db, thr_level,
-                 colortab, origin, first_frame, agc_state, want_rgb, out, want_range):
-    """one *_run_display call of an I/Q or zoom plan, with the keywords and outputs of GramPlan.run_display"""
+                 colortab, origin, first_frame, agc_state, want_rgb, out, want_range, lead=()):
+    """one *_run_display call of an I/Q or zoom plan, with the keywords and outputs of GramPlan.run_display; lead: (C,)
+    for a zoom bank, whose outputs and agc_state carry a leading channel axis"""
     out = out or {}
-    levels = out.get("levels") if "levels" in out else np.empty((nframes, bins), np.uint8)
-    assert levels.dtype == np.uint8 and levels.size >= nframes * bins
-    rgb = np.empty((nframes, bins, 3), np.uint8) if want_rgb else None
+    nc = int(np.prod(lead, dtype=np.int64))
+    levels = out.get("levels") if "levels" in out else np.empty(lead + (nframes, bins), np.uint8)
+    assert levels.dtype == np.uint8 and levels.size >= nc * nframes * bins
+    rgb = np.empty(lead + (nframes, bins, 3), np.uint8) if want_rgb else None
     rng = None
     if autoscale and want_range:
-        rng = out.get("range") if "range" in out else np.empty((nframes, 2), np.float32)
+        rng = out.get("range") if "range" in out else np.empty(lead + (nframes, 2), np.float32)
     if colortab is not None:
         colortab = np.ascontiguousarray(colortab, dtype=np.uint8)
         assert colortab.size == 768
     dc = DisplayConfig(int(log_scale), int(autoscale), max_level_db, min_level_db, thr_level,
                        colortab.ctypes.data if colortab is not None else None)
-    state = agc_state if agc_state is not None else np.zeros(2, np.float32)
+    state = agc_state if agc_state is not None else np.zeros(lead + (2,), np.float32)
     _check(fn(handle, ptr, origin, count, first_frame, nframes, C.byref(dc), state.ctypes.data, _ptr(levels), _ptr(rgb),
               _ptr(rng)))
     return dict(levels=levels, rgb=rgb, range=rng, agc_state=state)
@@ -482,16 +491,27 @@ class ZoomPlan:
     Rows hold n bins in frequency order, bin j at center_hz() + (j - n/2) * sample_rate / (decim * n).
     iq=True: complex (I/Q) input (glfer_zoom_plan_create_iq), centre in [-sample_rate/2, sample_rate/2].
     multitaper=True: rows of K' = mtm_kmax + 1 DPSS tapers of NW = mtm_w (glfer_zoom_plan_create[_iq]_mtm; window_type
-    is ignored)."""
+    is ignored).
+    center_hz a sequence: a channel bank (glfer_zoom_plan_create_bank[_mtm]), one channel per centre; run,
+    run_mtm_ftest and run_display then return arrays with a leading channel axis, (C, nframes, n), and run_display
+    takes and returns agc_state of shape (C, 2)."""
 
     def __init__(self, n=4096, decim=256, window_type=HANNING, overlap=0.0, center_hz=800.0, sample_rate=48000.0,
                  device=0, iq=False, multitaper=False, mtm_w=4.0, mtm_kmax=7):
-        self.cfg = ZoomConfig(n, decim, window_type, overlap, center_hz, sample_rate, device)
+        self.bank = np.ndim(center_hz) > 0
+        centers = np.ascontiguousarray(center_hz, dtype=np.float64).reshape(-1)
+        self.cfg = ZoomConfig(n, decim, window_type, overlap, 0.0 if self.bank else center_hz, sample_rate, device)
         self._h = C.c_void_p()
         self.iq = iq
         self.multitaper = multitaper
         self.mtm_kmax = mtm_kmax
-        if multitaper:
+        if self.bank and multitaper:
+            _check(lib().glfer_zoom_plan_create_bank_mtm(C.byref(self.cfg), centers.ctypes.data, len(centers), int(iq),
+                                                         mtm_w, mtm_kmax, C.byref(self._h)))
+        elif self.bank:
+            _check(lib().glfer_zoom_plan_create_bank(C.byref(self.cfg), centers.ctypes.data, len(centers), int(iq),
+                                                     C.byref(self._h)))
+        elif multitaper:
             create = lib().glfer_zoom_plan_create_iq_mtm if iq else lib().glfer_zoom_plan_create_mtm
             _check(create(C.byref(self.cfg), mtm_w, mtm_kmax, C.byref(self._h)))
         else:
@@ -501,6 +521,8 @@ class ZoomPlan:
         self.decim = decim
         self.hop = lib().glfer_zoom_hop(self._h)
         self.bins = lib().glfer_zoom_bins(self._h)
+        self.channels = lib().glfer_zoom_channels(self._h)
+        self._lead = (self.channels,) if self.bank else ()
 
     def close(self):
         if self._h:
@@ -514,8 +536,12 @@ class ZoomPlan:
             pass
 
     def center_hz(self) -> float:
-        """the actual centre, step * sample_rate / 2**32"""
+        """the actual centre, step * sample_rate / 2**32 (channel 0's of a bank)"""
         return float(lib().glfer_zoom_center_hz(self._h))
+
+    def centers_hz(self) -> np.ndarray:
+        """the actual centre of every channel, float64 [C]"""
+        return np.array([lib().glfer_zoom_channel_center_hz(self._h, c) for c in range(self.channels)], np.float64)
 
     def num_frames(self, nsamples: int) -> int:
         return int(lib().glfer_zoom_num_frames(self._h, nsamples))
@@ -534,14 +560,14 @@ class ZoomPlan:
 
     def run(self, samples: np.ndarray, origin: int = 0, first_frame: int = 0, nframes: int | None = None,
             out: np.ndarray | None = None) -> np.ndarray:
-        """glfer_zoom_run / glfer_zoom_run_pcm16 (int16 samples): rows [nframes][n].  out: optional
-        pre-allocated (e.g. pinned) rows.  An I/Q plan takes the formats of IqPlan.run."""
+        """glfer_zoom_run / glfer_zoom_run_pcm16 (int16 samples): rows [nframes][n] ([C][nframes][n] for a bank).
+        out: optional pre-allocated (e.g. pinned) rows.  An I/Q plan takes the formats of IqPlan.run."""
         if self.iq:
             ptr, count, pcm = _iq_samples(samples)
             if nframes is None:
                 nframes = self.num_frames(origin + count) - first_frame
-            rows = out if out is not None else np.empty((nframes, self.bins), np.float32)
-            assert rows.dtype == np.float32 and rows.size >= nframes * self.bins
+            rows = out if out is not None else np.empty(self._lead + (nframes, self.bins), np.float32)
+            assert rows.dtype == np.float32 and rows.size >= self.channels * nframes * self.bins
             fn = lib().glfer_zoom_run_iq_pcm16 if pcm else lib().glfer_zoom_run_iq
             _check(fn(self._h, ptr, origin, count, first_frame, nframes, rows.ctypes.data))
             return rows
@@ -549,8 +575,8 @@ class ZoomPlan:
         assert samples.flags["C_CONTIGUOUS"] and (pcm or samples.dtype == np.float32)
         if nframes is None:
             nframes = self.num_frames(origin + len(samples)) - first_frame
-        rows = out if out is not None else np.empty((nframes, self.bins), np.float32)
-        assert rows.dtype == np.float32 and rows.size >= nframes * self.bins
+        rows = out if out is not None else np.empty(self._lead + (nframes, self.bins), np.float32)
+        assert rows.dtype == np.float32 and rows.size >= self.channels * nframes * self.bins
         fn = lib().glfer_zoom_run_pcm16 if pcm else lib().glfer_zoom_run
         _check(fn(self._h, samples.ctypes.data, origin, len(samples), first_frame, nframes, rows.ctypes.data))
         return rows
@@ -569,7 +595,8 @@ class ZoomPlan:
             fn = lib().glfer_zoom_run_mtm_ftest_pcm16 if pcm else lib().glfer_zoom_run_mtm_ftest
         if nframes is None:
             nframes = self.num_frames(origin + count) - first_frame
-        return _run_ftest(fn, self._h, ptr, origin, count, first_frame, nframes, self.bins, want_psd, want_ftest)
+        return _run_ftest(fn, self._h, ptr, origin, count, first_frame, nframes, self.bins, want_psd, want_ftest,
+                          self._lead)
 
     def run_display(self, samples: np.ndarray, log_scale=True, autoscale=True, max_level_db=-20.0, min_level_db=-80.0,
                     thr_level=0.0, colortab: np.ndarray | None = None, origin: int = 0, first_frame: int = 0,
@@ -588,7 +615,7 @@ class ZoomPlan:
         if nframes is None:
             nframes = self.num_frames(origin + count) - first_frame
         return _run_display(fn, self._h, ptr, count, self.bins, nframes, log_scale, autoscale, max_level_db, min_level_db,
-                            thr_level, colortab, origin, first_frame, agc_state, want_rgb, out, want_range)
+                            thr_level, colortab, origin, first_frame, agc_state, want_rgb, out, want_range, self._lead)
 
 
 class IqPlan:
@@ -671,9 +698,9 @@ class IqPlan:
                             thr_level, colortab, origin, first_frame, agc_state, want_rgb, out, want_range)
 
 
-def _run_ftest(fn, h, ptr, origin, count, first_frame, nframes, bins, want_psd, want_ftest):
-    psd = np.empty((nframes, bins), np.float32) if want_psd else None
-    ft = np.empty((nframes, bins), np.float32) if want_ftest else None
+def _run_ftest(fn, h, ptr, origin, count, first_frame, nframes, bins, want_psd, want_ftest, lead=()):
+    psd = np.empty(lead + (nframes, bins), np.float32) if want_psd else None
+    ft = np.empty(lead + (nframes, bins), np.float32) if want_ftest else None
     _check(fn(h, ptr, origin, count, first_frame, nframes, _ptr(psd), _ptr(ft)))
     return dict(psd=psd, ftest=ft)
 

@@ -143,6 +143,110 @@ zoom_decim_kernel(const T *__restrict__ x, long long origin, long long count, in
   }
 }
 
+// The bank decimator: zoom_decim_kernel for C channels (centres) of one input in one pass.  A CTA owns a tile of
+// NB G kZR consecutive outputs and CG channels (CG NB <= kZWarps warps, warp w: channel w mod CG, output block
+// w / CG of G kZR outputs); blockIdx.y picks the channel group.  The tile's input is staged in shared memory one
+// phase chunk of LG phases at a time -- rows q of u_p[q] for p in the chunk, converted once -- and every warp runs
+// its channel's 33-tap FIRs over it.  A lane owns the same (phase set, outputs) as in zoom_decim_kernel, walks the
+// chunks in ascending phase order and the taps in ascending order, and the partials are summed in the same order,
+// so every output is bit-identical to zoom_decim_kernel's with that channel's taps and dstep.
+template <typename T> struct ZStage { using type = float; };
+template <> struct ZStage<float2> { using type = float2; };
+template <> struct ZStage<short2> { using type = float2; };
+struct ZBankSteps { unsigned v[GLB_ZOOM_MAX_CHANNELS]; };
+
+template <typename T>
+__global__ void __launch_bounds__(kZWarps * 32, 2)
+zoom_bank_decim_kernel(const T *__restrict__ x, long long origin, long long count, int D, int LG, int G, int nchan,
+                       int CG, int NB, const float2 *__restrict__ taps, ZBankSteps dstep, long long m_first,
+                       long long m_count, float2 *__restrict__ y, long long y_stride) {
+  using S = typename ZStage<T>::type;
+  extern __shared__ float4 zb_smem[];
+  S *stage = reinterpret_cast<S *>(zb_smem);                   // [nout + kZT - 1][LG]
+  __shared__ float part[kZWarps][32][2 * kZR + 1];
+  const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+  const int gi = lane / LG, sl = lane - gi * LG;
+  const int bw = w / CG, ch = blockIdx.y * CG + (w - bw * CG);
+  const bool warp_on = bw < NB && ch < nchan;
+  const bool active = warp_on && gi < G;
+  const int nout = NB * G * kZR, rows = nout + kZT - 1;
+  const int ob = (bw * G + gi) * kZR;                          // the lane's first output (row) in the tile
+  const float2 *tp = taps + (size_t) (warp_on ? ch : 0) * kZT * D;
+  const long long K = 16LL * D;
+  const long long ntile = (m_count + nout - 1) / nout;
+  for (long long b = blockIdx.x; b < ntile; b += gridDim.x) {
+    const long long mt = m_first + b * nout;
+    const long long i0 = mt * D - K - origin;
+    float ar[kZR], ai[kZR];
+#pragma unroll
+    for (int r = 0; r < kZR; r++) ar[r] = ai[r] = 0.f;
+    for (int p0 = 0; p0 < D; p0 += LG) {
+      const int pw = D - p0 < LG ? D - p0 : LG;
+      __syncthreads();
+#pragma unroll 4
+      for (int e = threadIdx.x; e < rows * pw; e += blockDim.x) {
+        const int q = e / pw, pp = e - q * pw;
+        stage[q * LG + pp] = zload(x, i0 + (long long) q * D + p0 + pp, count);
+      }
+      __syncthreads();
+      if (active && sl < pw) {
+        const int p = p0 + sl;
+        float tr[kZT], ti[kZT];
+#pragma unroll
+        for (int t = 0; t < kZT; t++) {
+          const float2 c = __ldg(tp + t * D + p);
+          tr[t] = c.x;
+          ti[t] = c.y;
+        }
+        const S *u_p = stage + ob * LG + sl;
+#pragma unroll
+        for (int q = 0; q < kZR + kZT - 1; q++) {
+          const S u = u_p[q * LG];
+#pragma unroll
+          for (int r = 0; r < kZR; r++) {
+            const int t = q - r;
+            if (t >= 0 && t < kZT) {
+              if constexpr (ZComplex<T>::value) {
+                ar[r] = fmaf(tr[t], u.x, ar[r]);
+                ar[r] = fmaf(-ti[t], u.y, ar[r]);
+                ai[r] = fmaf(ti[t], u.x, ai[r]);
+                ai[r] = fmaf(tr[t], u.y, ai[r]);
+              } else {
+                ar[r] = fmaf(tr[t], u, ar[r]);
+                ai[r] = fmaf(ti[t], u, ai[r]);
+              }
+            }
+          }
+        }
+      }
+    }
+#pragma unroll
+    for (int r = 0; r < kZR; r++) {
+      part[w][lane][2 * r] = ar[r];
+      part[w][lane][2 * r + 1] = ai[r];
+    }
+    __syncwarp();
+    if (warp_on) {
+      for (int o = lane; o < G * kZR; o += 32) {
+        const int g = o / kZR, r = o - g * kZR;
+        const long long m = mt + (long long) bw * G * kZR + o;
+        float sr = 0.f, si = 0.f;
+        for (int s = 0; s < LG; s++) {
+          sr += part[w][g * LG + s][2 * r];
+          si += part[w][g * LG + s][2 * r + 1];
+        }
+        if (m < m_first + m_count) {
+          const unsigned ph = (unsigned) (unsigned long long) m * dstep.v[ch];
+          float sn, cs;
+          sincospif((float) (int) ph * 4.656612873077393e-10f, &sn, &cs);
+          y[(size_t) ch * y_stride + (m - m_first)] = make_float2(fmaf(sr, cs, si * sn), fmaf(si, cs, -(sr * sn)));
+        }
+      }
+    }
+    __syncwarp();
+  }
+}
+
 // Z[k] = E + iO of the complex frame from X[k], k = 0..Nz, the real FFT of its interleaved (re, im) samples seen as
 // 2 Nz real points: E = (X[k] + conj X[Nz-k]) / 2,  O = (X[k] - conj X[Nz-k]) / (2 W^k),  W = e^{-i pi / Nz}
 static __device__ __forceinline__ float2 iq_split_z(const float2 *X, int nz, int k) {
@@ -266,6 +370,57 @@ extern "C" int glb_launch_zoom_decim_iq(const void *x, int pcm16, long long orig
   if (m_count <= 0) return GLB_OK;
   if (pcm16) return launch_decim((const short2 *) x, origin, count, decim, taps, dstep, m_first, m_count, y, stream);
   return launch_decim((const float2 *) x, origin, count, decim, taps, dstep, m_first, m_count, y, stream);
+}
+
+template <typename T>
+static int launch_bank_decim(const T *x, long long origin, long long count, int decim, int nchan, const void *taps,
+                             const unsigned *dstep, long long m_first, long long m_count, void *y, long long y_stride,
+                             void *stream) {
+  const int lg = decim < 32 ? decim : 32;
+  const int g = 32 / lg;
+  const int cg = nchan < kZWarps ? nchan : kZWarps;
+  const int nb = kZWarps / cg;
+  const int nout = nb * g * kZR;
+  const size_t smem = (size_t) (nout + kZT - 1) * lg * sizeof(typename ZStage<T>::type);
+  // the stage is at most 40 KB beside the partials' 33 KB of static shared memory (on the current device)
+  ZCU(cudaFuncSetAttribute(zoom_bank_decim_kernel<T>, cudaFuncAttributeMaxDynamicSharedMemorySize, 48 << 10));
+  ZBankSteps st;
+  memset(&st, 0, sizeof st);
+  for (int c = 0; c < nchan; c++) st.v[c] = dstep[c];
+  const int gy = (nchan + cg - 1) / cg;
+  const long long ntile = (m_count + nout - 1) / nout;
+  long long gx = (long long) sm_count() * 2 / gy;
+  if (gx < 1) gx = 1;
+  if (gx > ntile) gx = ntile;
+  zoom_bank_decim_kernel<T><<<dim3((unsigned) gx, (unsigned) gy), kZWarps * 32, smem, (cudaStream_t) stream>>>(
+      x, origin, count, decim, lg, g, nchan, cg, nb, (const float2 *) taps, st, m_first, m_count, (float2 *) y,
+      y_stride);
+  ZCU(cudaGetLastError());
+  g_launches++;
+  return GLB_OK;
+}
+
+extern "C" int glb_launch_zoom_bank_decim(const void *x, int pcm16, int iq, long long origin, long long count,
+                                          int decim, int nchan, const void *taps, const unsigned *dstep,
+                                          long long m_first, long long m_count, void *y, long long y_stride,
+                                          void *stream) {
+  if (decim < 2 || decim > 1024 || nchan < 1 || nchan > GLB_ZOOM_MAX_CHANNELS || !taps || !dstep || !y ||
+      origin < 0 || count < 0 || m_first < 0 || (nchan > 1 && y_stride < m_count)) {
+    glb_set_error("glb_launch_zoom_bank_decim: invalid arguments");
+    return GLB_EINVAL;
+  }
+  if (m_count <= 0) return GLB_OK;
+  if (iq && pcm16)
+    return launch_bank_decim((const short2 *) x, origin, count, decim, nchan, taps, dstep, m_first, m_count, y,
+                             y_stride, stream);
+  if (iq)
+    return launch_bank_decim((const float2 *) x, origin, count, decim, nchan, taps, dstep, m_first, m_count, y,
+                             y_stride, stream);
+  if (pcm16)
+    return launch_bank_decim((const short *) x, origin, count, decim, nchan, taps, dstep, m_first, m_count, y,
+                             y_stride, stream);
+  return launch_bank_decim((const float *) x, origin, count, decim, nchan, taps, dstep, m_first, m_count, y, y_stride,
+                           stream);
 }
 
 extern "C" int glb_launch_zoom_split(const void *spec, int nz, long long nframes, float *rows, void *stream) {

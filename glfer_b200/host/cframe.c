@@ -11,6 +11,9 @@
  * A run walks the frames in chunks on the slots in turn: a slot's stream is synchronised before the slot is reused, so
  * a chunk's kernels and downloads overlap the next chunk's upload, and device memory is bounded by the chunk, not by
  * the recording.
+ *
+ * A zoom bank's call has C channels: the stage lays the channels' samples at a fixed stride, and one frame stage
+ * launch covers every channel (glb_cframe_stage), so the launches per chunk do not grow with C.
  */
 #include <math.h>
 #include <stdlib.h>
@@ -259,9 +262,11 @@ int glb_cframe_run(glb_cframe *f, const glb_cframe_call *c)
   if ((c->lo < 0 ? 0 : c->lo) < c->origin || c->hi > c->origin + c->count)
     return glb_host_fail(GLFER_EINVAL, c->short_span);
   const int n = f->n;
+  const int nchan = c->nchan > 1 ? c->nchan : 1;
   glb_display_run dr;
   if (c->display)
-    TRY(glb_display_begin(&f->disp, &dr, c->dc, c->agc_state, c->nframes, c->range_out != NULL, f->slot[0]->stream));
+    TRY(glb_display_begin(&f->disp, &dr, c->dc, c->agc_state, c->nframes, nchan, c->range_out != NULL,
+                          f->slot[0]->stream));
   int rc = 0, ci = 0;
   long long done = 0;
   while (done < c->nframes && rc == 0) {
@@ -269,22 +274,30 @@ int glb_cframe_run(glb_cframe *f, const glb_cframe_call *c)
     glb_cslot *s = f->slot[i];
     const long long c0 = c->first_frame + done;
     const long long cn = (c->nframes - done < c->chunk_frames) ? c->nframes - done : c->chunk_frames;
+    /* channels at a stride of crows frames, so that one launch of nl frames covers them all: frame c0 + c crows + j is
+       channel c's frame c0 + j, and the crows - cn frames between two channels are computed and never fetched */
+    const long long crows = nchan > 1 ? cn + (n - f->hop + f->hop - 1) / f->hop : cn;
+    const long long nl = (nchan - 1) * crows + cn;
     const float *z = NULL;
     long long z_origin = 0, z_count = 0;
     rc = glb_host_shim(glb_stream_sync(s->stream));
-    if (rc == 0 && c->display) rc = glb_display_reserve(&s->disp, cn, n, c->rgb != NULL);
-    if (rc == 0) rc = c->stage(c->plan, c, i, prev, c0, cn, &z, &z_origin, &z_count);
-    if (rc == 0) rc = cframe_launch(f, s, c, &dr, z, z_origin, z_count, c0, cn);
+    if (rc == 0 && c->display) rc = glb_display_reserve(&s->disp, nl, n, c->rgb != NULL);
+    if (rc == 0) rc = c->stage(c->plan, c, i, prev, c0, cn, crows * f->hop, &z, &z_origin, &z_count);
+    if (rc == 0) rc = cframe_launch(f, s, c, &dr, z, z_origin, z_count, c0, nl);
     if (rc == 0 && c->display && !c->fuse)
       rc = glb_display_map(&f->disp, &dr, &s->disp, prev >= 0 ? &f->slot[prev]->disp : NULL, s->d_rows, s->d_rows, n,
-                           c0, cn, done, f->overlap, c->rgb != NULL, s->stream);
-    if (rc == 0 && c->display) rc = glb_display_fetch(&s->disp, cn, n, done, c->levels, c->rgb, s->stream);
-    if (rc == 0 && c->rows)
-      rc = glb_host_shim(glb_memcpy_d2h(c->rows + (size_t) done * n, s->d_rows, sizeof(float) * (size_t) (cn * n),
-                                        s->stream));
-    if (rc == 0 && c->ftest)
-      rc = glb_host_shim(glb_memcpy_d2h(c->ftest + (size_t) done * n, s->d_ftest, sizeof(float) * (size_t) (cn * n),
-                                        s->stream));
+                           c0, cn, crows, done, f->overlap, c->rgb != NULL, s->stream);
+    if (rc == 0 && c->display)
+      rc = glb_display_fetch(&dr, &s->disp, cn, crows, n, done, c->levels, c->rgb, s->stream);
+    for (int ch = 0; ch < nchan && rc == 0; ch++) {
+      const size_t to = (size_t) (ch * c->nframes + done) * n, from = (size_t) (ch * crows) * n;
+      if (c->rows)
+        rc = glb_host_shim(glb_memcpy_d2h(c->rows + to, s->d_rows + from, sizeof(float) * (size_t) (cn * n),
+                                          s->stream));
+      if (rc == 0 && c->ftest)
+        rc = glb_host_shim(glb_memcpy_d2h(c->ftest + to, s->d_ftest + from, sizeof(float) * (size_t) (cn * n),
+                                          s->stream));
+    }
     done += cn;
     ci++;
   }

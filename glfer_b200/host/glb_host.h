@@ -54,23 +54,27 @@ typedef struct {                /* one run */
   float thr;                    /* thr_level / 100 */
   float fixed[2];               /* fixed display range (display_max, display_min), dB in the log scales */
   float *st_range;              /* staging of the caller's display_range, or NULL */
+  int nchan;                    /* channels: the caller's arrays are [nchan][nframes]..., one AGC chain each */
+  long long nframes;
 } glb_display_run;
 int glb_make_level_tables(void **tables);
 void glb_display_free(glb_display *d);
 void glb_display_slot_free(glb_display_slot *s);
-/* device state for a run (synchronises `stream`); want_range: the caller asked for display_range */
+/* device state for a run (synchronises `stream`); nchan: channels of a zoom bank (1..GLB_ZOOM_MAX_CHANNELS, 1
+ * elsewhere), agc_state [nchan][2]; want_range: the caller asked for display_range */
 int glb_display_begin(glb_display *d, glb_display_run *r, const glfer_display_config *dc, const float *agc_state,
-                      long long nframes, int want_range, void *stream);
+                      long long nframes, int nchan, int want_range, void *stream);
 /* the slot's level (and RGB) buffers for nframes rows of nbins */
 int glb_display_reserve(glb_display_slot *s, long long nframes, int nbins, int rgb);
 /* levels (and RGB) of the cn device rows d_shown (floor statistics of d_psd when autoscaling) of frames [c0, c0 + cn),
- * frames [done, done + cn) of the run; prev: the slot of the run's previous chunk, or NULL for the first */
+ * frames [done, done + cn) of the run; channel c's rows start at row c crows (crows >= cn; the slot is reserved for
+ * (nchan - 1) crows + cn rows); prev: the slot of the run's previous chunk, or NULL for the first */
 int glb_display_map(const glb_display *d, const glb_display_run *r, glb_display_slot *s, const glb_display_slot *prev,
-                    const float *d_psd, const float *d_shown, int nbins, long long c0, long long cn, long long done,
-                    float overlap, int rgb, void *stream);
-/* download the slot's levels / RGB (either may be NULL) to rows [done, done + cn) */
-int glb_display_fetch(const glb_display_slot *s, long long cn, int nbins, long long done, unsigned char *levels,
-                      unsigned char *rgb, void *stream);
+                    const float *d_psd, const float *d_shown, int nbins, long long c0, long long cn, long long crows,
+                    long long done, float overlap, int rgb, void *stream);
+/* download the slot's levels / RGB (either may be NULL) of each channel to its rows [done, done + cn) */
+int glb_display_fetch(const glb_display_run *r, const glb_display_slot *s, long long cn, long long crows, int nbins,
+                      long long done, unsigned char *levels, unsigned char *rgb, void *stream);
 /* after the run's streams are synchronised: the carried AGC state and the staged display range */
 int glb_display_end(const glb_display *d, const glb_display_run *r, long long nframes, float *agc_state,
                     float *range_out);
@@ -116,9 +120,12 @@ void glb_cframe_destroy(glb_cframe *f);
 int glb_cframe_tapers(const glb_cframe *f, double *tapers, double *lambda);
 typedef struct glb_cframe_call glb_cframe_call;
 /* the plan's stage of a chunk: the complex samples that frames [c0, c0 + cn) read, on the device of slot i (prev: the
- * slot of the run's previous chunk, or -1), on that slot's stream; *z holds samples [*z_origin, *z_origin + *z_count) */
+ * slot of the run's previous chunk, or -1), on that slot's stream; *z holds samples [*z_origin, *z_origin + *z_count).
+ * A call with nchan > 1 channels lays channel c's samples at z + c z_stride (complex samples, z_stride = crows hop),
+ * so that frame c0 + c crows + j of one launch is frame c0 + j of channel c; the stage zeroes what a channel c >= 1
+ * frame reads before its channel's samples (stream indices < 0), and *z_count covers the last channel. */
 typedef int (*glb_cframe_stage)(void *plan, const glb_cframe_call *c, int i, int prev, long long c0, long long cn,
-                                const float **z, long long *z_origin, long long *z_count);
+                                long long z_stride, const float **z, long long *z_origin, long long *z_count);
 struct glb_cframe_call {        /* one run entry's call */
   const void *src;              /* the caller's samples [origin, origin + count), float or int16 (pcm16) */
   int pcm16;
@@ -130,6 +137,7 @@ struct glb_cframe_call {        /* one run entry's call */
   float *agc_state, *range_out;
   unsigned char *levels, *rgb;
   /* from the plan */
+  int nchan;                    /* channels (zoom bank): the caller's outputs are [nchan][nframes]...; 0 or 1: one */
   void *plan;
   glb_cframe_stage stage;
   long long chunk_frames;

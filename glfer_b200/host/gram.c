@@ -856,7 +856,7 @@ static int run_display_impl(glfer_gram_plan *p, const float *samples, const shor
   if (lo < origin || hi > origin + count)
     return fail(GLFER_EINVAL, "samples do not cover the requested frames (see glfer_gram_required_span)");
   glb_display_run dr;
-  TRY(glb_display_begin(&p->disp, &dr, dc, agc_state, nframes, range_out != NULL, p->slot[0].stream));
+  TRY(glb_display_begin(&p->disp, &dr, dc, agc_state, nframes, 1, range_out != NULL, p->slot[0].stream));
   const long long cf = chunk_frames(p);
   const int avg_on = p->cfg.avg_mode != GLFER_NO_AVG;
   /* fixed display range, rows shown = the estimator's own rows: the spectrogram kernel writes the 8-bit
@@ -886,10 +886,10 @@ static int run_display_impl(glfer_gram_plan *p, const float *samples, const shor
       const float *d_psd = (p->cfg.mode == GLFER_MODE_LMP) ? s->d_avg : s->d_psd + (size_t) s->out_halo * p->bins;
       const float *d_shown = avg_on ? s->d_avg : d_psd;               /* g_main.c:1192-1201 */
       rc = glb_display_map(&p->disp, &dr, &s->disp, ci > 0 ? &p->slot[(ci - 1) % NSLOT].disp : NULL, d_psd, d_shown,
-                           p->bins, c0, cn, done, p->cfg.overlap, rgb != NULL, s->stream);
+                           p->bins, c0, cn, cn, done, p->cfg.overlap, rgb != NULL, s->stream);
       if (rc) break;
     }
-    rc = glb_display_fetch(&s->disp, cn, p->bins, done, levels, rgb, s->stream);
+    rc = glb_display_fetch(&dr, &s->disp, cn, cn, p->bins, done, levels, rgb, s->stream);
     done += cn;
     ci++;
   }

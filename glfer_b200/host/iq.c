@@ -101,8 +101,8 @@ int glfer_iq_tapers(const glfer_iq_plan *p, double *tapers, double *lambda)
 }
 
 /* the complex samples of frames [c0, c0 + cn) into slot i's d_in (glb_cframe_stage) */
-static int iq_stage(void *plan, const glb_cframe_call *c, int i, int prev, long long c0, long long cn, const float **z,
-                    long long *z_origin, long long *z_count)
+static int iq_stage(void *plan, const glb_cframe_call *c, int i, int prev, long long c0, long long cn,
+                    long long z_stride, const float **z, long long *z_origin, long long *z_count)
 {
   glfer_iq_plan *p = plan;
   islot *s = &p->slot[i];

@@ -20,6 +20,10 @@
  * Multitaper plans (glfer_zoom_plan_create_mtm / _create_iq_mtm) replace the window by K' DPSS tapers; the frame stage
  * then runs one spectrum per taper into the same scratch plane.  glfer_zoom_run[_iq]_mtm_ftest add the hn spectrum and
  * the mu and den planes to that scratch and bring back F rows beside or instead of the rows.
+ *
+ * Banks (glfer_zoom_plan_create_bank[_mtm]) hold C centres of one config.  Each chunk's input is uploaded once and the
+ * bank decimator (glb_launch_zoom_bank_decim) writes every channel's decimated samples at the channel stride the frame
+ * stage asks for; one frame stage launch then covers all channels.  A single-centre plan keeps zoom_decim_kernel.
  */
 #include <math.h>
 #include <stdlib.h>
@@ -34,13 +38,15 @@ typedef struct {
   float *d_y;                 /* y[m], m in [y_base, y_end), as (re, im) pairs */
   size_t y_cap;               /* complex samples */
   long long y_base, y_end;
+  long long y_stride;         /* complex samples between two channels' y[y_base] (banks) */
 } zslot;
 
 struct glfer_zoom_plan {
   glfer_zoom_config cfg;
   int K;
-  unsigned step;
-  float *d_taps;              /* [33 D] (re, im) pairs: g[j] = h[K - j] e^{+2 pi i phi(K - j)}, zero past 2K */
+  int nchan;                  /* channels (centres): 1 for the single-centre constructors */
+  unsigned step[GLB_ZOOM_MAX_CHANNELS];
+  float *d_taps;              /* [nchan][33 D] (re, im) pairs: g[j] = h[K - j] e^{+2 pi i phi(K - j)}, zero past 2K */
   int iq;                     /* 1: complex (I, Q) input (glfer_zoom_plan_create_iq), signed centre */
   glb_cframe fs;
   zslot slot[GLB_CSLOTS];
@@ -97,12 +103,15 @@ void glfer_zoom_config_default(glfer_zoom_config *c)
 
 int glfer_zoom_hop(const glfer_zoom_plan *p) { return p->fs.hop; }
 int glfer_zoom_bins(const glfer_zoom_plan *p) { return p->cfg.n; }
-double glfer_zoom_center_hz(const glfer_zoom_plan *p)
+int glfer_zoom_channels(const glfer_zoom_plan *p) { return p->nchan; }
+double glfer_zoom_channel_center_hz(const glfer_zoom_plan *p, int c)
 {
+  if (c < 0 || c >= p->nchan) return NAN;
   /* an I/Q plan's step is a signed 32-bit fraction of a turn: centres below the dial are negative */
-  const double s = p->iq ? (double) (int) p->step : (double) p->step;
+  const double s = p->iq ? (double) (int) p->step[c] : (double) p->step[c];
   return s * p->cfg.sample_rate / 4294967296.0;
 }
+double glfer_zoom_center_hz(const glfer_zoom_plan *p) { return glfer_zoom_channel_center_hz(p, 0); }
 
 long long glfer_zoom_num_frames(const glfer_zoom_plan *p, long long nsamples)
 {
@@ -134,49 +143,59 @@ void glfer_zoom_plan_destroy(glfer_zoom_plan *p)
   free(p);
 }
 
-/* the decimator's complex taps on the device */
+/* the decimator's complex taps of every channel on the device */
 static int upload_taps(glfer_zoom_plan *p)
 {
   const int D = p->cfg.decim, K = p->K;
+  const size_t per = (size_t) 66 * D, bytes = sizeof(float) * per * p->nchan;
   float *h = malloc(sizeof(float) * (2 * K + 1));
-  float *g = calloc((size_t) 66 * D, sizeof(float));
+  float *g = calloc(per * p->nchan, sizeof(float));
   int rc = 0;
   if (!h || !g) rc = glb_host_fail(GLFER_ENOMEM, "out of memory");
   if (rc == 0) rc = glfer_zoom_taps(D, h);
-  if (rc == 0) {
+  for (int c = 0; c < p->nchan && rc == 0; c++) {
     /* g[j] = h[K - j] e^{+2 pi i phi(K - j)}: h is symmetric, so h[K - j] is taps[j] */
+    float *gc = g + per * c;
     for (int j = 0; j <= 2 * K; j++) {
-      const unsigned ph = (unsigned) ((long long) (K - j) * (long long) p->step);
+      const unsigned ph = (unsigned) ((long long) (K - j) * (long long) p->step[c]);
       const double a = 2.0 * M_PI * (double) ph / 4294967296.0;
-      g[2 * j] = (float) ((double) h[j] * cos(a));
-      g[2 * j + 1] = (float) ((double) h[j] * sin(a));
+      gc[2 * j] = (float) ((double) h[j] * cos(a));
+      gc[2 * j + 1] = (float) ((double) h[j] * sin(a));
     }
-    rc = glb_host_shim(glb_malloc((void **) &p->d_taps, sizeof(float) * 66 * (size_t) D));
-    if (rc == 0) rc = glb_host_shim(glb_memcpy_h2d(p->d_taps, g, sizeof(float) * 66 * (size_t) D, NULL));
+  }
+  if (rc == 0) {
+    rc = glb_host_shim(glb_malloc((void **) &p->d_taps, bytes));
+    if (rc == 0) rc = glb_host_shim(glb_memcpy_h2d(p->d_taps, g, bytes, NULL));
   }
   free(h); free(g);
   return rc;
 }
 
-static int zoom_plan_create(const glfer_zoom_config *cfg, int iq, int mtm, float mtm_w, int mtm_kmax,
-                            glfer_zoom_plan **out)
+/* centers[c], c = 0..nchan-1: the channels' centres (cfg->center_hz is not read); validated before any device call */
+static int zoom_plan_create(const glfer_zoom_config *cfg, const double *centers, int nchan, int iq, int mtm,
+                            float mtm_w, int mtm_kmax, glfer_zoom_plan **out)
 {
   glb_host_clear_error();
-  if (!cfg || !out) return glb_host_fail(GLFER_EINVAL, "null argument");
+  if (!cfg || !out || !centers) return glb_host_fail(GLFER_EINVAL, "null argument");
   *out = NULL;
+  if (nchan < 1 || nchan > GLB_ZOOM_MAX_CHANNELS) return glb_host_fail(GLFER_EINVAL, "zoom channels must be in 1..32");
   if (cfg->decim < 2 || cfg->decim > 1024) return glb_host_fail(GLFER_EINVAL, "zoom decimation must be in 2..1024");
   if (!(cfg->sample_rate > 0.0) || !isfinite(cfg->sample_rate)) return glb_host_fail(GLFER_EINVAL, "sample rate must be positive");
-  if (!iq && !(cfg->center_hz >= 0.0 && cfg->center_hz <= 0.5 * cfg->sample_rate))
-    return glb_host_fail(GLFER_EINVAL, "centre frequency must be in [0, sample_rate / 2]");
-  if (iq && !(cfg->center_hz >= -0.5 * cfg->sample_rate && cfg->center_hz <= 0.5 * cfg->sample_rate))
-    return glb_host_fail(GLFER_EINVAL, "I/Q centre frequency must be in [-sample_rate / 2, sample_rate / 2]");
+  for (int c = 0; c < nchan; c++) {
+    if (!iq && !(centers[c] >= 0.0 && centers[c] <= 0.5 * cfg->sample_rate))
+      return glb_host_fail(GLFER_EINVAL, "centre frequency must be in [0, sample_rate / 2]");
+    if (iq && !(centers[c] >= -0.5 * cfg->sample_rate && centers[c] <= 0.5 * cfg->sample_rate))
+      return glb_host_fail(GLFER_EINVAL, "I/Q centre frequency must be in [-sample_rate / 2, sample_rate / 2]");
+  }
   glfer_zoom_plan *p = calloc(1, sizeof *p);
   if (!p) return glb_host_fail(GLFER_ENOMEM, "out of memory");
   p->cfg = *cfg;
   p->K = 16 * cfg->decim;
   p->iq = iq;
+  p->nchan = nchan;
   /* modulo 2^32: a negative I/Q centre is a step above 2^31 */
-  p->step = (unsigned) (unsigned long long) llround(cfg->center_hz / cfg->sample_rate * 4294967296.0);
+  for (int c = 0; c < nchan; c++)
+    p->step[c] = (unsigned) (unsigned long long) llround(centers[c] / cfg->sample_rate * 4294967296.0);
   glb_cslot *const slot[GLB_CSLOTS] = { &p->slot[0].cs, &p->slot[1].cs, &p->slot[2].cs };
   int rc = glb_cframe_create(&p->fs, slot, cfg->n, cfg->window_type, cfg->overlap, cfg->device, mtm, mtm_w, mtm_kmax,
                              "zoom FFT size must be a power of two in 32..16384");
@@ -200,22 +219,34 @@ static int zoom_plan_create(const glfer_zoom_config *cfg, int iq, int mtm, float
 
 int glfer_zoom_plan_create(const glfer_zoom_config *cfg, glfer_zoom_plan **out)
 {
-  return zoom_plan_create(cfg, 0, 0, 0.0f, 0, out);
+  return zoom_plan_create(cfg, cfg ? &cfg->center_hz : NULL, 1, 0, 0, 0.0f, 0, out);
 }
 
 int glfer_zoom_plan_create_iq(const glfer_zoom_config *cfg, glfer_zoom_plan **out)
 {
-  return zoom_plan_create(cfg, 1, 0, 0.0f, 0, out);
+  return zoom_plan_create(cfg, cfg ? &cfg->center_hz : NULL, 1, 1, 0, 0.0f, 0, out);
 }
 
 int glfer_zoom_plan_create_mtm(const glfer_zoom_config *cfg, float mtm_w, int mtm_kmax, glfer_zoom_plan **out)
 {
-  return zoom_plan_create(cfg, 0, 1, mtm_w, mtm_kmax, out);
+  return zoom_plan_create(cfg, cfg ? &cfg->center_hz : NULL, 1, 0, 1, mtm_w, mtm_kmax, out);
 }
 
 int glfer_zoom_plan_create_iq_mtm(const glfer_zoom_config *cfg, float mtm_w, int mtm_kmax, glfer_zoom_plan **out)
 {
-  return zoom_plan_create(cfg, 1, 1, mtm_w, mtm_kmax, out);
+  return zoom_plan_create(cfg, cfg ? &cfg->center_hz : NULL, 1, 1, 1, mtm_w, mtm_kmax, out);
+}
+
+int glfer_zoom_plan_create_bank(const glfer_zoom_config *cfg, const double *centers_hz, int nchan, int iq,
+                                glfer_zoom_plan **out)
+{
+  return zoom_plan_create(cfg, centers_hz, nchan, iq != 0, 0, 0.0f, 0, out);
+}
+
+int glfer_zoom_plan_create_bank_mtm(const glfer_zoom_config *cfg, const double *centers_hz, int nchan, int iq,
+                                    float mtm_w, int mtm_kmax, glfer_zoom_plan **out)
+{
+  return zoom_plan_create(cfg, centers_hz, nchan, iq != 0, 1, mtm_w, mtm_kmax, out);
 }
 
 int glfer_zoom_tapers(const glfer_zoom_plan *p, double *tapers, double *lambda)
@@ -224,9 +255,9 @@ int glfer_zoom_tapers(const glfer_zoom_plan *p, double *tapers, double *lambda)
 }
 
 /* the decimated samples of frames [c0, c0 + cn) into slot i's d_y, those its first frame shares with the previous
- * chunk (slot prev) copied device to device (glb_cframe_stage) */
+ * chunk (slot prev) copied device to device (glb_cframe_stage); a bank's channel c at d_y + c z_stride */
 static int zoom_stage(void *plan, const glb_cframe_call *c, int i, int prev, long long c0, long long cn,
-                      const float **z, long long *z_origin, long long *z_count)
+                      long long z_stride, const float **z, long long *z_origin, long long *z_count)
 {
   glfer_zoom_plan *p = plan;
   zslot *s = &p->slot[i];
@@ -241,7 +272,9 @@ static int zoom_stage(void *plan, const glb_cframe_call *c, int i, int prev, lon
     base = m_lo > 0 ? m_lo : 0;
     from = base;
   }
-  TRY(glb_ensure((void **) &s->d_y, &s->y_cap, (size_t) (m_hi - base), 2 * sizeof(float)));
+  const int C = p->nchan;
+  const long long ys = C > 1 ? z_stride : 0;
+  TRY(glb_ensure((void **) &s->d_y, &s->y_cap, (size_t) ((C - 1) * ys + m_hi - base), 2 * sizeof(float)));
   long long x_lo = from * D - p->K;
   const long long x_hi = (m_hi - 1) * D + p->K + 1;
   if (x_lo < 0) x_lo = 0;
@@ -252,23 +285,34 @@ static int zoom_stage(void *plan, const glb_cframe_call *c, int i, int prev, lon
   if (from > base) {
     /* the history this chunk's first frame shares with the previous chunk */
     TRY(glb_stream_wait_event(s->cs.stream, ps->ev_dec));
-    TRY(glb_memcpy_d2d(s->d_y, ps->d_y + 2 * (base - ps->y_base), (size_t) (from - base) * 2 * sizeof(float),
-                       s->cs.stream));
+    for (int ch = 0; ch < C; ch++)
+      TRY(glb_memcpy_d2d(s->d_y + 2 * ch * ys, ps->d_y + 2 * (ch * ps->y_stride + base - ps->y_base),
+                         (size_t) (from - base) * 2 * sizeof(float), s->cs.stream));
   }
-  if (p->iq)
+  /* a channel c >= 1 frame that starts before y[base] reads the samples just below channel c's: zeros, as y[m < 0] */
+  for (int ch = 1; ch < C && m_lo < base; ch++)
+    TRY(glb_memset(s->d_y + 2 * (ch * ys - (base - m_lo)), 0, (size_t) (base - m_lo) * 2 * sizeof(float),
+                   s->cs.stream));
+  if (C > 1) {
+    unsigned dstep[GLB_ZOOM_MAX_CHANNELS];
+    for (int ch = 0; ch < C; ch++) dstep[ch] = (unsigned) ((unsigned long long) D * p->step[ch]);
+    TRY(glb_launch_zoom_bank_decim(s->d_in, c->pcm16, p->iq, x_lo, x_hi - x_lo, (int) D, C, p->d_taps, dstep, from,
+                                   m_hi - from, s->d_y + 2 * (from - base), ys, s->cs.stream));
+  } else if (p->iq)
     TRY(glb_launch_zoom_decim_iq(s->d_in, c->pcm16, x_lo, x_hi - x_lo, (int) D, p->d_taps,
-                                 (unsigned) ((unsigned long long) D * p->step), from, m_hi - from,
+                                 (unsigned) ((unsigned long long) D * p->step[0]), from, m_hi - from,
                                  s->d_y + 2 * (from - base), s->cs.stream));
   else
     TRY(glb_launch_zoom_decim(s->d_in, c->pcm16, x_lo, x_hi - x_lo, (int) D, p->d_taps,
-                              (unsigned) ((unsigned long long) D * p->step), from, m_hi - from,
+                              (unsigned) ((unsigned long long) D * p->step[0]), from, m_hi - from,
                               s->d_y + 2 * (from - base), s->cs.stream));
   TRY(glb_event_record(s->ev_dec, s->cs.stream));
   s->y_base = base;
   s->y_end = m_hi;
+  s->y_stride = ys;
   *z = s->d_y;
   *z_origin = base;
-  *z_count = m_hi - base;
+  *z_count = (C - 1) * ys + m_hi - base;
   return 0;
 }
 
@@ -286,6 +330,7 @@ static int zoom_run(glfer_zoom_plan *p, int iq, glb_cframe_call *c)
                        : "an I/Q zoom plan runs through glfer_zoom_run_iq / glfer_zoom_run_iq_pcm16";
   c->plan = p;
   c->stage = zoom_stage;
+  c->nchan = p->nchan;
   /* ~32 MiB of new float input per chunk, as the spectrogram's pipeline; at least one frame */
   c->chunk_frames = (32LL << 20) / ((long long) p->fs.hop * p->cfg.decim * (p->iq ? 8 : 4));
   if (c->chunk_frames < 1) c->chunk_frames = 1;

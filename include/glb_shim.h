@@ -211,6 +211,16 @@ int glb_launch_zoom_split(const void *spec, int nz, long long nframes, float *ro
  * so with Q = 0 every output is bit-identical to glb_launch_zoom_decim's of I. */
 int glb_launch_zoom_decim_iq(const void *x, int pcm16, long long origin, long long count, int decim, const void *taps,
                              unsigned dstep, long long m_first, long long m_count, void *y, void *stream);
+/* Bank decimator: glb_launch_zoom_decim (iq = 0) or glb_launch_zoom_decim_iq (iq = 1) for nchan channels
+ * (1..GLB_ZOOM_MAX_CHANNELS) of the same x in one launch: taps [nchan][33 decim] (re, im) pairs on the device,
+ * dstep [nchan] on the host, channel c's outputs at y + c y_stride (complex samples; y_stride >= m_count when
+ * nchan > 1).  Each input sample is loaded and converted once per tile for a group of up to 8 channels.  Every output
+ * of channel c is bit-identical to the single-channel decimator's with taps + c 33 decim and dstep[c]: the same lane
+ * partials over the same phases, taps in the same order, summed in the same order. */
+#define GLB_ZOOM_MAX_CHANNELS 32
+int glb_launch_zoom_bank_decim(const void *x, int pcm16, int iq, long long origin, long long count, int decim,
+                               int nchan, const void *taps, const unsigned *dstep, long long m_first, long long m_count,
+                               void *y, long long y_stride, void *stream);
 
 /* Rows of complex frames (I/Q spectrogram, zoom frame stage) of an interleaved (I, Q) stream z:
  *     rows[f - first_frame][j] = |sum_i w[i] z[f hop - (n - hop) + i] e^{-2 pi i (j - n/2) i / n}|^2 / n

@@ -323,6 +323,27 @@ int glfer_zoom_plan_create_iq_mtm(const glfer_zoom_config *cfg, float mtm_w, int
 int glfer_iq_tapers(const glfer_iq_plan *plan, double *tapers, double *lambda);
 int glfer_zoom_tapers(const glfer_zoom_plan *plan, double *tapers, double *lambda);
 
+/* ---- zoom channel banks: several centres of one recording ----
+ * A bank is a zoom plan with C channels: C centre frequencies that share one config (n, decim, window, overlap, sample
+ * rate, device), real (iq = 0) or I/Q (iq = 1) input, periodogram or multitaper (mtm_w, mtm_kmax as
+ * glfer_zoom_plan_create_mtm).  cfg->center_hz is ignored; centers_hz[c], c = 0..nchan-1, is validated as the
+ * single-centre constructors validate center_hz ([0, sample_rate / 2] real, [-sample_rate / 2, sample_rate / 2] I/Q);
+ * duplicates are allowed; nchan in 1..32.  All of this is checked before any device call (GLFER_EINVAL).
+ * Each run uploads the input once and decimates it for every channel in one kernel.  Every zoom run, run_display,
+ * mtm_ftest and query entry point serves banks with its own signature; per-channel outputs are stacked on a leading
+ * axis: rows, F rows and levels [C][nframes][n], RGB [C][nframes][n][3], display_range [C][nframes][2], agc_state
+ * [C][2] (one AGC recurrence per channel).  The required span, hop, bins and frame count do not depend on the centre.
+ * A plan from the single-centre constructors has C = 1, and with C = 1 every layout is the one above.
+ * Channel c of a bank is bit-identical to a single-centre zoom plan at centers_hz[c] with the same config: rows, F
+ * rows, levels, RGB, display range and AGC state, for every input format and estimator. */
+int glfer_zoom_plan_create_bank(const glfer_zoom_config *cfg, const double *centers_hz, int nchan, int iq,
+                                glfer_zoom_plan **plan);
+int glfer_zoom_plan_create_bank_mtm(const glfer_zoom_config *cfg, const double *centers_hz, int nchan, int iq,
+                                    float mtm_w, int mtm_kmax, glfer_zoom_plan **plan);
+int glfer_zoom_channels(const glfer_zoom_plan *plan);                      /* C; 1 for the single-centre constructors */
+/* as glfer_zoom_center_hz, of channel c (NaN outside 0..C-1); glfer_zoom_center_hz is channel 0's */
+double glfer_zoom_channel_center_hz(const glfer_zoom_plan *plan, int c);
+
 /* Thomson's harmonic F-test of multitaper I/Q and zoom plans (real and I/Q zoom).  Frame f is the plan's complex frame
  * z_f above (I/Q samples, or the decimated y of a zoom), v_k and lambda_k the plan's tapers (glfer_iq_tapers /
  * glfer_zoom_tapers), K' = mtm_kmax + 1, and
