@@ -69,6 +69,10 @@ class IqConfig(C.Structure):         # include/glfer_b200.h glfer_iq_config
     _fields_ = [("n", C.c_int), ("window_type", C.c_int), ("overlap", C.c_float), ("device", C.c_int)]
 
 
+class LinesConfig(C.Structure):      # include/glfer_b200.h glfer_lines_config
+    _fields_ = [("pfa", C.c_double), ("max_lines", C.c_int), ("bin_lo", C.c_int), ("bin_hi", C.c_int)]
+
+
 class Wav(C.Structure):
     _fields_ = [("sample_rate", C.c_int), ("bits", C.c_int), ("channels", C.c_int), ("nsamples", C.c_longlong),
                 ("data", C.c_void_p)]
@@ -173,6 +177,10 @@ def lib() -> C.CDLL:
         for name in ("glfer_iq_run_mtm_ftest", "glfer_iq_run_mtm_ftest_pcm16", "glfer_zoom_run_mtm_ftest",
                      "glfer_zoom_run_mtm_ftest_pcm16", "glfer_zoom_run_iq_mtm_ftest", "glfer_zoom_run_iq_mtm_ftest_pcm16"):
             getattr(l, name).argtypes = zoom_args + [C.c_void_p]
+        for name in ("glfer_iq_run_mtm_lines", "glfer_iq_run_mtm_lines_pcm16", "glfer_zoom_run_mtm_lines",
+                     "glfer_zoom_run_mtm_lines_pcm16", "glfer_zoom_run_iq_mtm_lines", "glfer_zoom_run_iq_mtm_lines_pcm16"):
+            getattr(l, name).argtypes = zoom_args[:-1] + [C.POINTER(LinesConfig)] + [C.c_void_p] * 4
+        l.glfer_ftest_threshold.argtypes = [C.c_int, C.c_double, C.POINTER(C.c_float)]
         for name in ("glfer_iq_run_display", "glfer_iq_run_display_pcm16", "glfer_zoom_run_display",
                      "glfer_zoom_run_display_pcm16", "glfer_zoom_run_display_iq", "glfer_zoom_run_display_iq_pcm16"):
             getattr(l, name).argtypes = disp_args
@@ -493,7 +501,7 @@ class ZoomPlan:
     multitaper=True: rows of K' = mtm_kmax + 1 DPSS tapers of NW = mtm_w (glfer_zoom_plan_create[_iq]_mtm; window_type
     is ignored).
     center_hz a sequence: a channel bank (glfer_zoom_plan_create_bank[_mtm]), one channel per centre; run,
-    run_mtm_ftest and run_display then return arrays with a leading channel axis, (C, nframes, n), and run_display
+    run_mtm_ftest, run_mtm_lines and run_display then return arrays with a leading channel axis, (C, nframes, ...), and run_display
     takes and returns agc_state of shape (C, 2)."""
 
     def __init__(self, n=4096, decim=256, window_type=HANNING, overlap=0.0, center_hz=800.0, sample_rate=48000.0,
@@ -598,6 +606,25 @@ class ZoomPlan:
         return _run_ftest(fn, self._h, ptr, origin, count, first_frame, nframes, self.bins, want_psd, want_ftest,
                           self._lead)
 
+    def run_mtm_lines(self, samples: np.ndarray, pfa: float = 1e-3, max_lines: int = 16, bin_range=None,
+                      origin: int = 0, first_frame: int = 0, nframes: int | None = None, want_ftest: bool = True,
+                      want_psd: bool = True):
+        """glfer_zoom_run[_iq]_mtm_lines[_pcm16]: the harmonic lines of each frame, selected on the device from the F rows
+        of run_mtm_ftest at the F(2, 2K' - 2) threshold of pfa.  Keywords and outputs of IqPlan.run_mtm_lines, with the
+        bank's leading channel axis.  Input formats of run."""
+        if self.iq:
+            ptr, count, pcm = _iq_samples(samples)
+            fn = lib().glfer_zoom_run_iq_mtm_lines_pcm16 if pcm else lib().glfer_zoom_run_iq_mtm_lines
+        else:
+            pcm = samples.dtype == np.int16
+            assert samples.flags["C_CONTIGUOUS"] and (pcm or samples.dtype == np.float32)
+            ptr, count = samples.ctypes.data, len(samples)
+            fn = lib().glfer_zoom_run_mtm_lines_pcm16 if pcm else lib().glfer_zoom_run_mtm_lines
+        if nframes is None:
+            nframes = self.num_frames(origin + count) - first_frame
+        return _run_lines(fn, self._h, ptr, origin, count, first_frame, nframes, self.bins, pfa, max_lines, bin_range,
+                          want_ftest, want_psd, self._lead)
+
     def run_display(self, samples: np.ndarray, log_scale=True, autoscale=True, max_level_db=-20.0, min_level_db=-80.0,
                     thr_level=0.0, colortab: np.ndarray | None = None, origin: int = 0, first_frame: int = 0,
                     nframes: int | None = None, agc_state: np.ndarray | None = None, want_rgb: bool = False,
@@ -684,6 +711,20 @@ class IqPlan:
         fn = lib().glfer_iq_run_mtm_ftest_pcm16 if pcm else lib().glfer_iq_run_mtm_ftest
         return _run_ftest(fn, self._h, ptr, origin, count, first_frame, nframes, self.bins, want_psd, want_ftest)
 
+    def run_mtm_lines(self, iq: np.ndarray, pfa: float = 1e-3, max_lines: int = 16, bin_range=None, origin: int = 0,
+                      first_frame: int = 0, nframes: int | None = None, want_ftest: bool = True, want_psd: bool = True):
+        """glfer_iq_run_mtm_lines / _pcm16: the harmonic lines of each frame, selected on the device from the F rows of
+        run_mtm_ftest at the F(2, 2K' - 2) threshold of pfa (ftest_threshold), searched over row positions
+        bin_range = (lo, hi) (None: the whole row).  Returns dict(count [nframes] int32, bin [nframes][max_lines] int32,
+        ftest and psd [nframes][max_lines] float32, None when not wanted); unused slots hold bin -1 and 0.0.  Input
+        formats of run."""
+        ptr, count, pcm = _iq_samples(iq)
+        if nframes is None:
+            nframes = self.num_frames(origin + count) - first_frame
+        fn = lib().glfer_iq_run_mtm_lines_pcm16 if pcm else lib().glfer_iq_run_mtm_lines
+        return _run_lines(fn, self._h, ptr, origin, count, first_frame, nframes, self.bins, pfa, max_lines, bin_range,
+                          want_ftest, want_psd)
+
     def run_display(self, iq: np.ndarray, log_scale=True, autoscale=True, max_level_db=-20.0, min_level_db=-80.0,
                     thr_level=0.0, colortab: np.ndarray | None = None, origin: int = 0, first_frame: int = 0,
                     nframes: int | None = None, agc_state: np.ndarray | None = None, want_rgb: bool = False,
@@ -703,6 +744,27 @@ def _run_ftest(fn, h, ptr, origin, count, first_frame, nframes, bins, want_psd, 
     ft = np.empty(lead + (nframes, bins), np.float32) if want_ftest else None
     _check(fn(h, ptr, origin, count, first_frame, nframes, _ptr(psd), _ptr(ft)))
     return dict(psd=psd, ftest=ft)
+
+
+def _run_lines(fn, h, ptr, origin, count, first_frame, nframes, bins, pfa, max_lines, bin_range, want_ftest, want_psd,
+               lead=()):
+    lo, hi = (0, bins) if bin_range is None else bin_range
+    lc = LinesConfig(pfa, max_lines, lo, hi)
+    m = max(int(max_lines), 0)
+    cnt = np.empty(lead + (nframes,), np.int32)
+    b = np.empty(lead + (nframes, m), np.int32)
+    ft = np.empty(lead + (nframes, m), np.float32) if want_ftest else None
+    psd = np.empty(lead + (nframes, m), np.float32) if want_psd else None
+    _check(fn(h, ptr, origin, count, first_frame, nframes, C.byref(lc), cnt.ctypes.data, b.ctypes.data, _ptr(ft),
+              _ptr(psd)))
+    return dict(count=cnt, bin=b, ftest=ft, psd=psd)
+
+
+def ftest_threshold(ntapers: int, pfa: float) -> float:
+    """glfer_ftest_threshold: the F(2, 2K' - 2) threshold of a per-bin false-alarm probability pfa; needs no device"""
+    thr = C.c_float()
+    _check(lib().glfer_ftest_threshold(int(ntapers), float(pfa), C.byref(thr)))
+    return float(thr.value)
 
 
 def zoom_taps(decim: int) -> np.ndarray:

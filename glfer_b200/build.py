@@ -16,7 +16,8 @@ LIB_FFTW = os.path.join(HERE, "libglfer_b200_fftw.so")      # fft_params_t in th
 OBJ = os.path.join(HERE, "_build")
 
 # (source, tag, extra flags): gram_part.cu is compiled once per subset of FFT sizes, in parallel
-CU_UNITS = ([("csrc/gram_kernels.cu", "", []), ("csrc/gram_big.cu", "", []), ("csrc/zoom.cu", "", []), ("csrc/iq.cu", "", [])]
+CU_UNITS = ([("csrc/gram_kernels.cu", "", []), ("csrc/gram_big.cu", "", []), ("csrc/zoom.cu", "", []), ("csrc/iq.cu", "", []),
+             ("csrc/lines.cu", "", [])]
             + [("csrc/gram_part.cu", f".p{k}", [f"-DGLB_PART={k}"]) for k in range(4)])
 C_SOURCES = ["host/window.c", "host/dpss.c", "host/gram.c", "host/dropin.c", "host/wav.c", "host/levels.c",
              "host/zoom.c", "host/iq.c", "host/cframe.c", "host/display.c"]

@@ -3,7 +3,8 @@
  * Both plans turn a chunk of their input into complex samples on the device -- the I/Q plan uploads them, the zoom
  * mixes, filters and decimates them -- and from there do the same work: complex FFT frames of n samples through one
  * shim entry (glb_launch_iq_gram, or glb_launch_iq_gram_general for the zoom), rows and/or the harmonic F-test's F rows
- * back to the host, or 8-bit levels through the display chain of host/display.c.  This unit owns that work: the taper
+ * back to the host, 8-bit levels through the display chain of host/display.c, or the harmonic lines selected from the
+ * F rows on the device (glb_launch_ftest_lines).  This unit owns that work: the taper
  * table (the window, or K' DPSS tapers, each scaled as the real multitaper plan scales its own in host/gram.c) with the
  * F-test's table and the FFT tables, the GLB_CSLOTS streams with their rows, F rows and scratch, the argument checks of
  * the run entries and the chunk loop.  The plan supplies its per-chunk stage as a callback.
@@ -172,7 +173,8 @@ void glb_cframe_destroy(glb_cframe *f)
   for (int i = 0; i < GLB_CSLOTS; i++) {
     glb_cslot *s = f->slot[i];
     if (s->stream) glb_stream_sync(s->stream);
-    glb_free(s->d_rows); glb_free(s->d_ftest); glb_free(s->d_scratch);
+    glb_free(s->d_rows); glb_free(s->d_ftest); glb_free(s->d_scratch); glb_free(s->d_lines);
+    if (s->h_lines) glb_host_free(s->h_lines);
     glb_display_slot_free(&s->disp);
     glb_stream_destroy(s->stream);
   }
@@ -193,12 +195,14 @@ int glb_cframe_tapers(const glb_cframe *f, double *tapers, double *lambda)
 }
 
 /* frames [c0, cn) of the staged samples z ([z_origin, z_origin + z_count)) on slot s: with c->fuse the fixed-range
- * levels into s->disp.d_levels, otherwise rows into s->d_rows (when the run wants them) and F rows into s->d_ftest */
+ * levels into s->disp.d_levels, otherwise rows into s->d_rows (when the run wants them) and F rows into s->d_ftest
+ * (always for a lines run, whose rows are wanted only for line_psd) */
 static int cframe_launch(glb_cframe *f, glb_cslot *s, const glb_cframe_call *c, const glb_display_run *dr,
                          const float *z, long long z_origin, long long z_count, long long c0, long long cn)
 {
   const long long n = f->n;
-  const int rows_on = c->display ? !c->fuse : c->rows != NULL, ftest_on = c->ftest != NULL;
+  const int rows_on = c->display ? !c->fuse : c->lines ? c->line_psd != NULL : c->rows != NULL;
+  const int ftest_on = c->ftest != NULL || c->lines;
   if (rows_on) TRY(glb_ensure((void **) &s->d_rows, &s->rows_cap, (size_t) (cn * n), sizeof(float)));
   if (ftest_on) TRY(glb_ensure((void **) &s->d_ftest, &s->ftest_cap, (size_t) (cn * n), sizeof(float)));
   const long long sb = c->general ? glb_iq_gram_general_scratch_bytes((int) n, cn, c->fuse, ftest_on)
@@ -240,15 +244,80 @@ static int cframe_launch(glb_cframe *f, glb_cslot *s, const glb_cframe_call *c, 
   return 0;
 }
 
+/* bytes of one chunk's line arrays for nf output frames: count [nf] ints, then bin [nf][max_lines] ints, F and psd
+ * [nf][max_lines] floats when wanted; the device buffer and its pinned staging share the layout */
+static size_t lines_bytes(const glb_cframe_call *c, long long nf)
+{
+  const size_t slots = (size_t) nf * c->lc->max_lines;
+  return sizeof(int) * ((size_t) nf + slots) + sizeof(float) * slots * ((c->line_ftest != NULL) + (c->line_psd != NULL));
+}
+
+/* the lines of the chunk's F rows on slot s (nchan channels at a stride of crows rows), downloaded in one copy to the
+ * slot's pinned staging, which glb_cframe_run hands over once the slot's stream is synchronised */
+static int lines_chunk(glb_cframe *f, glb_cslot *s, const glb_cframe_call *c, float thr, int nchan, long long cn,
+                       long long crows, long long done)
+{
+  const long long nf = nchan * cn;
+  const size_t slots = (size_t) nf * c->lc->max_lines, bytes = lines_bytes(c, nf);
+  TRY(glb_ensure(&s->d_lines, &s->dlines_cap, bytes, 1));
+  if (bytes > s->hlines_cap) {
+    /* into the caller's arrays directly, each chunk's copy would block the host thread whenever they are pageable,
+       and with it the chunk pipeline (as the display range, host/display.c) */
+    if (s->h_lines) glb_host_free(s->h_lines);
+    s->h_lines = NULL; s->hlines_cap = 0;
+    const size_t cap = bytes + bytes / 2 + 4096;
+    TRY(glb_host_alloc(&s->h_lines, cap));
+    s->hlines_cap = cap;
+  }
+  int *d_count = s->d_lines, *d_bin = d_count + nf;
+  float *d_f = (float *) (d_bin + slots);
+  float *d_p = d_f + (c->line_ftest ? slots : 0);
+  TRY(glb_launch_ftest_lines(s->d_ftest, c->line_psd ? s->d_rows : NULL, f->n, f->n, cn, nchan, crows, thr,
+                             c->lc->max_lines, c->lc->bin_lo, c->lc->bin_hi, d_count, d_bin,
+                             c->line_ftest ? d_f : NULL, c->line_psd ? d_p : NULL, s->stream));
+  TRY(glb_memcpy_d2h(s->h_lines, s->d_lines, bytes, s->stream));
+  s->lines_done = done;
+  s->lines_cn = cn;
+  return 0;
+}
+
+/* the staged lines of slot s (its stream synchronised) into the caller's arrays */
+static void lines_handover(const glb_cframe_call *c, glb_cslot *s, int nchan)
+{
+  const long long cn = s->lines_cn, nf = nchan * cn, M = c->lc->max_lines;
+  const size_t slots = (size_t) nf * M;
+  const int *h_count = s->h_lines, *h_bin = h_count + nf;
+  const float *h_f = (const float *) (h_bin + slots);
+  const float *h_p = h_f + (c->line_ftest ? slots : 0);
+  for (int ch = 0; ch < nchan; ch++) {
+    const size_t to = (size_t) (ch * c->nframes + s->lines_done), from = (size_t) (ch * cn);
+    const size_t m = sizeof(float) * (size_t) (cn * M);
+    memcpy(c->line_count + to, h_count + from, sizeof(int) * (size_t) cn);
+    memcpy(c->line_bin + to * M, h_bin + from * M, m);
+    if (c->line_ftest) memcpy(c->line_ftest + to * M, h_f + from * M, m);
+    if (c->line_psd) memcpy(c->line_psd + to * M, h_p + from * M, m);
+  }
+  s->lines_cn = 0;
+}
+
 int glb_cframe_run(glb_cframe *f, const glb_cframe_call *c)
 {
-  if (!c->src || (c->display ? !c->dc : (!c->ftest_on && !c->rows)))
+  if (!c->src || (c->display ? !c->dc : c->lines ? (!c->lc || !c->line_count || !c->line_bin)
+                                                  : (!c->ftest_on && !c->rows)))
     return glb_host_fail(GLFER_EINVAL, "null argument");
   if (c->wrong_kind) return glb_host_fail(GLFER_EINVAL, c->wrong_kind);
-  if (c->ftest_on) {
+  if (c->ftest_on || c->lines) {
     if (!f->h_tapers) return glb_host_fail(GLFER_EINVAL, c->no_mtm);
     if (f->ntapers < 2) return glb_host_fail(GLFER_EINVAL, "the F-test needs mtm_kmax >= 1 (K' - 1 degrees of freedom)");
-    if (!c->rows && !c->ftest) return glb_host_fail(GLFER_EINVAL, "null argument: rows and ftest are both NULL");
+    if (c->ftest_on && !c->rows && !c->ftest) return glb_host_fail(GLFER_EINVAL, "null argument: rows and ftest are both NULL");
+  }
+  float thr = 0.0f;
+  if (c->lines) {
+    const int rt = glfer_ftest_threshold(f->ntapers, c->lc->pfa, &thr);
+    if (rt != 0) return rt;
+    if (c->lc->max_lines < 1 || c->lc->max_lines > 1024) return glb_host_fail(GLFER_EINVAL, "max_lines must be in 1..1024");
+    if (c->lc->bin_lo < 0 || c->lc->bin_lo >= c->lc->bin_hi || c->lc->bin_hi > f->n)
+      return glb_host_fail(GLFER_EINVAL, "bin range must satisfy 0 <= bin_lo < bin_hi <= n");
   }
   if (c->nframes < 0 || c->first_frame < 0) return glb_host_fail(GLFER_EINVAL, "negative frame range");
   if (c->origin < 0 || c->count < 0) return glb_host_fail(GLFER_EINVAL, "negative origin or sample count");
@@ -269,6 +338,7 @@ int glb_cframe_run(glb_cframe *f, const glb_cframe_call *c)
                           f->slot[0]->stream));
   int rc = 0, ci = 0;
   long long done = 0;
+  for (int i = 0; i < GLB_CSLOTS; i++) f->slot[i]->lines_cn = 0;
   while (done < c->nframes && rc == 0) {
     const int i = ci % GLB_CSLOTS, prev = ci > 0 ? (ci - 1) % GLB_CSLOTS : -1;
     glb_cslot *s = f->slot[i];
@@ -281,6 +351,7 @@ int glb_cframe_run(glb_cframe *f, const glb_cframe_call *c)
     const float *z = NULL;
     long long z_origin = 0, z_count = 0;
     rc = glb_host_shim(glb_stream_sync(s->stream));
+    if (rc == 0 && s->lines_cn) lines_handover(c, s, nchan);
     if (rc == 0 && c->display) rc = glb_display_reserve(&s->disp, nl, n, c->rgb != NULL);
     if (rc == 0) rc = c->stage(c->plan, c, i, prev, c0, cn, crows * f->hop, &z, &z_origin, &z_count);
     if (rc == 0) rc = cframe_launch(f, s, c, &dr, z, z_origin, z_count, c0, nl);
@@ -289,6 +360,7 @@ int glb_cframe_run(glb_cframe *f, const glb_cframe_call *c)
                            c0, cn, crows, done, f->overlap, c->rgb != NULL, s->stream);
     if (rc == 0 && c->display)
       rc = glb_display_fetch(&dr, &s->disp, cn, crows, n, done, c->levels, c->rgb, s->stream);
+    if (rc == 0 && c->lines) rc = lines_chunk(f, s, c, thr, nchan, cn, crows, done);
     for (int ch = 0; ch < nchan && rc == 0; ch++) {
       const size_t to = (size_t) (ch * c->nframes + done) * n, from = (size_t) (ch * crows) * n;
       if (c->rows)
@@ -304,6 +376,8 @@ int glb_cframe_run(glb_cframe *f, const glb_cframe_call *c)
   for (int i = 0; i < GLB_CSLOTS; i++) {
     const int r2 = glb_host_shim(glb_stream_sync(f->slot[i]->stream));
     if (rc == 0) rc = r2;
+    if (rc == 0 && f->slot[i]->lines_cn) lines_handover(c, f->slot[i], nchan);
+    f->slot[i]->lines_cn = 0;
   }
   if (rc == 0 && c->display) rc = glb_display_end(&f->disp, &dr, c->nframes, c->agc_state, c->range_out);
   return rc;

@@ -178,3 +178,14 @@ void glb_mtm_ftest_weights(int n, int K, const double *tapers, double *u0, float
   }
   *s = s2;
 }
+
+/* include/glfer_b200.h: the F(2, 2K' - 2) threshold of a per-bin false-alarm probability, in double, rounded to float */
+int glfer_ftest_threshold(int ntapers, double pfa, float *thr)
+{
+  if (!thr) return glb_host_fail(GLFER_EINVAL, "null argument");
+  if (ntapers < 2) return glb_host_fail(GLFER_EINVAL, "the F-test needs K' >= 2 tapers (K' - 1 degrees of freedom)");
+  if (!(pfa > 0.0 && pfa < 1.0)) return glb_host_fail(GLFER_EINVAL, "pfa must be in (0, 1)");
+  const double m = ntapers - 1;
+  *thr = (float) (m * expm1(-log(pfa) / m));
+  return 0;
+}

@@ -93,6 +93,9 @@ typedef struct {                /* per slot (stream); embedded in the plan's own
   void *d_scratch;              /* the general path's (glb_iq_gram_scratch_bytes) */
   size_t scratch_cap;           /* bytes */
   glb_display_slot disp;        /* display mapping */
+  void *d_lines, *h_lines;      /* *_run_mtm_lines: the chunk's line arrays on the device and their pinned staging */
+  size_t dlines_cap, hlines_cap;     /* bytes */
+  long long lines_done, lines_cn;    /* h_lines holds frames [lines_done, lines_done + lines_cn) of the run (0: none) */
 } glb_cslot;
 typedef struct {                /* per plan */
   int n, hop, device;
@@ -136,6 +139,10 @@ struct glb_cframe_call {        /* one run entry's call */
   const glfer_display_config *dc;
   float *agc_state, *range_out;
   unsigned char *levels, *rgb;
+  int lines;                    /* a *_run_mtm_lines entry: the F rows stay on the device, only the lines come back */
+  const glfer_lines_config *lc;
+  int *line_count, *line_bin;
+  float *line_ftest, *line_psd;
   /* from the plan */
   int nchan;                    /* channels (zoom bank): the caller's outputs are [nchan][nframes]...; 0 or 1: one */
   void *plan;
@@ -148,7 +155,7 @@ struct glb_cframe_call {        /* one run entry's call */
   const char *no_mtm, *short_span;   /* the plan's messages: F-test without a multitaper plan, samples short */
 };
 /* checks the call, then walks its frames in chunks of chunk_frames on the slots in turn: the plan's stage, the launch,
- * and the rows / F rows downloads or the display chain */
+ * and the rows / F rows downloads, the display chain or the line selection */
 int glb_cframe_run(glb_cframe *f, const glb_cframe_call *c);
 
 /* values of the hidden globals (weak `opt` / `glfer` when the host program has them) */

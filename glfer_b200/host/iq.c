@@ -14,7 +14,8 @@
  *
  * Multitaper plans (glfer_iq_plan_create_mtm) always bring float rows to the device: their waterfall goes through the
  * display chain, for a fixed range too.  Every multitaper plan serves glfer_iq_run_mtm_ftest, whose chunks bring back
- * F rows beside or instead of the rows.
+ * F rows beside or instead of the rows, and glfer_iq_run_mtm_lines, whose chunks keep the F rows on the device and
+ * bring back only the lines selected from them.
  */
 #include <stdlib.h>
 #include <string.h>
@@ -175,6 +176,25 @@ int glfer_iq_run_mtm_ftest_pcm16(glfer_iq_plan *p, const short *iq, long long or
   return iq_run(p, &(glb_cframe_call) { .src = iq, .pcm16 = 1, .origin = origin, .count = count,
                                         .first_frame = first_frame, .nframes = nframes, .ftest_on = 1, .rows = rows,
                                         .ftest = ftest });
+}
+
+int glfer_iq_run_mtm_lines(glfer_iq_plan *p, const float *iq, long long origin, long long count, long long first_frame,
+                           long long nframes, const glfer_lines_config *lc, int *line_count, int *line_bin,
+                           float *line_ftest, float *line_psd)
+{
+  return iq_run(p, &(glb_cframe_call) { .src = iq, .origin = origin, .count = count, .first_frame = first_frame,
+                                        .nframes = nframes, .lines = 1, .lc = lc, .line_count = line_count,
+                                        .line_bin = line_bin, .line_ftest = line_ftest, .line_psd = line_psd });
+}
+
+int glfer_iq_run_mtm_lines_pcm16(glfer_iq_plan *p, const short *iq, long long origin, long long count,
+                                 long long first_frame, long long nframes, const glfer_lines_config *lc,
+                                 int *line_count, int *line_bin, float *line_ftest, float *line_psd)
+{
+  return iq_run(p, &(glb_cframe_call) { .src = iq, .pcm16 = 1, .origin = origin, .count = count,
+                                        .first_frame = first_frame, .nframes = nframes, .lines = 1, .lc = lc,
+                                        .line_count = line_count, .line_bin = line_bin, .line_ftest = line_ftest,
+                                        .line_psd = line_psd });
 }
 
 /* main_window_draw's mapping of the plan's own rows (include/glfer_b200.h, glfer_iq_run_display) */

@@ -400,6 +400,46 @@ int glfer_zoom_run_iq_mtm_ftest_pcm16(glfer_zoom_plan *p, const short *iq, long 
                                              .rows = rows, .ftest = ftest });
 }
 
+int glfer_zoom_run_mtm_lines(glfer_zoom_plan *p, const float *samples, long long origin, long long count,
+                         long long first_frame, long long nframes, const glfer_lines_config *lc, int *line_count,
+                         int *line_bin, float *line_ftest, float *line_psd)
+{
+  return zoom_run(p, 0, &(glb_cframe_call) { .src = samples, .origin = origin, .count = count,
+                                             .first_frame = first_frame, .nframes = nframes, .lines = 1, .lc = lc,
+                                             .line_count = line_count, .line_bin = line_bin,
+                                             .line_ftest = line_ftest, .line_psd = line_psd });
+}
+
+int glfer_zoom_run_mtm_lines_pcm16(glfer_zoom_plan *p, const short *pcm, long long origin, long long count,
+                               long long first_frame, long long nframes, const glfer_lines_config *lc, int *line_count,
+                               int *line_bin, float *line_ftest, float *line_psd)
+{
+  return zoom_run(p, 0, &(glb_cframe_call) { .src = pcm, .pcm16 = 1, .origin = origin, .count = count,
+                                             .first_frame = first_frame, .nframes = nframes, .lines = 1, .lc = lc,
+                                             .line_count = line_count, .line_bin = line_bin,
+                                             .line_ftest = line_ftest, .line_psd = line_psd });
+}
+
+int glfer_zoom_run_iq_mtm_lines(glfer_zoom_plan *p, const float *iq, long long origin, long long count,
+                            long long first_frame, long long nframes, const glfer_lines_config *lc, int *line_count,
+                            int *line_bin, float *line_ftest, float *line_psd)
+{
+  return zoom_run(p, 1, &(glb_cframe_call) { .src = iq, .origin = origin, .count = count,
+                                             .first_frame = first_frame, .nframes = nframes, .lines = 1, .lc = lc,
+                                             .line_count = line_count, .line_bin = line_bin,
+                                             .line_ftest = line_ftest, .line_psd = line_psd });
+}
+
+int glfer_zoom_run_iq_mtm_lines_pcm16(glfer_zoom_plan *p, const short *iq, long long origin, long long count,
+                                  long long first_frame, long long nframes, const glfer_lines_config *lc, int *line_count,
+                                  int *line_bin, float *line_ftest, float *line_psd)
+{
+  return zoom_run(p, 1, &(glb_cframe_call) { .src = iq, .pcm16 = 1, .origin = origin, .count = count,
+                                             .first_frame = first_frame, .nframes = nframes, .lines = 1, .lc = lc,
+                                             .line_count = line_count, .line_bin = line_bin,
+                                             .line_ftest = line_ftest, .line_psd = line_psd });
+}
+
 /* main_window_draw's mapping of the plan's own rows (include/glfer_b200.h, glfer_zoom_run_display) */
 int glfer_zoom_run_display(glfer_zoom_plan *p, const float *samples, long long origin, long long count,
                            long long first_frame, long long nframes, const glfer_display_config *dc,

@@ -286,6 +286,18 @@ int glb_launch_iq_gram_general(const glb_iq_gram_args *a, void *stream);
  * the two-pass levels of glb_launch_iq_gram) or the mu and den planes (ftest = 1) */
 long long glb_iq_gram_general_scratch_bytes(int n, long long nframes, int levels, int ftest);
 
+/* Harmonic lines of nframes F rows (glfer_b200/csrc/lines.cu; include/glfer_b200.h, glfer_iq_run_mtm_lines): one launch
+ * for nchan channels laid as the frame stage lays them, channel c's frame i at row c crows + i of ftest (and of rows,
+ * the multitaper rows, needed only for line_psd), rows of n floats at a stride of `stride` floats.  Bin j of
+ * [bin_lo, bin_hi) is a candidate when F[j] > thr, F[j] > F[(j - 1) mod n] and F[j] >= F[(j + 1) mod n]; count[o] is
+ * the number of candidates of output frame o = c nframes + i, and slots 0 .. min(count, max_lines) - 1 of bin / line_ftest
+ * / line_psd ([nchan nframes][max_lines]) hold all of them, or the max_lines largest by (F, -j), in ascending j; the
+ * other slots hold -1 / 0.0f / 0.0f.  line_ftest and line_psd may be NULL.  n a power of two in 32..16384, max_lines
+ * 1..1024. */
+int glb_launch_ftest_lines(const float *ftest, const float *rows, int n, long long stride, long long nframes, int nchan,
+                           long long crows, float thr, int max_lines, int bin_lo, int bin_hi, int *count, int *bin,
+                           float *line_ftest, float *line_psd, void *stream);
+
 /* counters */
 unsigned long long glb_kernel_launches(void);
 /* family of the last spectrogram kernel launched: 1 general, 2 TMA ring (or its I/Q form, gram_iq_kernel), 3 warp-per-frame,

@@ -374,6 +374,59 @@ int glfer_zoom_run_iq_mtm_ftest(glfer_zoom_plan *plan, const float *iq, long lon
 int glfer_zoom_run_iq_mtm_ftest_pcm16(glfer_zoom_plan *plan, const short *iq, long long origin, long long count,
                                       long long first_frame, long long nframes, float *rows, float *ftest);
 
+/* ---- harmonic line detection of multitaper I/Q and zoom plans ----
+ * Threshold of the harmonic F-test at a per-bin false-alarm probability pfa under the null, F(2, 2K' - 2):
+ *     P(F > x) = (1 + x / (K' - 1))^-(K' - 1)   =>   x = (K' - 1) expm1(-log(pfa) / (K' - 1)),
+ * computed in double and rounded to float.  Host only, needs no device.  GLFER_EINVAL for ntapers < 2, pfa outside
+ * (0, 1) or thr NULL. */
+int glfer_ftest_threshold(int ntapers, double pfa, float *thr);
+
+typedef struct {
+  double pfa;          /* per-bin false-alarm probability, 0 < pfa < 1 -> thr = glfer_ftest_threshold(K', pfa) */
+  int max_lines;       /* slots per frame, 1..1024 */
+  int bin_lo, bin_hi;  /* row positions searched, 0 <= bin_lo < bin_hi <= n (a zoom's clean span is about n/2 +- 0.4 n) */
+} glfer_lines_config;
+
+/* The lines of each frame, selected on the device from the F rows, which never leave it.  F[f][j] and P[f][j] are the
+ * F row and the row that the *_run_mtm_ftest entry of the same input form returns for the same plan and call (on the
+ * same path: fused or general, glb_force_generic_kernel alike).
+ *   Candidates: bin j in [bin_lo, bin_hi) of frame f with F[j] > thr, F[j] > F[(j - 1) mod n] and F[j] >= F[(j + 1)
+ *   mod n], all float comparisons; the neighbours are cyclic and read from the whole row, also outside the range.  One
+ *   bin per peak, the leftmost of a plateau.  IEEE rules apply: a NaN bin is never a candidate and never beats a
+ *   neighbour (an all-zero frame, F = 0 / 0 = NaN, has no lines); an infinite F can be a line.
+ *   line_count[f]: the number of candidates, also when it exceeds max_lines (the frame was truncated).
+ *   Selected: every candidate when count <= max_lines, otherwise the max_lines candidates with the largest F, ties to
+ *   the smaller j.  They are stored in ascending j in slots 0 .. min(count, max_lines) - 1: line_bin[f][s] = j,
+ *   line_ftest[f][s] = F[f][j], line_psd[f][s] = P[f][j], the same floats bit for bit; the other slots hold bin -1, F
+ *   0.0f and psd 0.0f.
+ *   Layouts: line_count [nframes], the others [nframes][max_lines]; a bank adds a leading channel axis ([C][nframes],
+ *   [C][nframes][max_lines]) and channel c is bit-identical to a single-centre plan at its centre.  line_count and
+ *   line_bin are required; line_ftest and line_psd may be NULL (without line_psd no rows are formed on the device).
+ *   The outputs are staged in pinned memory of the plan, so pageable arrays do not stall the chunk pipeline.
+ * GLFER_EINVAL for everything the *_mtm_ftest entries reject, and for lc NULL, pfa outside (0, 1), max_lines outside
+ * 1..1024, a bin range outside 0 <= bin_lo < bin_hi <= n, and line_count or line_bin NULL; all checked before any
+ * device call.
+ * Not covered: the sub-bin frequency and the complex amplitude (mu) of a line, and line detection of real
+ * GLFER_MODE_MTM plans, whose F-test has DC and Nyquist special cases (inf at n/2). */
+int glfer_iq_run_mtm_lines(glfer_iq_plan *plan, const float *iq, long long origin, long long count,
+                           long long first_frame, long long nframes, const glfer_lines_config *lc, int *line_count,
+                           int *line_bin, float *line_ftest, float *line_psd);
+int glfer_iq_run_mtm_lines_pcm16(glfer_iq_plan *plan, const short *iq, long long origin, long long count,
+                                 long long first_frame, long long nframes, const glfer_lines_config *lc,
+                                 int *line_count, int *line_bin, float *line_ftest, float *line_psd);
+int glfer_zoom_run_mtm_lines(glfer_zoom_plan *plan, const float *samples, long long origin, long long count,
+                             long long first_frame, long long nframes, const glfer_lines_config *lc, int *line_count,
+                             int *line_bin, float *line_ftest, float *line_psd);
+int glfer_zoom_run_mtm_lines_pcm16(glfer_zoom_plan *plan, const short *pcm, long long origin, long long count,
+                                   long long first_frame, long long nframes, const glfer_lines_config *lc,
+                                   int *line_count, int *line_bin, float *line_ftest, float *line_psd);
+int glfer_zoom_run_iq_mtm_lines(glfer_zoom_plan *plan, const float *iq, long long origin, long long count,
+                                long long first_frame, long long nframes, const glfer_lines_config *lc,
+                                int *line_count, int *line_bin, float *line_ftest, float *line_psd);
+int glfer_zoom_run_iq_mtm_lines_pcm16(glfer_zoom_plan *plan, const short *iq, long long origin, long long count,
+                                      long long first_frame, long long nframes, const glfer_lines_config *lc,
+                                      int *line_count, int *line_bin, float *line_ftest, float *line_psd);
+
 /* ---- display output of I/Q and zoom plans ----
  * The waterfall of the plan's own rows, as glfer_gram_run_display gives it for real audio: levels, rgb, agc_state
  * and display_range as there, and exactly main_window_draw's mapping (g_main.c:1109-1229) of the rows that
